@@ -10,6 +10,8 @@ workload: synthetic MovieGraphs-shaped clips (SURVEY.md §8d C4) whose pooled ve
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torchrun)
   python bench.py --preset {modalities,int_rels,int_ch,int_rel_ch,stress} [--batch B]
   python bench.py --impl reference ...                      CPU arm: oracle port of the reference
+  python bench.py ... --dump-outputs DIR                    also write the last timed step's loss, parameters and
+                                                            gradients as .npy files (same arguments, same inputs)
 
 One JSON line on stdout (rank 0).
   value   device-resident throughput (batches already staged in HBM).
@@ -100,6 +102,8 @@ def parse_args():
     ap.add_argument("--no_traffic", action="store_true", help="skip the live DRAM-traffic capture (ncu child process)")
     ap.add_argument("--only_value", action="store_true", help="device-resident leg only (profiling runs)")
     ap.add_argument("--dump_profile", default="", help="write the per-launch GEMM event timings to this file")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step computed to DIR/{loss,params,grads}.npy (see dump_outputs)")
     ap.add_argument("--nccl_allreduce", action="store_true",
                     help="N > 1: use ncclAllReduce + Adam instead of the in-switch reduce + Adam kernels")
     ap.add_argument("--dp_mode", default="", choices=["", "shard", "bucket"],
@@ -446,7 +450,7 @@ class Bench:
         for i in range(steps):
             if profile:                       # per-launch GEMM events on every PROFILE_EVERY-th step only: an event
                 _ext.profile_sample(i % PROFILE_EVERY == 0)      # pair per launch breaks the PDL chain of the step
-            self.step(self.resident[i % len(self.resident)])
+            self.last_loss = self.step(self.resident[i % len(self.resident)])
         e1.record()
         self.barrier()
         if sampler is not None:
@@ -518,6 +522,26 @@ def measure_traffic(args):
         return None, "no GEMM launch in the ncu capture"
     return int(total), "dram__bytes_read.sum + dram__bytes_write.sum summed over the %d GEMM launches of one step, " \
                        "measured by an `ncu --metrics` child process of this run" % len(launches)
+
+
+DUMP_MAX_ELEMS = 4 << 20          # per sampled array: 16 MB of float32, so the three files stay under 64 MB
+
+
+def dump_outputs(model, loss, out_dir):
+    """What the last timed step handed its caller, as float32 .npy files in `out_dir`: `loss` (the value
+    train_step returned), `params` (every parameter after the step's Adam update) and `grads` (the step's
+    gradients), both flattened in named_parameters order.  Above DUMP_MAX_ELEMS elements both keep the same
+    sorted sample of positions drawn with a fixed seed, so two builds of the same model compare entry for entry."""
+    os.makedirs(out_dir, exist_ok=True)
+    params = list(model.parameters())
+    p = torch.cat([q.detach().reshape(-1) for q in params])
+    g = torch.cat([q.grad.detach().reshape(-1) for q in params])
+    if p.numel() > DUMP_MAX_ELEMS:
+        pick = np.sort(np.random.default_rng(0).choice(p.numel(), DUMP_MAX_ELEMS, replace=False))
+        pick = torch.from_numpy(pick).to(p.device)
+        p, g = p[pick], g[pick]
+    for name, t in (("loss", loss.detach().reshape(1)), ("params", p), ("grads", g)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def dp_parity_check(b):
@@ -614,6 +638,8 @@ def run_ours(args):
     # ---------------- device-resident timed region ----------------
     ms_total, prof, launches = b.timed_resident(steps, warmup, sampler if rank == 0 else None,
                                                 ncu_window=args.ncu_window)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(b.model, b.last_loss, args.dump_outputs)
     clips_total = args.batch * world * steps
     value = clips_total / (ms_total / 1e3)
     profiled_steps_main = b.profiled_steps

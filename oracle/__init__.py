@@ -5,10 +5,8 @@ tests/, by __graft_entry__.smoke() and by bench.py's cpu_baseline / --impl refer
 the checker and the reported CPU baseline, never as the product path.
 
 Parity status: the reference ships no tests, golden vectors or fixtures for this path
-(SURVEY.md §4, §8c), so the restatement is pinned against the reference ITSELF: in the build
-container the unmodified reference modules are imported from /root/reference
-(oracle/reference_shim.py) and (a) compared live with this restatement
-(tests/test_oracle_vs_reference.py, skipped where /root/reference is absent) and (b) used to
-generate the golden input/output vectors committed under tests/golden/
+(SURVEY.md §4, §8c), so the restatement is pinned against the reference ITSELF: the unmodified
+reference modules, imported through oracle/reference_shim.py where a reference tree is available,
+generated the golden input/output vectors committed under tests/golden/
 (tests/golden/make_golden.py), which the restatement is checked against everywhere.
 """

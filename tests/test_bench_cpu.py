@@ -70,3 +70,32 @@ def test_clock_samples_are_sorted_into_their_regions(bench):
     s2.region(False)
     assert [x[0] for x in s2.spans] == ["value", "e2e"] and all(b >= a for _, a, b in s2.spans)
     assert s2.stop()["samples"] == 0
+
+
+def test_dump_outputs_writes_loss_params_and_grads(bench, tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    model = torch.nn.Sequential(torch.nn.Linear(6, 5), torch.nn.Linear(5, 3))
+    n = sum(q.numel() for q in model.parameters())
+    with torch.no_grad():                     # parameter value = its position in named_parameters order
+        for q, start in zip(model.parameters(), np.cumsum([0] + [q.numel() for q in model.parameters()])):
+            q.copy_(torch.arange(start, start + q.numel(), dtype=torch.float32).view(q.shape))
+            q.grad = 2 * q + 1
+    loss = torch.tensor(0.25)
+
+    def load(d):
+        return {k: np.load(os.path.join(str(tmp_path), d, k + ".npy")) for k in ("loss", "params", "grads")}
+    bench.dump_outputs(model, loss, os.path.join(str(tmp_path), "all"))
+    z = load("all")
+    assert all(v.dtype == np.float32 for v in z.values())
+    assert z["loss"].tolist() == [0.25]
+    assert np.array_equal(z["params"], np.arange(n, dtype=np.float32))
+    assert np.array_equal(z["grads"], 2 * z["params"] + 1)
+    # above the cap: one fixed sample of positions, the same for both arrays and from run to run
+    monkeypatch.setattr(bench, "DUMP_MAX_ELEMS", 10)
+    bench.dump_outputs(model, loss, os.path.join(str(tmp_path), "a"))
+    bench.dump_outputs(model, loss, os.path.join(str(tmp_path), "b"))
+    a, b = load("a"), load("b")
+    assert a["params"].shape == (10,) and np.all(np.diff(a["params"]) > 0) and a["params"].max() < n
+    assert np.array_equal(a["grads"], 2 * a["params"] + 1)
+    assert all(np.array_equal(a[k], b[k]) for k in a)

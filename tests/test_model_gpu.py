@@ -89,7 +89,7 @@ def test_relationship_only_model_parity(train, opt_preset):
     """opt.ints == 0 (reference mlp/model.py:102, 140, 151, 208; loss :391): no interaction branch, no interaction
     head — the context branch and the relationship head alone, trained by the relationship term of
     MultiTaskMaxMargin.  The reference's GatingUnit needs both features, so gates are off.  The oracle of this
-    configuration is pinned against the unmodified reference in tests/test_oracle_vs_reference.py."""
+    configuration is pinned against the unmodified reference in tests/test_oracle_golden.py."""
     import lirec_b200.mlp.model as M
     opt = opt_preset("int_rels", ints=0, gates=0)
     for seed in (3, 4):

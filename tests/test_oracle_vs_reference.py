@@ -1,110 +1,49 @@
-"""Live check of the oracle against the UNMODIFIED reference imported from /root/reference (only in
-the build container; skipped where the reference tree is absent, e.g. on the GPU box).  Full-size
-model (18.4 M parameters), synthetic MovieGraphs-shaped dense batch from the same generator the GPU
-parity tests use."""
+"""lirec_b200's models against the UNMODIFIED reference's initial parameters, stored with the golden cases
+(tests/golden/*.npz, `p_*` arrays): tests/golden/make_golden.py builds every case's model with the reference's
+own create_model under torch.manual_seed(<position of the case in its CASES list>), at the reduced dims below."""
+import ast
+import glob
+import os
+
 import numpy as np
-import pytest
 import torch
 
-from oracle import reference_shim as rs
-
-pytestmark = pytest.mark.skipif(not rs.available(), reason="/root/reference is not mounted")
-
-
-def _rel(a, b):
-    return float((a.double() - b.double()).abs().max() / (b.double().abs().max() + 1e-30))
-
-
-@pytest.mark.parametrize("train", [False, True], ids=["eval", "train"])
-@pytest.mark.parametrize("preset,over", [("int_rel_ch", {}), ("int_rel_ch", dict(tr_correct=True)),
-                                         ("int_rel_ch", dict(tr_max_neg=True)), ("int_ch", {}),
-                                         ("int_rels", {}), ("modalities", {}),
-                                         # opt.ints == 0: the context branch and the relationship head alone
-                                         # (mlp/model.py:102, 140, 151, 208; loss :391); the gate needs both features
-                                         ("int_rels", dict(ints=0, gates=0))])
-def test_full_size_forward_loss_backward(preset, over, train):
-    """eval: dropout off on both sides.  train: the UNMODIFIED reference forward runs in train mode with
-    its nn.Dropout modules (mlp/model.py:52, 347) replaced by a replayer that applies, in the reference's
-    call order, the very masks the oracle receives by key — this pins the oracle's dropout sites, their
-    order and the relu(dropout(.)) / dropout(tanh(.)) / dropout(relu(.)) placements (:62, 88, 353)."""
-    from lirec_b200.mixed_utils import synthetic
-    from oracle import losses as ol, model as om
-    B = 3
-    pb = synthetic.make_batch(B, seed=21, preset=preset)
-    dense = pb.to_dense(np.float64)
-    model, loss = rs.create_model(preset, 101, 15, seed=1, **over)
-    model.eval()
-    masks = None
-    if train:
-        kind0 = synthetic.PRESETS[preset]["kind"]
-        ctx0 = preset in ("int_rels", "int_rel_ch")
-        rows = B * dense["features"].shape[1] if kind0 == "maxtracks" else B
-        masks = rs.random_masks(kind0, rows, 18, 512, 3072, 0.3, torch.Generator().manual_seed(77), ctx=ctx0,
-                                gates=ctx0 and bool(over.get("gates", 1)), ints=bool(over.get("ints", 1)))
-        queue = rs.replay_dropout(model, masks, 0.3)
-    batch = {k: (v.clone() if isinstance(v, torch.Tensor) else v) for k, v in dense.items()}
-    kind = synthetic.PRESETS[preset]["kind"]
-    if kind == "modalities":
-        batch["features"] = batch["features"].reshape(B, 1, -1)
-    elif kind == "midfusion":
-        S1 = batch["features"].shape[2]
-        batch["features"] = batch["features"].reshape(B, S1, -1)
-        batch["rels_mask"] = batch["rels_mask"].reshape(B, -1, 1)
-        batch["labels"] = batch["labels"].reshape(B, 1, 1).expand(B, S1, 1).contiguous()
-        batch["rels_label"] = batch["rels_label"].reshape(B)
-    out = model(batch)
-    if train:
-        assert not queue, "the reference forward consumed %d masks fewer than the oracle has sites" % len(queue)
-    lv = rs.run_loss(loss, out, batch)
-    lv.backward()
-
-    sd = {k: v.detach().clone().double().requires_grad_(True) for k, v in model.state_dict().items()}
-    ctx = preset in ("int_rels", "int_rel_ch")
-    cfg = om.default_cfg(ctx=int(ctx), gates=int(ctx and over.get("gates", 1)), ints=int(over.get("ints", 1)), dropout=0.3)
-    f = dense["features"]
-    if kind == "modalities":
-        o = om.modalities_forward(sd, f.reshape(B, 1, -1), cfg, masks)
-        l = ol.max_margin_ce(o["inters"], dense["labels"], dense["multilab_weights"], 0.101)
-    elif kind == "midfusion":
-        o = om.midfusion_forward(sd, f.reshape(B, -1, f.shape[-1]), dense["rels_mask"].reshape(B, -1, 1), cfg, masks)
-        l = ol.multitask_max_margin(o["inters"], o["rels"], dense["labels"].reshape(B, 1, 1),
-                                    dense["rels_label"].reshape(B), dense["multilab_weights"], 0.101, 1.0, 15,
-                                    ints=int(over.get("ints", 1)))
-        assert (o["inters"] is None) == (out["inters"] is None)
-    elif ctx:
-        o = om.maxtracks_forward(sd, f, dense["rels_mask"], cfg, masks)
-        l = ol.margin_track_rels(o["inters"], o["rels"], dense["labels"], dense["rels_label"], dense["mem_mask"],
-                                 dense["multilab_weights"], dense["gt_tracks"], 0.101, 1.0, 15,
-                                 tr_correct=bool(over.get("tr_correct")), max_neg=bool(over.get("tr_max_neg")))[0]
-    else:
-        o = om.maxtracks_forward(sd, f, None, cfg, masks)
-        l = ol.margin_loss(o["inters"], dense["labels"], dense["mem_mask"], dense["multilab_weights"],
-                           dense["gt_tracks"], 0.101)[0]
-    l.backward()
-    assert abs(l.item() - lv.item()) < 1e-5 * abs(lv.item())
-    for k, p in model.named_parameters():
-        assert _rel(sd[k].grad, p.grad) < 2e-4, k          # fp64 oracle vs fp32 reference
+GOLDEN = sorted(p for p in glob.glob(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "*.npz"))
+                if not os.path.basename(p).startswith(("dataloader_", "pooling_", "eval_")))
+DIMS = dict(text_dim=24, visual_dim=40, track_dim=40, joint_dim=16, mid_m_ints=6)
+C, R = 11, 5
+# make_golden.py's CASES, in order: a case's position is the torch seed its model was built under
+CASE_SEEDS = {stem: seed for seed, stem in enumerate((
+    "modalities", "modalities_modality-t_tracks-False", "modalities_modality-v_tracks-False", "modalities_tracks-False",
+    "int_rels", "int_ch", "int_ch_tr_correct", "int_ch_tr_max_neg", "int_rel_ch", "int_rel_ch_tr_correct",
+    "int_rel_ch_tr_max_neg", "int_rel_ch_tr_correct_tr_max_neg", "modalities_train", "int_rels_train", "int_ch_train",
+    "int_rel_ch_train", "int_rels_gates-0_ints-0", "int_rels_gates-0_ints-0_train"))}
 
 
-def test_same_seed_gives_the_reference_initial_weights():
+def test_same_seed_gives_the_reference_initial_weights(opt_preset):
     """lirec_b200's modules are constructed in the reference's order, so torch.manual_seed(s) yields
-    bit-identical initial parameters (checked on CPU: construction does not need the GPU)."""
-    import contextlib
-    import io
-    model, _ = rs.create_model("int_rel_ch", 101, 15, seed=5)
-    from lirec_b200.utils.arg_pars import opt
-    saved = dict(vars(opt))
-    try:
-        for k, v in dict(tr_maximize=True, tracks=True, ints=1, ctx=1, gates=1, rels_multitask=True, modality="m",
-                         mod_check=False).items():
-            setattr(opt, k, v)
-        import lirec_b200.mlp.model as M
-        torch.manual_seed(5)
-        ours = M.MidFusionMultiClipMaxTracks(101, 15)
-    finally:
-        for k, v in saved.items():
-            setattr(opt, k, v)
-    ref_sd, our_sd = model.state_dict(), ours.state_dict()
-    assert list(ref_sd.keys()) == list(our_sd.keys())
-    for k in ref_sd:
-        assert torch.equal(ref_sd[k], our_sd[k]), k
+    bit-identical initial parameters, for every model class and flag combination of the golden cases (checked on
+    CPU: construction does not need the GPU)."""
+    import lirec_b200.mlp.model as M
+    assert sorted(os.path.basename(p)[:-4] for p in GOLDEN) == sorted(CASE_SEEDS)
+    for path in GOLDEN:
+        stem = os.path.basename(path)[:-4]
+        z = np.load(path)
+        preset, over = str(z["meta"][0]), dict(ast.literal_eval(str(z["meta"][1])))
+        over.pop("train", None)
+        opt_preset(preset, **DIMS, **over)
+        torch.manual_seed(CASE_SEEDS[stem])
+        if preset == "modalities":
+            # create_model (reference mlp/model.py:578-609) builds a MidFusionMultiClip first and replaces it with
+            # Modalities when opt.mod_check is set: the first model's draws come before Modalities' own
+            M.MidFusionMultiClip(C, R)
+            model = M.Modalities(C)
+        elif preset == "int_rels":
+            model = M.MidFusionMultiClip(C, R)
+        else:
+            model = M.MidFusionMultiClipMaxTracks(C, R)
+        ours = model.state_dict()
+        ref = {k[2:]: z[k] for k in z.files if k.startswith("p_")}
+        assert list(ours) == list(ref), stem
+        for k in ref:
+            assert torch.equal(ours[k], torch.from_numpy(ref[k])), (stem, k)

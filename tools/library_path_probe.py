@@ -1,8 +1,8 @@
 """The "library path" on the same B200 (SURVEY.md §8d, optional row): the reference's schedule — DENSE zero-padded
 batches, one ATen call per op, autograd, torch.optim.Adam — run by stock PyTorch eager ON THE GPU, next to this
-package's packed / fused path on the same synthetic clips.  The reference tree cannot travel to the GPU box, so
+package's packed / fused path on the same synthetic clips.  The reference tree is not part of this repository, so
 the dense model + loss are the oracle's restatement (pinned against the unmodified reference, tests/golden,
-tests/test_oracle_vs_reference.py) with its tensors moved to cuda:0; matmuls run as TF32 tensor-core GEMMs
+tests/test_oracle_golden.py) with its tensors moved to cuda:0; matmuls run as TF32 tensor-core GEMMs
 (cuBLAS), everything else as the usual elementwise ATen kernels.
 
     python tools/library_path_probe.py [--batches 64,256] [--preset int_rel_ch]
