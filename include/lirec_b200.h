@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define LIREC_ABI_VERSION 1
+#define LIREC_ABI_VERSION 2
 
 enum lirec_status {
   LIREC_OK = 0,
@@ -140,7 +140,7 @@ typedef struct lirec_gemm_problem {
 
 /* One persistent launch over all tiles of all problems (host array).  Kernel choice per launch: the
  * CTA-pair kernel (256-row tiles, tcgen05 cta_group::2) unless the launch is too small to fill 60 % of
- * the clusters and fits one wave of 128x128 tiles (single-CTA kernel); LIREC_GEMM_PAIR=1/0 forces one. */
+ * the clusters and fits one wave of 128x128 tiles (single-CTA kernel). */
 int lirec_gemm_grouped(const lirec_gemm_problem* problems_host, int num_problems,
                        void* stream);
 /* Per-launch timing of the GEMM kernel (CUDA events on the launching stream), for bench.py's
@@ -161,17 +161,14 @@ int lirec_last_launch_count(void);
  * (reference: np.max(axis=0) at mixed_utils/mixed_features.py:54,61,105; empty
  * segment -> zeros, text_utils/text_features.py:171-178, mixed_features.py:89-93).
  * x: [total_rows, dim] fp32, seg_off: [nseg+1] int32 prefix sums.
- * mode: 0 = max, 1 = mean.  out_bf16 / out_f32 may each be NULL.            */
-int lirec_seg_reduce_f32(const float* x, const int32_t* seg_off, int32_t nseg,
-                         int32_t dim, int32_t mode, float* out_f32, int64_t out_f32_ld,
-                         void* out_bf16, int64_t out_bf16_ld, void* stream);
-
-/* Same reduction over GATHERED rows: segment s reduces x[row_idx[r]] for r in [seg_off[s], seg_off[s+1]).
+ * mode: 0 = max, 1 = mean.  out_bf16 / out_f32 may each be NULL.
+ * row_idx: NULL for contiguous segments (segment s reduces rows [seg_off[s], seg_off[s+1])), else the
+ * reduction runs over GATHERED rows: segment s reduces x[row_idx[r]] for r in [seg_off[s], seg_off[s+1]).
  * The dialog tokens of a clip are the union of the token ranges of every subtitle line that overlaps the
  * clip's time span (reference text_utils/text_features.py:151-168), not one contiguous range.          */
-int lirec_seg_reduce_gather_f32(const float* x, const int32_t* row_idx, const int32_t* seg_off,
-                                int32_t nseg, int32_t dim, int32_t mode, float* out_f32,
-                                int64_t out_f32_ld, void* out_bf16, int64_t out_bf16_ld, void* stream);
+int lirec_seg_reduce_f32(const float* x, const int32_t* row_idx, const int32_t* seg_off,
+                         int32_t nseg, int32_t dim, int32_t mode, float* out_f32,
+                         int64_t out_f32_ld, void* out_bf16, int64_t out_bf16_ld, void* stream);
 
 /* Softmax-weighted member of the same family, forward and backward — PARITY UNPINNED BY CONSTRUCTION: the
  * reference has no softmax / attention pooling (np.max at mixed_features.py:54, 61, 105; masked mean at
@@ -394,18 +391,14 @@ size_t lirec_model_workspace_bytes(const lirec_model_cfg* cfg, const lirec_batch
 int lirec_model_forward(const lirec_model_cfg* cfg, const lirec_model_params* params,
                         const lirec_batch* batch, void* workspace, size_t workspace_bytes,
                         float* out_ints, float* out_rels, void* stream);
-/* d_ints / d_rels: fp32 gradients w.r.t. the logits.  Writes every grad_w / grad_b. */
+/* d_ints / d_rels: fp32 gradients w.r.t. the logits.  Writes every grad_w / grad_b.
+ * heads_event (a cudaEvent_t; may be NULL): recorded on `stream` as soon as the gradients of the gate and of the
+ * two heads are final in the flat gradient buffer: a data-parallel caller starts the exchange + Adam of that range
+ * (53 % of the weights) on another stream while the encoder stages of backward still run (lirec_b200/dp.py).
+ * Autograd runs backward as one opaque call (mlp/train.py:62). */
 int lirec_model_backward(const lirec_model_cfg* cfg, const lirec_model_params* params,
                          const lirec_batch* batch, void* workspace, size_t workspace_bytes,
-                         const float* d_ints, const float* d_rels, void* stream);
-
-/* Same, and records the CUDA event `heads_event` (a cudaEvent_t; may be NULL) on `stream` as soon as the
- * gradients of the gate and of the two heads are final in the flat gradient buffer: a data-parallel caller
- * starts the exchange + Adam of that range (53 % of the weights) on another stream while the encoder stages of
- * backward still run (lirec_b200/dp.py).  Autograd runs backward as one opaque call (mlp/train.py:62). */
-int lirec_model_backward_ex(const lirec_model_cfg* cfg, const lirec_model_params* params,
-                            const lirec_batch* batch, void* workspace, size_t workspace_bytes,
-                            const float* d_ints, const float* d_rels, void* stream, void* heads_event);
+                         const float* d_ints, const float* d_rels, void* stream, void* heads_event);
 
 /* White-box test aid: byte offsets of the named workspace buffers (see csrc/model.cu). */
 int lirec_model_workspace_layout(const lirec_model_cfg* cfg, const lirec_batch* batch_host,
@@ -450,16 +443,13 @@ int lirec_collate_gather(const int64_t* ds_cand_off, const int32_t* ds_cand, con
 
 /* ---- optimizer -----------------------------------------------------------
  * torch.optim.Adam with coupled L2 (reference mlp/model.py:599-601) over one
- * flat buffer; also refreshes the bf16 shadow of the weights.                */
-int lirec_adam_flat(float* param, const float* grad, float* exp_avg, float* exp_avg_sq,
-                    void* param_bf16, int64_t n, float lr, float beta1, float beta2, float eps,
-                    float weight_decay, int32_t step, float grad_scale, void* stream);
-/* Same pass; coresident != 0 launches it in CTAs small enough to share an SM with a resident CTA of the
+ * flat buffer; also refreshes the bf16 shadow of the weights.
+ * coresident != 0 launches the same pass in CTAs small enough to share an SM with a resident CTA of the
  * persistent GEMM kernels (which leave ~18 % of the register file), for a range whose gradients are final while
  * backward is still running on another stream.  Identical results.                                              */
-int lirec_adam_flat_ex(float* param, const float* grad, float* exp_avg, float* exp_avg_sq,
-                       void* param_bf16, int64_t n, float lr, float beta1, float beta2, float eps,
-                       float weight_decay, int32_t step, float grad_scale, int32_t coresident, void* stream);
+int lirec_adam_flat(float* param, const float* grad, float* exp_avg, float* exp_avg_sq,
+                    void* param_bf16, int64_t n, float lr, float beta1, float beta2, float eps,
+                    float weight_decay, int32_t step, float grad_scale, int32_t coresident, void* stream);
 
 /* ---- data parallel: in-switch gradient exchange, bucket by bucket --------
  * Replaces ncclAllReduce(flat gradient) of a data-parallel step (the reference is single-process, SURVEY.md
@@ -473,7 +463,7 @@ int lirec_adam_flat_ex(float* param, const float* grad, float* exp_avg, float* e
  * lirec_dp_flag_words(world) uint32; `channel` (0..3) selects the flag slots, so chains for different buckets may
  * be in flight on different streams at the same time (all ranks must use the same channel for the same bucket).
  * coresident != 0 (all three passes): CTAs small enough to share an SM with a resident CTA of the persistent GEMM
- * kernels, for a bucket exchanged on a side stream while backward still runs (see lirec_adam_flat_ex).          */
+ * kernels, for a bucket exchanged on a side stream while backward still runs (see lirec_adam_flat).          */
 int lirec_dp_flag_words(int32_t world);
 /* Exchange + optimizer + parameter broadcast in ONE pass (ZeRO-1 style), the default data-parallel step: every
  * rank owns the Adam moments of its 1/world shard.  For its shard it sums the gradients inside the switch

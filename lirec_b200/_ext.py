@@ -116,10 +116,8 @@ def lib():
     L.lirec_device_check.argtypes = [C.c_int]
     L.lirec_dropout_keep_host.argtypes = [C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_float]
     L.lirec_gemm_grouped.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
-    L.lirec_seg_reduce_f32.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
+    L.lirec_seg_reduce_f32.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                        C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
-    L.lirec_seg_reduce_gather_f32.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
-                                              C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
     L.lirec_seg_softmax_pool_fwd.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_int32,
                                              C.c_float, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
     L.lirec_seg_softmax_pool_bwd.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_int32,
@@ -150,9 +148,7 @@ def lib():
     L.lirec_predict_tracks.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
     L.lirec_adam_flat.argtypes = [C.c_void_p] * 5 + [C.c_int64] + [C.c_float] * 5 + [C.c_int32, C.c_float,
-                                                                                  C.c_void_p]
-    L.lirec_adam_flat_ex.argtypes = [C.c_void_p] * 5 + [C.c_int64] + [C.c_float] * 5 + [C.c_int32, C.c_float,
-                                                                                     C.c_int32, C.c_void_p]
+                                                                                  C.c_int32, C.c_void_p]
     L.lirec_profile_sample.argtypes = [C.c_int32]
     L.lirec_dp_flag_words.argtypes = [C.c_int32]
     L.lirec_dp_flag_words.restype = C.c_int
@@ -170,9 +166,7 @@ def lib():
     L.lirec_model_forward.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
                                       C.c_void_p, C.c_void_p, C.c_void_p]
     L.lirec_model_backward.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
-                                       C.c_void_p, C.c_void_p, C.c_void_p]
-    L.lirec_model_backward_ex.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
-                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.lirec_collate_arena_bound.argtypes = [C.c_int64, C.c_int64, C.c_int64, C.c_int32]
     L.lirec_collate_arena_bound.restype = C.c_int64
     L.lirec_collate_tables.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32,
@@ -180,7 +174,7 @@ def lib():
                                        C.c_void_p]
     L.lirec_collate_gather.argtypes = [C.c_void_p] * 6 + [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                                           C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
-    if L.lirec_abi_version() != 1:
+    if L.lirec_abi_version() != 2:
         raise RuntimeError("liblirec_b200.so ABI version mismatch; rebuild it")
     _lib = L
     return L
@@ -188,9 +182,9 @@ def lib():
 
 EXPORTED_SYMBOLS = [
     "lirec_abi_version", "lirec_last_error", "lirec_device_check", "lirec_dropout_keep_host", "lirec_last_launch_count",
-    "lirec_gemm_grouped", "lirec_profile_begin", "lirec_profile_end", "lirec_seg_reduce_f32", "lirec_seg_reduce_gather_f32", "lirec_seg_softmax_pool_fwd", "lirec_seg_softmax_pool_bwd", "lirec_rows_expand_fwd", "lirec_rows_expand_bwd",
+    "lirec_gemm_grouped", "lirec_profile_begin", "lirec_profile_end", "lirec_seg_reduce_f32", "lirec_seg_softmax_pool_fwd", "lirec_seg_softmax_pool_bwd", "lirec_rows_expand_fwd", "lirec_rows_expand_bwd",
     "lirec_split_f32", "lirec_cast_bf16", "lirec_gather_rows", "lirec_roi_max_pool_f32", "lirec_loss_track_fwd_bwd", "lirec_loss_rowmargin_fwd_bwd", "lirec_loss_ce_fwd_bwd", "lirec_predict_tracks",
-    "lirec_model_workspace_bytes", "lirec_model_workspace_layout", "lirec_model_forward", "lirec_model_backward", "lirec_model_backward_ex", "lirec_adam_flat", "lirec_adam_flat_ex", "lirec_profile_sample", "lirec_dp_flag_words", "lirec_dp_exchange", "lirec_dp_reduce_adam_bcast", "lirec_dp_reduce_adam_bcast_peer",
+    "lirec_model_workspace_bytes", "lirec_model_workspace_layout", "lirec_model_forward", "lirec_model_backward", "lirec_adam_flat", "lirec_profile_sample", "lirec_dp_flag_words", "lirec_dp_exchange", "lirec_dp_reduce_adam_bcast", "lirec_dp_reduce_adam_bcast_peer",
     "lirec_collate_arena_bound", "lirec_collate_tables", "lirec_collate_gather",
 ]
 

@@ -20,7 +20,7 @@ NVCC_FLAGS = [
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=default",
     "--shared",
 ]
-# A/B knobs for kernel experiments (defaults are what ships): LIREC_NVCC_DEFINES="-DLIREC_EPI_WARPS=16 ..."
+# Extra -D flags for instrumented builds (tools/build_variants.sh): LIREC_NVCC_DEFINES="-DLIREC_GEMM_TRACE=1"
 NVCC_FLAGS += [f for f in os.environ.get("LIREC_NVCC_DEFINES", "").split() if f.startswith("-D")]
 
 

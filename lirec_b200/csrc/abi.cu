@@ -20,15 +20,6 @@ int fail(int code, const char* fmt, ...) {
 }
 
 void note_launch(int n) { g_launches += n; }
-
-bool pdl_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("LIREC_PDL");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v != 0;
-}
 void reset_launch_count() { g_launches = 0; }
 
 // Largest CTA of `kernel` (a multiple of 32 threads, <= cap) whose registers fit beside one resident GEMM CTA.

@@ -44,11 +44,8 @@ int check_arch();  // LIREC_OK when the current device is sm_100
 // 10 % of a 64-clip step.  Kernels launched through launch_pdl() may be scheduled BEFORE their predecessor has
 // finished; each calls pdl_wait() ahead of its first global access (it returns once every prerequisite grid has
 // completed and flushed its memory) and pdl_trigger() right after, so its own successor can be set up early too.
-// LIREC_PDL=0 launches them as ordinary stream-ordered kernels (A/B knob).
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
-bool pdl_enabled();
 
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
@@ -62,7 +59,7 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 

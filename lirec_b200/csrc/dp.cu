@@ -18,7 +18,7 @@
 //             backward may overwrite the gradients);
 //
 // followed by lirec_adam_flat over the bucket.  The first bucket's chain is launched on a side stream as
-// soon as backward has recorded its "head gradients final" event (lirec_model_backward_ex), so its exchange
+// soon as backward has recorded its "head gradients final" event (lirec_model_backward), so its exchange
 // and its Adam pass overlap the second-layer / first-layer backward stages.
 //
 // Round 1 did all of this in ONE kernel whose CTAs spun on each other (grid-wide flags): that needs every

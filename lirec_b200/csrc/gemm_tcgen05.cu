@@ -36,11 +36,6 @@ constexpr int BM = 128;       // tile rows  (UMMA M, cta_group::1)
 constexpr int BK = 64;        // bf16 elements per k-block = one 128B swizzle span
 constexpr int BN128 = 128;    // tile columns of the single-CTA kernel
 constexpr int UMMA_K = 16;
-#ifndef LIREC_EPI_WARPS
-#define LIREC_EPI_WARPS 8
-#endif
-// A/B knobs of the epilogue (tools/build_variants.sh): per-tile copy of the epilogue descriptor out of parameter
-// space, and the auxiliary-tensor loads of the backward epilogues issued ahead of the accumulator wait
 // LIREC_GEMM_TRACE=1 (variant build, tools/gemm_trace.py): every role stamps clock64() per tile into a device
 // buffer — producer first / last issue, MMA accumulator-free / first-operands / commit, epilogue wake / done.
 #ifndef LIREC_GEMM_TRACE
@@ -54,16 +49,7 @@ constexpr int UMMA_K = 16;
 #else
 #define LIREC_TRACE(field) do { } while (0)
 #endif
-#ifndef LIREC_EPI_STAGE_NATURAL
-#define LIREC_EPI_STAGE_NATURAL 1
-#endif
-#ifndef LIREC_EPI_HOIST
-#define LIREC_EPI_HOIST 1
-#endif
-#ifndef LIREC_EPI_PREFETCH
-#define LIREC_EPI_PREFETCH 1
-#endif
-constexpr int NUM_EPI_WARPS = LIREC_EPI_WARPS;  // 4 or 8
+constexpr int NUM_EPI_WARPS = 8;
 constexpr int NUM_THREADS = 64 + 32 * NUM_EPI_WARPS;
 // Warp roles.  The SM's issue arbiter favours the highest warp id of a sub-partition, so the two
 // single-thread roles whose latency paces the whole CTA (TMA producer, MMA issuer) take the TOP ids
@@ -381,9 +367,6 @@ struct AuxRegs {
 };
 __device__ __forceinline__ void aux_prefetch(const DevEpi& e, int M, int N, int m_true, int n0, AuxRegs& a) {
   a.ready = false;
-#if !LIREC_EPI_PREFETCH
-  return;
-#endif
   if ((e.post != LIREC_POST_DRELU && e.post != LIREC_POST_DTANH) || !e.aux_vec_ok || n0 + 32 > N) return;
   const int m = min(m_true, M - 1);
   const uint4* ap = reinterpret_cast<const uint4*>(e.aux + static_cast<int64_t>(m) * e.aux_ld + e.aux_col_off + n0);
@@ -425,7 +408,7 @@ __device__ __forceinline__ void epilogue_chunk(const DevEpi& e, int M, int N, in
   // instruction — 32 wavefronts and 32 half-written sectors each (in-kernel trace: the epilogue of the
   // second-layer data-gradient tiles, alpha * acc -> fp32, took 7.9 us against 5.3 us of MMA).  Staged, a store
   // instruction carries whole 128-byte lines of 4 rows (fp32) / 64-byte halves of 8 rows (bf16 hi, lo).
-  const bool staged_n = LIREC_EPI_STAGE_NATURAL && stage != nullptr && (N - n0 >= 32) && e.vec_ok &&
+  const bool staged_n = stage != nullptr && (N - n0 >= 32) && e.vec_ok &&
                         ((e.out_kind == LIREC_OUT_F32 && e.out_ld_n == 1 && !e.accumulate) ||
                          e.out_kind == LIREC_OUT_SPLIT_BF16);
   if (m_true >= M && !staged_t && !staged_n) return;
@@ -906,11 +889,7 @@ __device__ __forceinline__ void gemm_body(const GemmParams& P, uint8_t* smem_raw
       const int chunks = tile_n >> 5;
       // the epilogue descriptor out of parameter space once per tile (indexed constant loads per use cost a
       // long-scoreboard stall each), and the first chunk's auxiliary loads in flight BEFORE the accumulator wait
-#if LIREC_EPI_HOIST
       const DevEpi e = pr.epi;
-#else
-      const DevEpi& e = pr.epi;
-#endif
       const int M = pr.M, N = pr.N;
       const int m_row = m0 + quarter * 32 + lane;
       const int64_t slice_off = static_cast<int64_t>(slice) * pr.split_stride;
@@ -1208,22 +1187,12 @@ static int launch_pair(const GemmParams& P, cudaStream_t stream) {
   return LIREC_OK;
 }
 
-// Which kernel runs a launch.  LIREC_GEMM_PAIR=1 / 0 forces the CTA-pair (256-row tiles over two SMs) or
-// the single-CTA 128x128 kernel; unset = choose per launch.  The pair kernel is the fast one per tile,
-// but at small row counts (the reference's 64-clip batches: ~530 candidate rows = 3 pair tiles per
-// column of tiles) its tiles cover under 60 % of the 74 clusters while the same launch cut into
-// 128x128 tiles still fits one wave of the 148 SMs: then the single-CTA kernel finishes sooner.
-static int pair_mode() {
-  static int v = -2;
-  if (v == -2) {
-    const char* e = getenv("LIREC_GEMM_PAIR");
-    v = (e == nullptr || e[0] == '\0') ? -1 : (e[0] == '0' ? 0 : 1);
-  }
-  return v;
-}
+// Which kernel runs a launch: the CTA-pair kernel (256-row tiles over two SMs) or the single-CTA 128x128
+// kernel.  The pair kernel is the fast one per tile, but at small row counts (the reference's 64-clip
+// batches: ~530 candidate rows = 3 pair tiles per column of tiles) its tiles cover under 60 % of the 74
+// clusters while the same launch cut into 128x128 tiles still fits one wave of the 148 SMs: then the
+// single-CTA kernel finishes sooner.
 static bool choose_pair_kernel(const lirec_gemm_problem* probs, int nprobs) {
-  const int mode = pair_mode();
-  if (mode >= 0) return mode != 0;
   long pair_tiles = 0, single_tiles = 0;
   for (int i = 0; i < nprobs; ++i) {
     const lirec_gemm_problem& g = probs[i];

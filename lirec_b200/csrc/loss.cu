@@ -518,15 +518,8 @@ extern "C" int lirec_predict_tracks(const float* ints, const float* rels, const 
 
 extern "C" int lirec_adam_flat(float* param, const float* grad, float* exp_avg, float* exp_avg_sq,
                                void* param_bf16, int64_t n, float lr, float beta1, float beta2, float eps,
-                               float weight_decay, int32_t step, float grad_scale, void* stream) {
-  return lirec_adam_flat_ex(param, grad, exp_avg, exp_avg_sq, param_bf16, n, lr, beta1, beta2, eps, weight_decay,
-                            step, grad_scale, 0, stream);
-}
-
-extern "C" int lirec_adam_flat_ex(float* param, const float* grad, float* exp_avg, float* exp_avg_sq,
-                                  void* param_bf16, int64_t n, float lr, float beta1, float beta2, float eps,
-                                  float weight_decay, int32_t step, float grad_scale, int32_t coresident,
-                                  void* stream) {
+                               float weight_decay, int32_t step, float grad_scale, int32_t coresident,
+                               void* stream) {
   LIREC_ENTER();
   LIREC_REQUIRE(param && grad && exp_avg && exp_avg_sq && n >= 0 && step >= 1, "adam: bad arguments");
   if (n == 0) return LIREC_OK;

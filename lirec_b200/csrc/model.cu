@@ -378,7 +378,7 @@ static int weight_transposes(const Dims& d, const lirec_model_params& P, const W
 // The copies only depend on the weights, which are final when forward starts: a TRAINING forward launches them on
 // a side stream of the library's own, next to the forward GEMMs, and leaves a note for the backward call on the
 // same workspace, which then just waits for them (29 us off the critical path of a 1024-clip step).  A backward
-// without that note (eval-mode autograd, another workspace) transposes inline as before.
+// without that note (eval-mode autograd, another workspace) transposes inline.
 static int context_ref_tables(const Dims& d, const lirec_batch& B, const Workspace& w, cudaStream_t stream) {
   rows::RefTableJobs rj;
   for (int y = 0; y < 3; ++y) {
@@ -408,8 +408,6 @@ static bool side_ready() {
   int dev = -1;
   if (cudaGetDevice(&dev) != cudaSuccess) return false;
   if (g_side.stream && g_side.device == dev) return true;
-  const char* e = getenv("LIREC_SIDE_TRANSPOSE");
-  if (e && e[0] == '0') return false;
   if (g_side.stream) return false;   // created for another device: keep it simple, inline on this one
   if (cudaStreamCreateWithFlags(&g_side.stream, cudaStreamNonBlocking) != cudaSuccess) return false;
   if (cudaEventCreateWithFlags(&g_side.in, cudaEventDisableTiming) != cudaSuccess ||
@@ -647,11 +645,6 @@ static void add_dgrad_passes_inplace(lirec_gemm_problem& g, const TGrad& dy, int
   add_pass(g, mk_pass(a, 0, dy.hi, b, in_off, 0, out_f));
   add_pass(g, mk_pass(a, 0, dy.lo, b, in_off, 0, out_f));
 }
-// LIREC_DEFER_REDUCTIONS=0 keeps every parameter-gradient reduction in the launch of its own stage (A/B knob).
-static bool defer_reductions() {
-  const char* e = getenv("LIREC_DEFER_REDUCTIONS");
-  return !(e && e[0] == '0');
-}
 static void out_split_t(lirec_gemm_problem& g, bf16* out, int64_t pitch, int row_off, int lo_off) {
   g.epi.out_kind = LIREC_OUT_SPLIT_BF16_T;
   g.epi.out = out; g.epi.out_ld_m = pitch; g.epi.out_col_off = row_off; g.epi.out_lo_off = lo_off;
@@ -746,8 +739,7 @@ int backward(const lirec_model_cfg& cfg, const lirec_model_params& P, const lire
   // where their long memory-bound reductions (the [101, 3072] gradient streams the whole gate output) fill the
   // schedule next to the gate's compute-bound tiles instead of stretching this short launch.
   std::vector<lirec_gemm_problem> pr, head_red;
-  const bool defer_heads = d.gates && defer_reductions();
-  std::vector<lirec_gemm_problem>& hr = defer_heads ? head_red : pr;
+  std::vector<lirec_gemm_problem>& hr = d.gates ? head_red : pr;
   if (d.ints) {
     push_reduction(hr, wgrad_t(d.C, hw, dli, hx, 2 * hw, 2 * hw, 0, hw, Ni, 1.f, P.out_ints.grad_w, hw), d.C, hw, Ni,
                    true, sc);
@@ -825,17 +817,15 @@ int backward(const lirec_model_cfg& cfg, const lirec_model_params& P, const lire
   // scatter-reduce of this stage's DATA gradients), leaving this launch the eight short data-gradient GEMMs.
   pr.clear();
   std::vector<lirec_gemm_problem> l2_red;
-  const bool defer_l2 = defer_reductions();
-  std::vector<lirec_gemm_problem>& lr = defer_l2 ? l2_red : pr;
   for (int br = d.br0; br < nbr; ++br) {
     const lirec_encoder& enc = br ? P.enc_ctx : P.enc_ints;
     for (int s = 0; s < 4; ++s) {
       if (!d.act[s]) continue;
       const TGrad dz{w.dz2T[br], 2 * F, NiP, d.cs[s], F + d.cs[s]};
-      push_reduction(lr, wgrad_t(d.outw[s], J, dz, w.a2[br], 8 * J, 8 * J, s * 2 * J, s * 2 * J + J, Ni, keep_scale,
-                                 enc.l2[s].grad_w, J), d.outw[s], J, Ni, true, sc);
-      push_reduction(lr, bgrad_t(d.outw[s], dz, br ? w.flagT : w.onesT, Ni, enc.l2[s].grad_b), d.outw[s], 1, Ni,
-                     false, sc);
+      push_reduction(l2_red, wgrad_t(d.outw[s], J, dz, w.a2[br], 8 * J, 8 * J, s * 2 * J, s * 2 * J + J, Ni,
+                                     keep_scale, enc.l2[s].grad_w, J), d.outw[s], J, Ni, true, sc);
+      push_reduction(l2_red, bgrad_t(d.outw[s], dz, br ? w.flagT : w.onesT, Ni, enc.l2[s].grad_b), d.outw[s], 1,
+                     Ni, false, sc);
       lirec_gemm_problem g = mk_problem(Ni, J, true, false);
       if (inplace) add_dgrad_passes_inplace(g, dz, Ni, enc.l2[s].w_bf16, d.outw[s], J, 0);
       else add_dgrad_passes(g, dz, Ni, w.l2T[br][s], J, d.outw[s], 0, d.outw[s]);
@@ -950,16 +940,7 @@ extern "C" int lirec_model_forward(const lirec_model_cfg* cfg, const lirec_model
 
 extern "C" int lirec_model_backward(const lirec_model_cfg* cfg, const lirec_model_params* params,
                                     const lirec_batch* batch, void* workspace, size_t workspace_bytes,
-                                    const float* d_ints, const float* d_rels, void* stream) {
-  LIREC_ENTER();
-  int rc = model::validate(cfg, params, batch, workspace, workspace_bytes);
-  if (rc != LIREC_OK) return rc;
-  return model::backward(*cfg, *params, *batch, workspace, d_ints, d_rels, static_cast<cudaStream_t>(stream), nullptr);
-}
-
-extern "C" int lirec_model_backward_ex(const lirec_model_cfg* cfg, const lirec_model_params* params,
-                                       const lirec_batch* batch, void* workspace, size_t workspace_bytes,
-                                       const float* d_ints, const float* d_rels, void* stream, void* heads_event) {
+                                    const float* d_ints, const float* d_rels, void* stream, void* heads_event) {
   LIREC_ENTER();
   int rc = model::validate(cfg, params, batch, workspace, workspace_bytes);
   if (rc != LIREC_OK) return rc;

@@ -256,26 +256,8 @@ ref_tables_kernel(const RefTableJobs jobs) {
 constexpr int EBT_ROWS = 64;
 constexpr int EBT_COLS = 64;
 constexpr int EBT_REFS = 1536;
-#ifndef LIREC_EBT_ZSPLIT
-#define LIREC_EBT_ZSPLIT 4
-#endif
-constexpr int EBT_ZSPLIT = LIREC_EBT_ZSPLIT;   // references cached in shared memory per CTA (the rest is read in place)
-#ifndef LIREC_EBT_PREFETCH
-#define LIREC_EBT_PREFETCH 1
-#endif
-#ifndef LIREC_EBT_MIN_BLOCKS
-#define LIREC_EBT_MIN_BLOCKS 4
-#endif
-// A/B knob (undefined = what ships): references of a unique row walked N at a time, so the row gathers of
-// consecutive references are in flight together (tools/build_variants.sh builds the alternatives)
-#define LIREC_PRAGMA_(x) _Pragma(#x)
-#define LIREC_PRAGMA_UNROLL(n) LIREC_PRAGMA_(unroll n)
-#ifdef LIREC_EBT_UNROLL
-#define LIREC_EBT_UNROLL_PRAGMA LIREC_PRAGMA_UNROLL(LIREC_EBT_UNROLL)
-#else
-#define LIREC_EBT_UNROLL_PRAGMA     /* default: the compiler's own choice, as shipped and measured */
-#endif
-__global__ void __launch_bounds__(256, LIREC_EBT_MIN_BLOCKS)
+constexpr int EBT_ZSPLIT = 4;
+__global__ void __launch_bounds__(256, 4)
 expand_bwd_t_kernel(const ExpandBwdJobs jobs) {
   pdl_wait();
   pdl_trigger();
@@ -329,7 +311,6 @@ expand_bwd_t_kernel(const ExpandBwdJobs jobs) {
     const int j = c0 + q4;
     uint2 gate = make_uint2(0u, 0u);       // issued ahead of the reference loop (c0 % 64 == 0: 8-byte aligned)
     if (live && jb.sign) gate = *reinterpret_cast<const uint2*>(jb.sign + static_cast<int64_t>(u) * jb.sign_ld + (c0 >> 5));
-#if LIREC_EBT_PREFETCH
     // Latency hiding without registers: the ReLU gate of this chunk (read after the reference loop) and the
     // gradient pieces of the NEXT chunk are pulled into L2 now; a row's 64 columns are two 128-byte lines, taken
     // by the first two lanes of its quad.
@@ -342,8 +323,6 @@ expand_bwd_t_kernel(const ExpandBwdJobs jobs) {
             prefetch_l2(jb.d_in + static_cast<int64_t>(ref_out[q - q0]) * jb.d_ld + c0 + EBT_COLS + half);
       }
     }
-#endif
-    LIREC_EBT_UNROLL_PRAGMA
     for (int q = beg; q < end; ++q) {
       int i, o;
       float w;
@@ -698,20 +677,6 @@ gather_rows_kernel(const uint4* __restrict__ bank, int64_t bank_ld16, int n_bank
   }
 }
 
-__global__ void __launch_bounds__(256)
-gather_rows_flat_kernel(const uint4* __restrict__ bank, int64_t bank_ld16, int n_bank, const int32_t* __restrict__ idx,
-                        int n, int cols16, uint4* __restrict__ out, int64_t out_ld16) {
-  const int64_t total = static_cast<int64_t>(n) * cols16;
-  for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < total;
-       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-    const int r = static_cast<int>(i / cols16), c = static_cast<int>(i - static_cast<int64_t>(r) * cols16);
-    const int src = idx[r];
-    uint4 v = make_uint4(0u, 0u, 0u, 0u);
-    if (src >= 0 && src < n_bank) v = bank[static_cast<int64_t>(src) * bank_ld16 + c];   // out of range -> zero row
-    out[static_cast<int64_t>(r) * out_ld16 + c] = v;
-  }
-}
-
 // ---------------------------------------------------------------------------
 // host launchers
 // ---------------------------------------------------------------------------
@@ -746,17 +711,9 @@ int gather_rows(const void* bank, int64_t bank_ld, int n_bank, const int32_t* id
   LIREC_REQUIRE(bank && idx && out && n_bank > 0, "gather_rows: null argument");
   if (n <= 0) return LIREC_OK;
   const int cols16 = dim / 8;
-  const char* flat = getenv("LIREC_GATHER_FLAT");                // A/B knob: the element-strided form
-  if (flat && flat[0] == '1') {
-    const int64_t total = static_cast<int64_t>(n) * cols16;
-    const int grid = static_cast<int>(std::min<int64_t>((total + 255) / 256, 148 * 16));
-    gather_rows_flat_kernel<<<grid, 256, 0, stream>>>(static_cast<const uint4*>(bank), bank_ld / 8, n_bank, idx, n,
-                                                      cols16, static_cast<uint4*>(out), out_ld / 8);
-  } else {
-    const int grid = std::min((n + 7) / 8, 148 * 16);            // eight rows (warps) per CTA
-    gather_rows_kernel<<<grid, 256, 0, stream>>>(static_cast<const uint4*>(bank), bank_ld / 8, n_bank, idx, n, cols16,
-                                                 static_cast<uint4*>(out), out_ld / 8);
-  }
+  const int grid = std::min((n + 7) / 8, 148 * 16);              // eight rows (warps) per CTA
+  gather_rows_kernel<<<grid, 256, 0, stream>>>(static_cast<const uint4*>(bank), bank_ld / 8, n_bank, idx, n, cols16,
+                                               static_cast<uint4*>(out), out_ld / 8);
   LIREC_CUDA_OK(cudaGetLastError());
   note_launch();
   return LIREC_OK;
@@ -906,19 +863,10 @@ int cast_bf16(const float* x, void* out, int64_t n, cudaStream_t stream) {
 // ---------------------------------------------------------------------------
 using namespace lirec;
 
-extern "C" int lirec_seg_reduce_f32(const float* x, const int32_t* seg_off, int32_t nseg, int32_t dim,
-                                    int32_t mode, float* out_f32, int64_t out_f32_ld, void* out_bf16,
+extern "C" int lirec_seg_reduce_f32(const float* x, const int32_t* row_idx, const int32_t* seg_off, int32_t nseg,
+                                    int32_t dim, int32_t mode, float* out_f32, int64_t out_f32_ld, void* out_bf16,
                                     int64_t out_bf16_ld, void* stream) {
   LIREC_ENTER();
-  return rows::seg_reduce(x, seg_off, nseg, dim, mode, out_f32, out_f32_ld, out_bf16, out_bf16_ld,
-                          static_cast<cudaStream_t>(stream), nullptr);
-}
-
-extern "C" int lirec_seg_reduce_gather_f32(const float* x, const int32_t* row_idx, const int32_t* seg_off,
-                                           int32_t nseg, int32_t dim, int32_t mode, float* out_f32,
-                                           int64_t out_f32_ld, void* out_bf16, int64_t out_bf16_ld, void* stream) {
-  LIREC_ENTER();
-  LIREC_REQUIRE(row_idx != nullptr, "seg_reduce_gather: null row index");
   return rows::seg_reduce(x, seg_off, nseg, dim, mode, out_f32, out_f32_ld, out_bf16, out_bf16_ld,
                           static_cast<cudaStream_t>(stream), row_idx);
 }

@@ -18,8 +18,8 @@
 // Layout: one CTA of 128 threads per (segment, column group), one thread per four columns, the segment's rows
 // walked in batches of four (their loads issued together) with an online softmax in the base-2 domain (running
 // max, running normaliser, running weighted sum; one rescale per batch, no branch), so every global access is a
-// coalesced 16-byte load and the result is deterministic.  With few or long segments the CTA splits its rows over
-// four row lanes of 128 columns each and merges the lanes' states in a fixed order.  HBM-bound: forward reads x
+// coalesced 16-byte load and the result is deterministic.  The CTA splits its rows over four row lanes of 128
+// columns each and merges the lanes' states in a fixed order.  HBM-bound: forward reads x
 // (+ scores) once; backward reads x, scores, dy and the forward's log-normaliser once and writes dx (+ dscores) once.
 #include "rows.cuh"
 
@@ -43,6 +43,11 @@ constexpr float LOG2E = 1.4426950408889634f;
 constexpr float LN2 = 0.6931471805599453f;
 constexpr float M_EMPTY = -3.0e38f;      // running maximum of a column that has seen no row yet (finite: no inf - inf)
 constexpr int RB = 4;                    // rows per batch: their loads are issued together
+// Row lanes per CTA.  Measured on a B200 (profiles/r02_stress_sweep.txt): four row lanes of 128 columns tie with one
+// lane of 512 columns on many short segments (2048 segments of ~32 rows, dim 2048: 79 vs 81 % of the HBM peak) and
+// win everywhere else (dim 768: 74 vs 68 %, 512 segments of ~512 rows: 93 vs 80 %).
+constexpr int LANES = 4;
+constexpr int TPR = 128 / LANES;         // threads per row lane, four columns each
 
 // Online softmax-weighted sum of one column, base-2 domain: t = beta * log2(e) * score.  A batch of RB rows is
 // folded with ONE rescale of the running sums (RB + 1 ex2 per RB elements, no branch): with one row per update and
@@ -76,15 +81,13 @@ struct Online {
 };
 
 // One CTA of 128 threads per (segment, column group).  LANES row lanes share the CTA: lane l walks rows
-// beg + l, beg + l + LANES, ... over (128 / LANES) * 4 columns and the lanes' partial states are merged through
-// shared memory in lane order.  LANES = 1 (512 columns per CTA) when the grid fills the machine anyway, LANES = 4
-// (128 columns per CTA, four times the CTAs, a quarter of the dependent chain) for few / long segments.
+// beg + l, beg + l + LANES, ... over TPR * 4 columns and the lanes' partial states are merged through
+// shared memory in lane order.
 // MODE: 0 = score is x, 1 = per-element tensor [total, dim], 2 = one score per row [total].
-template <int LANES, int MODE>
+template <int MODE>
 __global__ void __launch_bounds__(128)
 fwd_kernel(const float* __restrict__ x, const float* __restrict__ scores, const int32_t* __restrict__ seg_off, int dim,
            float beta, float* __restrict__ out, int64_t out_ld, float* __restrict__ lse, int64_t lse_ld) {
-  constexpr int TPR = 128 / LANES;
   const int seg = blockIdx.x;
   const int ct = threadIdx.x % TPR, lane = threadIdx.x / TPR;
   const int col = (blockIdx.y * TPR + ct) * 4;
@@ -146,21 +149,19 @@ fwd_kernel(const float* __restrict__ x, const float* __restrict__ scores, const 
 #pragma unroll
     for (int k = 1; k < 4; ++k) { o[k].m = o[0].m; o[k].z = o[0].z; }
   }
-  if (LANES > 1) {
-    __shared__ float part[LANES > 1 ? LANES - 1 : 1][12][LANES > 1 ? TPR : 1];
-    if (lane > 0) {
+  __shared__ float part[LANES - 1][12][TPR];
+  if (lane > 0) {
 #pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        part[lane - 1][3 * k][ct] = o[k].m; part[lane - 1][3 * k + 1][ct] = o[k].z; part[lane - 1][3 * k + 2][ct] = o[k].acc;
-      }
+    for (int k = 0; k < 4; ++k) {
+      part[lane - 1][3 * k][ct] = o[k].m; part[lane - 1][3 * k + 1][ct] = o[k].z; part[lane - 1][3 * k + 2][ct] = o[k].acc;
     }
-    __syncthreads();
-    if (lane > 0) return;
-#pragma unroll
-    for (int l = 0; l < LANES - 1; ++l)
-#pragma unroll
-      for (int k = 0; k < 4; ++k) o[k].merge(part[l][3 * k][ct], part[l][3 * k + 1][ct], part[l][3 * k + 2][ct]);
   }
+  __syncthreads();
+  if (lane > 0) return;
+#pragma unroll
+  for (int l = 0; l < LANES - 1; ++l)
+#pragma unroll
+    for (int k = 0; k < 4; ++k) o[k].merge(part[l][3 * k][ct], part[l][3 * k + 1][ct], part[l][3 * k + 2][ct]);
   if (!live) return;
   float4 y = make_float4(0.f, 0.f, 0.f, 0.f), l = make_float4(0.f, 0.f, 0.f, 0.f);
   if (end > beg) {
@@ -180,13 +181,12 @@ fwd_kernel(const float* __restrict__ x, const float* __restrict__ scores, const 
 
 // Backward, per-element scores (score_mode 0 / 1), same CTA shape as the forward (no merge: rows are independent):
 //   w = exp(beta * s - lse);  dx = w * dy (+ ds when score is x);  ds = beta * w * (x - y) * dy
-template <int LANES, int MODE>
+template <int MODE>
 __global__ void __launch_bounds__(128)
 bwd_elem_kernel(const float* __restrict__ x, const float* __restrict__ scores, const int32_t* __restrict__ seg_off,
                 int dim, float beta, const float* __restrict__ y, int64_t y_ld, const float* __restrict__ lse,
                 int64_t lse_ld, const float* __restrict__ dy, int64_t dy_ld, float* __restrict__ dx,
                 float* __restrict__ dscores, int64_t total_rows) {
-  constexpr int TPR = 128 / LANES;
   const int seg = blockIdx.x;
   const int ct = threadIdx.x % TPR, lane = threadIdx.x / TPR;
   const int col = (blockIdx.y * TPR + ct) * 4;
@@ -312,14 +312,6 @@ bwd_row_kernel(const float* __restrict__ x, const float* __restrict__ scores, co
   }
 }
 
-// CTA shape.  Measured on a B200 (profiles/r02_stress_sweep.txt; tools/stress_sweep.py with LIREC_SP_LANES=1 / 4):
-// four row lanes of 128 columns tie with one lane of 512 columns on many short segments (2048 segments of ~32 rows,
-// dim 2048: 79 vs 81 % of the HBM peak) and win everywhere else (dim 768: 74 vs 68 %, 512 segments of ~512 rows: 93 vs
-// 80 %), so four lanes are the default; LIREC_SP_LANES=1 keeps the single-lane shape for A/B runs.
-static bool few_ctas(int, int) {
-  const char* e = getenv("LIREC_SP_LANES");      // read per call: the tests switch it
-  return !(e && atoi(e) == 1);
-}
 // row chunks per segment of the per-row-score backward: enough CTAs for ~8 per SM
 static int row_chunks(int nseg) {
   static int sms = 0;
@@ -360,15 +352,11 @@ extern "C" int lirec_seg_softmax_pool_fwd(const float* x, const float* scores, i
                 "seg_softmax_pool_fwd: lse not 16-byte aligned");
   if (nseg <= 0) return LIREC_OK;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-#define LIREC_SP_FWD(L, M)                                                                                       \
-  softpool::fwd_kernel<L, M><<<dim3(nseg, (dim / 4 + 128 / L - 1) / (128 / L)), 128, 0, s>>>(x, scores, seg_off, dim, \
-                                                                                             beta, out, out_ld, lse, lse_ld)
-  if (softpool::few_ctas(nseg, dim)) {
-    if (score_mode == 0) LIREC_SP_FWD(4, 0); else if (score_mode == 1) LIREC_SP_FWD(4, 1); else LIREC_SP_FWD(4, 2);
-  } else {
-    if (score_mode == 0) LIREC_SP_FWD(1, 0); else if (score_mode == 1) LIREC_SP_FWD(1, 1); else LIREC_SP_FWD(1, 2);
-  }
-#undef LIREC_SP_FWD
+  auto kernel = score_mode == 0   ? softpool::fwd_kernel<0>
+                : score_mode == 1 ? softpool::fwd_kernel<1>
+                                  : softpool::fwd_kernel<2>;
+  kernel<<<dim3(nseg, (dim / 4 + softpool::TPR - 1) / softpool::TPR), 128, 0, s>>>(x, scores, seg_off, dim, beta, out,
+                                                                                  out_ld, lse, lse_ld);
   LIREC_CUDA_OK(cudaGetLastError());
   note_launch();
   return LIREC_OK;
@@ -401,15 +389,9 @@ extern "C" int lirec_seg_softmax_pool_bwd(const float* x, const float* scores, i
     LIREC_REQUIRE((reinterpret_cast<uintptr_t>(lse) & 15) == 0 && lse_ld % 4 == 0 &&
                       (!d_scores || (reinterpret_cast<uintptr_t>(d_scores) & 15) == 0),
                   "seg_softmax_pool_bwd: lse / d_scores not 16-byte aligned");
-#define LIREC_SP_BWD(L, M)                                                                                       \
-  softpool::bwd_elem_kernel<L, M><<<dim3(nseg, (dim / 4 + 128 / L - 1) / (128 / L)), 128, 0, s>>>(                \
-      x, scores, seg_off, dim, beta, out, out_ld, lse, lse_ld, d_out, d_out_ld, d_x, d_scores, total_rows)
-    if (softpool::few_ctas(nseg, dim)) {
-      if (score_mode == 0) LIREC_SP_BWD(4, 0); else LIREC_SP_BWD(4, 1);
-    } else {
-      if (score_mode == 0) LIREC_SP_BWD(1, 0); else LIREC_SP_BWD(1, 1);
-    }
-#undef LIREC_SP_BWD
+    auto kernel = score_mode == 0 ? softpool::bwd_elem_kernel<0> : softpool::bwd_elem_kernel<1>;
+    kernel<<<dim3(nseg, (dim / 4 + softpool::TPR - 1) / softpool::TPR), 128, 0, s>>>(
+        x, scores, seg_off, dim, beta, out, out_ld, lse, lse_ld, d_out, d_out_ld, d_x, d_scores, total_rows);
   }
   LIREC_CUDA_OK(cudaGetLastError());
   note_launch();

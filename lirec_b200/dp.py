@@ -82,14 +82,14 @@ class SwitchReduceAdam:
     mode 'shard' (default): lirec_dp_reduce_adam_bcast — every rank sums its 1/world shard of the gradients inside
     the switch, applies Adam to that shard (it owns the shard's moments) and multicast-stores the new fp32
     parameters and their bf16 shadow into every replica.  With `overlap` the pass is split in two: the gate +
-    head parameters (53 %) run on a side stream behind the event lirec_model_backward_ex records when their
+    head parameters (53 %) run on a side stream behind the event lirec_model_backward records when their
     gradients are final, while the encoder stages of backward still go; the encoders follow after backward.  Parameters, bf16 shadow
     and gradients therefore live in ONE symmetric allocation; `optimizer.state_dict()` gathers the moments.
     Against exchange-then-Adam this removes the 553 MB full-replica optimizer pass from every rank's critical
     path and sends 6 bytes per parameter back instead of 4.
 
     mode 'bucket': the gradient sum (lirec_dp_exchange) and a full-replica lirec_adam_flat per bucket, the
-    gate + head bucket on a side stream behind the event lirec_model_backward_ex records when those gradients
+    gate + head bucket on a side stream behind the event lirec_model_backward records when those gradients
     are final (measured: the overlap buys < 1 % — the overlapped Adam pass competes with the L2-bound encoder
     stages for the same memory system — and the exchange alone is slower than NCCL's at 2 ranks).
 
@@ -228,7 +228,7 @@ class SwitchReduceAdam:
 
     # ---- per-step protocol --------------------------------------------------------------------------
     def arm(self, equal_shards=True):
-        """Before backward: ask lirec_model_backward_ex for the heads-final event (only when this step's exchange
+        """Before backward: ask lirec_model_backward for the heads-final event (only when this step's exchange
         needs no host-side re-weighting)."""
         self._armed = bool(self.overlap and equal_shards and 0 < self.split < self.n)
         self.model._heads_event = self.ev_heads if self._armed else None

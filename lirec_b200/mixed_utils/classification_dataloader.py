@@ -21,8 +21,6 @@ without `opt.synthetic` the dataset refuses to construct instead of pretending.
                   MovieGraphs annotations would take; `--resident_banks 1` keeps the split's pooled feature
                   banks in HBM so a batch ships only index tables.
 """
-import os
-
 import torch
 from torch.utils.data import Dataset
 
@@ -230,32 +228,6 @@ def _threaded_batches(dataset, batches, num_threads, batch_size, slots_ahead):
         pool.shutdown(wait=True, cancel_futures=True)
 
 
-_MALLOC_TUNED = False
-
-
-def _tune_malloc():
-    """Keep the loader's per-batch temporaries (index arrays of a few MB, allocated and freed once per batch by
-    several threads) inside glibc's heaps instead of a fresh mmap / munmap pair each: above the default 128 KB
-    threshold every such array is new anonymous memory that has to be faulted in page by page — and on a freshly
-    started VM every never-touched guest page is a round trip to the hypervisor, seen as sporadic 20-100 ms waits
-    for a batch during the first minutes of a process.  OPT-IN (LIREC_MALLOPT=1): four A/B runs on two fresh boxes
-    showed the stalls with and without it (they also hit legs that never allocate host memory), so the default
-    leaves the allocator alone."""
-    global _MALLOC_TUNED
-    if _MALLOC_TUNED or os.environ.get("LIREC_MALLOPT", "0") != "1":
-        return
-    _MALLOC_TUNED = True
-    try:
-        import ctypes
-        libc = ctypes.CDLL(None)
-        M_TRIM_THRESHOLD, M_TOP_PAD, M_MMAP_THRESHOLD = -1, -2, -3
-        libc.mallopt(M_MMAP_THRESHOLD, 1 << 30)
-        libc.mallopt(M_TRIM_THRESHOLD, (1 << 31) - 1)
-        libc.mallopt(M_TOP_PAD, 256 << 20)
-    except Exception:
-        pass
-
-
 def packed_loader(dataset, batch_size, shuffle, num_workers=0, device="cuda", rank=0, world=1, drop_last=False,
                   seed=0, repeat=1):
     """Iterate device-resident PackedBatches with one-batch-ahead async H2D prefetch.
@@ -264,7 +236,6 @@ def packed_loader(dataset, batch_size, shuffle, num_workers=0, device="cuda", ra
     global batch (lirec_b200/dp.py:shard_range), so the global batch equals the single-GPU one.  A rank whose
     share is empty receives an `EmptyShard` for that step (see there).  `repeat` > 1 chains that many epochs
     (each its own permutation) behind ONE set of worker processes instead of re-forking them per epoch."""
-    _tune_malloc()
     g = torch.Generator()
     g.manual_seed(int(seed) * 1000003 + int(getattr(dataset, "epoch", 0)))
     n = len(dataset)
@@ -274,13 +245,11 @@ def packed_loader(dataset, batch_size, shuffle, num_workers=0, device="cuda", ra
         batches += plan_batches(n, batch_size, order, rank, world, drop_last)
     if int(num_workers) > 0 and hasattr(dataset, "warm_records"):
         dataset.warm_records()              # workers fork with the record cache already built
-    # worker processes build the batches (items + native collate); with workers the DataLoader's own pinning
-    # thread calls PackedBatch.pin_memory(), so the training thread only issues the async copies
+    # worker processes build the batches (items + native collate)
     group = max(1, min(16, 512 // max(int(batch_size) // max(world, 1), 1))) if int(num_workers) > 0 else 1
     loader = torch.utils.data.DataLoader(_IndexView(dataset, batches, group), batch_size=None, shuffle=False,
                                          num_workers=int(num_workers), collate_fn=None,
-                                         pin_memory=(int(num_workers) > 0 and
-                                                     os.environ.get("LIREC_LOADER_PIN_THREAD", "0") != "0"),
+                                         pin_memory=False,
                                          prefetch_factor=(int(getattr(opt, "prefetch_factor", 2)) if int(num_workers) > 0
                                                           else None),
                                          persistent_workers=False)
@@ -292,7 +261,7 @@ def packed_loader(dataset, batch_size, shuffle, num_workers=0, device="cuda", ra
         banks = getattr(dataset, "_resident", None) or ResidentBanks(dataset, device)
         dataset._resident = banks
         copy_stream.wait_stream(torch.cuda.current_stream())
-    ring = _PinnedRing() if (banks is not None and os.environ.get("LIREC_LOADER_RING", "1") != "0") else None
+    ring = _PinnedRing() if banks is not None else None
 
     def flat(it):
         for item in it:
@@ -304,7 +273,7 @@ def packed_loader(dataset, batch_size, shuffle, num_workers=0, device="cuda", ra
 
     # datasets whose batches are assembled by GIL-free native code (get_batch): worker THREADS, pinned from birth
     threaded = (int(num_workers) > 0 and banks is not None and hasattr(dataset, "get_batch") and
-                hasattr(dataset, "arena_bound") and os.environ.get("LIREC_LOADER_THREADS", "1") != "0")
+                hasattr(dataset, "arena_bound"))
     if threaded:
         if getattr(dataset, "records", 1) is None:
             dataset.cache()
@@ -322,8 +291,7 @@ def packed_loader(dataset, batch_size, shuffle, num_workers=0, device="cuda", ra
             pending = (dev_pb, ev)
             continue
         with torch.cuda.stream(copy_stream):
-            if banks is not None and ring is not None and getattr(host_pb, "_host_arena", None) is not None \
-                    and not hasattr(host_pb, "_arena"):
+            if ring is not None and getattr(host_pb, "_host_arena", None) is not None and not hasattr(host_pb, "_arena"):
                 dev_pb = banks.stage(ring.stage(host_pb, copy_stream))
                 ring.mark(copy_stream)
             else:

@@ -25,8 +25,6 @@ objects those loaders return (`source`), e.g. from mixed_utils/synthetic_world.p
 from collections import defaultdict
 from itertools import permutations
 
-import os
-
 import numpy as np
 import torch
 from torch.utils.data import Dataset
@@ -648,10 +646,8 @@ def collate_indexed(records, dataset, resident=False):
     left out and `pb.extras['bank_rows']` lists the dataset-bank rows to gather on the device.
 
     The integer tables are built by the native `lirec_collate_tables` (csrc/collate.cu; host code, safe in
-    DataLoader workers) straight into one int32 arena; `LIREC_NATIVE_COLLATE=0` selects the numpy
-    statement of the same tables (`collate_indexed_numpy`, which the tests hold the native one to)."""
-    if os.environ.get("LIREC_NATIVE_COLLATE", "1") == "0":
-        return collate_indexed_numpy(records, dataset, resident=resident)
+    DataLoader workers) straight into one int32 arena; `collate_indexed_numpy` states the same tables in
+    numpy, and the tests hold the native one to it."""
     from lirec_b200 import _ext
     L = _ext.lib()
     B = len(records)
@@ -852,7 +848,7 @@ class ResidentBanks:
         if key not in warmed:
             warmed.add(key)
             hold = [torch.empty(caps[which], dim, dtype=torch.bfloat16, device=self.device)
-                    for _ in range(int(os.environ.get("LIREC_BANK_POOL_DEPTH", "6")))]
+                    for _ in range(6)]
             del hold
         return torch.empty(caps[which], dim, dtype=torch.bfloat16, device=self.device)[:n]
 

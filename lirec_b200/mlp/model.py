@@ -365,14 +365,9 @@ class _HotPath(nn.Module):
             d_rels = d_rels.contiguous()
             d_rels_ptr = d_rels.data_ptr()
         ev = getattr(self, "_heads_event", None)       # set by dp.SwitchReduceAdam.arm(): overlap bucket 0
-        if ev is not None:
-            _ext.check(_ext.lib().lirec_model_backward_ex(
-                C.byref(self._cfg_c), C.byref(self._params_c), C.byref(batch_c), ws.data_ptr(), ws.numel(),
-                d_inters_ptr, d_rels_ptr, _ext.stream_ptr(), C.c_void_p(ev.cuda_event)))
-        else:
-            _ext.check(_ext.lib().lirec_model_backward(
-                C.byref(self._cfg_c), C.byref(self._params_c), C.byref(batch_c), ws.data_ptr(), ws.numel(),
-                d_inters_ptr, d_rels_ptr, _ext.stream_ptr()))
+        _ext.check(_ext.lib().lirec_model_backward(
+            C.byref(self._cfg_c), C.byref(self._params_c), C.byref(batch_c), ws.data_ptr(), ws.numel(),
+            d_inters_ptr, d_rels_ptr, _ext.stream_ptr(), C.c_void_p(ev.cuda_event) if ev is not None else None))
         self._publish_grads()
 
     # ---- batches -------------------------------------------------------------------------------

@@ -64,16 +64,9 @@ def seg_reduce(x, seg_off, mode="max", out_f32=None, out_bf16=None, row_idx=None
     assert x.dtype == torch.float32 and x.dim() == 2 and x.is_contiguous()
     assert seg_off.dtype == torch.int32
     nseg = seg_off.numel() - 1
-    L = _ext.lib()
-    if row_idx is not None:
-        assert row_idx.dtype == torch.int32
-        _ext.check(L.lirec_seg_reduce_gather_f32(
-            _ext.ptr(x), _ext.ptr(row_idx), _ext.ptr(seg_off), nseg, x.shape[1], 0 if mode == "max" else 1,
-            _ext.ptr(out_f32), out_f32.stride(0) if out_f32 is not None else 0,
-            _ext.ptr(out_bf16), out_bf16.stride(0) if out_bf16 is not None else 0, _ext.stream_ptr()))
-        return
-    _ext.check(L.lirec_seg_reduce_f32(
-        _ext.ptr(x), _ext.ptr(seg_off), nseg, x.shape[1], 0 if mode == "max" else 1,
+    assert row_idx is None or row_idx.dtype == torch.int32
+    _ext.check(_ext.lib().lirec_seg_reduce_f32(
+        _ext.ptr(x), _ext.ptr(row_idx), _ext.ptr(seg_off), nseg, x.shape[1], 0 if mode == "max" else 1,
         _ext.ptr(out_f32), out_f32.stride(0) if out_f32 is not None else 0,
         _ext.ptr(out_bf16), out_bf16.stride(0) if out_bf16 is not None else 0, _ext.stream_ptr()))
 
@@ -258,12 +251,12 @@ def adam_flat(param, grad, exp_avg, exp_avg_sq, param_bf16, lr, beta1, beta2, ep
     L = _ext.lib()
     n = param.numel() - offset if n is None else n
     sp = _ext.stream_ptr() if stream is None else C.c_void_p(stream.cuda_stream)
-    _ext.check(L.lirec_adam_flat_ex(_ext.ptr(param) + 4 * offset, _ext.ptr(grad) + 4 * offset,
+    _ext.check(L.lirec_adam_flat(_ext.ptr(param) + 4 * offset, _ext.ptr(grad) + 4 * offset,
                                  _ext.ptr(exp_avg) + 4 * offset, _ext.ptr(exp_avg_sq) + 4 * offset,
                                  (_ext.ptr(param_bf16) + 2 * offset) if param_bf16 is not None else None, int(n),
                                  float(lr), float(beta1), float(beta2),
                                  float(eps), float(weight_decay), int(step), float(grad_scale), int(bool(coresident)),
-                                    sp))
+                                 sp))
 
 
 def dp_reduce_adam_bcast(grad_mc, param, param_mc, bf16_mc, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, weight_decay,

@@ -6,8 +6,8 @@ The reference walks the subtitle lines on the host, concatenates the token-index
 whose time span overlaps the clip (`Time.includes`, :24-31), indexes the `[n_tokens, 768]` feature array
 with that list and takes np.max; a clip without dialog gets a zero row (:171-178).  Here the token
 features are uploaded once, the index lists of as many clips as are queued are concatenated, and ONE
-gathered segmented-max launch (`lirec_seg_reduce_gather_f32`) writes the pooled bf16 rows.  WebVTT / token
-file parsing stays outside: the constructor takes the arrays.
+gathered segmented-max launch (`lirec_seg_reduce_f32` with a row index) writes the pooled bf16 rows.
+WebVTT / token file parsing stays outside: the constructor takes the arrays.
 """
 import numpy as np
 import torch

@@ -25,10 +25,12 @@ def test_header_symbols_exported(built_lib):
         assert hasattr(lib, name), "include/lirec_b200.h declares %s but the library does not export it" % name
 
 
-def test_binding_lists_every_symbol(built_lib):
+def test_binding_lists_every_symbol_of_abi_version_2(built_lib):
+    """Version 2: one entry point per operation (lirec_model_backward takes the nullable heads event,
+    lirec_adam_flat the coresident flag, lirec_seg_reduce_f32 the nullable row index)."""
     from lirec_b200 import _ext
     assert sorted(_ext.EXPORTED_SYMBOLS) == _declared_symbols()
-    assert _ext.lib().lirec_abi_version() == 1
+    assert _ext.lib().lirec_abi_version() == 2
 
 
 def test_sass_is_blackwell_native(built_lib):
@@ -157,7 +159,7 @@ def test_argtypes_arity_matches_the_header(built_lib):
         params = [p.strip() for p in params.split(",")] if params.strip() not in ("", "void") else []
         fn = getattr(L, name)
         if fn.argtypes is None:
-            assert not params or name in ("lirec_profile_begin", "lirec_dp_grid_size"), name
+            assert not params or name == "lirec_profile_begin", name
             continue
         assert len(fn.argtypes) == len(params), (name, len(fn.argtypes), params)
         for at, p in zip(fn.argtypes, params):

@@ -154,7 +154,7 @@ def test_flat_adam_matches_torch_adam():
 
 
 def test_coresident_adam_launch_shape_is_bit_identical():
-    """lirec_adam_flat_ex(coresident=1) — CTAs sized to share an SM with a resident GEMM CTA, used for the pass
+    """lirec_adam_flat(coresident=1) — CTAs sized to share an SM with a resident GEMM CTA, used for the pass
     overlapped with backward — is the same arithmetic on the same elements: bit-identical buffers, also on a
     sub-range and on a side stream."""
     from lirec_b200 import ops

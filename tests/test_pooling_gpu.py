@@ -76,8 +76,8 @@ def test_roi_pool_full_size_maps_against_numpy():
 
 
 def test_text_pooling_matches_the_reference():
-    """Gathered segmented max over dialog tokens (lirec_seg_reduce_gather_f32): bit-exact with np.max over the rows
-    the reference's unmodified TextFeatures returned; zero row for clips without dialog."""
+    """Gathered segmented max over dialog tokens (lirec_seg_reduce_f32 with a row index): bit-exact with np.max over
+    the rows the reference's unmodified TextFeatures returned; zero row for clips without dialog."""
     from test_pooling_cpu import load_text_world
     from lirec_b200.text_utils.text_features import TextFeatures
     g, meta, feats = load_text_world()
@@ -146,15 +146,12 @@ def _np_softpool_bwd(x, off, beta, scores, out, ws, dy):
     return dx, ds
 
 
-@pytest.mark.parametrize("lanes", ["4", "1"])
 @pytest.mark.parametrize("many", [False, True])
 @pytest.mark.parametrize("kind", ["self", "elem", "row"])
-def test_softmax_pool_forward_backward_vs_numpy(kind, many, lanes, monkeypatch):
-    """Both CTA shapes of the kernels (four row lanes of 128 columns merged in shared memory — the default — and one
-    lane of 512 columns, LIREC_SP_LANES=1), a handful of segments and thousands of them, ragged lengths around the
-    four-row batches and the row chunks of the per-row-score backward."""
+def test_softmax_pool_forward_backward_vs_numpy(kind, many):
+    """The kernels' CTA shape (four row lanes of 128 columns merged in shared memory), a handful of segments and
+    thousands of them, ragged lengths around the four-row batches and the row chunks of the per-row-score backward."""
     from lirec_b200 import ops
-    monkeypatch.setenv("LIREC_SP_LANES", lanes)
     rng = np.random.default_rng(3)
     lens = [5, 0, 1, 37, 12, 0, 64, 3]                       # ragged, with empty segments
     dim, beta = 768, 1.7

@@ -1,7 +1,7 @@
 #!/bin/bash
-# Build A/B variants of liblirec_b200.so into variants/<name>.so (git-ignored, travels with gpurun), then
-# restore the default build.  tools/ab_bench.sh runs the step bench for each of them on ONE box, interleaved:
-#   bash tools/build_variants.sh "name1:-DX=1 -DY=2" "name2:..." && gpurun --timeout 900 -- 'bash tools/ab_bench.sh'
+# Build instrumented variants of liblirec_b200.so into variants/<name>.so (git-ignored), then restore the default
+# build.  The one such variant is the in-kernel GEMM trace that tools/gemm_trace.py reads:
+#   bash tools/build_variants.sh "trace:-DLIREC_GEMM_TRACE=1"
 set -e
 cd "$(dirname "$0")/.."
 rm -rf variants

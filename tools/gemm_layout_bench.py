@@ -1,6 +1,6 @@
 """Throughput of the grouped tcgen05 GEMM by operand layout (K-major / MN-major), one problem per
 launch, against cuBLAS bf16 on the same shape.  Diagnostic; run on a B200:
-    python tools/gemm_layout_bench.py            (LIREC_GEMM_PAIR=0 selects the single-CTA kernel)"""
+    python tools/gemm_layout_bench.py"""
 import os
 import sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -46,7 +46,7 @@ def run(M, N, K, a_mn, b_mn, passes=1):
 
 
 if __name__ == "__main__":
-    print(torch.cuda.get_device_name(0), "pair" if os.environ.get("LIREC_GEMM_PAIR", "1") != "0" else "single")
+    print(torch.cuda.get_device_name(0))
     for (M, N, K) in [(8192, 3072, 6144), (8448, 3072, 3072), (3072, 1536, 8384)]:
         for a_mn, b_mn in [(False, False), (False, True), (True, False), (True, True)]:
             run(M, N, K, a_mn, b_mn)

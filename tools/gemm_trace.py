@@ -20,7 +20,7 @@ GHZ = float(os.environ.get("LIREC_TRACE_GHZ", "1.9"))
 
 def main():
     path = tempfile.mktemp(suffix=".trace")
-    env = dict(os.environ, LIREC_GEMM_TRACE_FILE=path, LIREC_PDL="0")
+    env = dict(os.environ, LIREC_GEMM_TRACE_FILE=path)
     args = sys.argv[1:] or ["--steps", "1", "--warmup", "3"]
     # warm-up steps are traced too: keep the LAST step's launches
     subprocess.run([sys.executable, os.path.join(HERE, "bench.py"), "--only_value"] + args, env=env, check=True,

@@ -2,7 +2,7 @@
 """Where does the overlapped pass really run?  One GPU, `--overlap_adam`-style step (gate + head bucket's Adam on
 a side stream behind the heads-final event of backward), with timing events on both streams:
 
-    t_heads   heads-final event (recorded mid-backward by lirec_model_backward_ex)
+    t_heads   heads-final event (recorded mid-backward by lirec_model_backward)
     t_a_done  end of the side-stream pass
     t_bwd     end of backward on the main stream (before the encoder bucket's Adam)
     t_end     end of the step
