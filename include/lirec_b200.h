@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define LIREC_ABI_VERSION 2
+#define LIREC_ABI_VERSION 3
 
 enum lirec_status {
   LIREC_OK = 0,
@@ -221,14 +221,15 @@ int lirec_rows_expand_fwd(const float* r1_txt, const float* r1_vis, const float*
  * owner : NULL (ints) or [n_rows] candidate index of each context row;
  * seg_off: NULL or [n_out+1] (context) to derive 1/n.
  * slot : 0 txt, 1 vis, 2 tr1, 3 tr2 (selects the dropout columns).
- * Writes dZ1 = [r1 > 0] * sum(...) as a hi/lo split [n_unique, 2*J] (out_t_pitch == 0),
- * or TRANSPOSED as [2*J, out_t_pitch] (hi rows [0,J), lo rows [J,2J); out_t_pitch >=
- * n_unique, a multiple of 8) — the K-major operand of the first-layer wgrad GEMM.   */
-int lirec_rows_expand_bwd(const float* d_in, int64_t d_ld, const float* r1, int32_t J,
-                          int32_t slot, const int32_t* inv_off, const int32_t* inv_idx,
+ * sign : ReLU gate [r1 > 0] of the unique rows as bits, in the LIREC_POST_SIGN_MASK layout: bit (j & 31)
+ *        of sign[u*sign_ld + (j >> 5)]; 8-byte aligned, sign_ld even and >= J/32 words.  J % 64 == 0.
+ * Writes dZ1 = [r1 > 0] * sum(...) TRANSPOSED as a hi/lo split [2*J, out_pitch] (hi rows [0,J),
+ * lo rows [J,2J); out_pitch >= n_unique, a multiple of 8; 16-byte aligned) — the K-major operand
+ * of the first-layer wgrad GEMM.                                                  */
+int lirec_rows_expand_bwd(const float* d_in, int64_t d_ld, const uint32_t* sign, int64_t sign_ld,
+                          int32_t J, int32_t slot, const int32_t* inv_off, const int32_t* inv_idx,
                           int32_t n_unique, const int32_t* owner, const int32_t* seg_off,
-                          lirec_dropout drop, void* out_split, int64_t out_ld,
-                          int64_t out_t_pitch, void* stream);
+                          lirec_dropout drop, void* out_split, int64_t out_pitch, void* stream);
 
 /* Spatial / person-box mean of I3D feature maps fused with the temporal max:
  *   out[s, c] = max over the elements e of segment s of mean(maps[frame_e, c, y0:y1, x0:x1]).
@@ -254,9 +255,10 @@ int lirec_roi_max_pool_f32(const float* maps, int32_t T, int32_t C, int32_t H, i
 int lirec_gather_rows(const void* bank, int64_t bank_ld, int32_t n_bank, const int32_t* idx,
                       int32_t n, int32_t dim, void* out, int64_t out_ld, void* stream);
 
-/* fp32 [rows, cols] -> hi/lo bf16 split [rows, 2*pad_cols] (zero padded). */
+/* fp32 [rows, cols] -> TRANSPOSED hi/lo bf16 split [2*pad, pitch]: hi at out_split[c*pitch + r],
+ * lo at out_split[(pad + c)*pitch + r]; rows c in [cols, pad) are zero (pad >= cols, pitch >= rows). */
 int lirec_split_f32(const float* x, int64_t ld, int32_t rows, int32_t cols, void* out_split,
-                    int64_t out_ld, int32_t pad_cols, void* stream);
+                    int64_t pitch, int32_t pad, void* stream);
 /* fp32 -> bf16 (round to nearest even), n elements. */
 int lirec_cast_bf16(const float* x, void* out, int64_t n, void* stream);
 

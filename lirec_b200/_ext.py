@@ -126,9 +126,9 @@ def lib():
     L.lirec_rows_expand_fwd.argtypes = [C.c_void_p] * 4 + [C.c_int32, C.c_void_p, C.c_void_p, C.c_int32,
                                                            C.c_int32, Dropout, C.c_void_p, C.c_int64,
                                                            C.c_void_p, C.c_void_p]
-    L.lirec_rows_expand_bwd.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_int32,
+    L.lirec_rows_expand_bwd.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int32, C.c_int32,
                                         C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
-                                        Dropout, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]
+                                        Dropout, C.c_void_p, C.c_int64, C.c_void_p]
     L.lirec_split_f32.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_int64,
                                   C.c_int32, C.c_void_p]
     L.lirec_roi_max_pool_f32.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32,
@@ -174,7 +174,7 @@ def lib():
                                        C.c_void_p]
     L.lirec_collate_gather.argtypes = [C.c_void_p] * 6 + [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                                           C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
-    if L.lirec_abi_version() != 2:
+    if L.lirec_abi_version() != 3:
         raise RuntimeError("liblirec_b200.so ABI version mismatch; rebuild it")
     _lib = L
     return L

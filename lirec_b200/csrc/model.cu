@@ -205,7 +205,7 @@ static Workspace carve(const Dims& d, void* base) {
   for (int br = 0; br < 2; ++br)
     for (int s = 0; s < 4; ++s) {
       w.sgn[br][s] = nullptr;
-      if (br >= d.br0 && br < nbr && d.act[s] && d.J % 64 == 0) {
+      if (br >= d.br0 && br < nbr && d.act[s]) {
         const int nu = (s < 2) ? (br ? d.nc : d.nci) : (br ? d.nt : d.nti);
         w.sgn[br][s] = static_cast<uint32_t*>(take((size_t)nu * (d.J / 32) * 4));
       }
@@ -464,11 +464,9 @@ int forward(const lirec_model_cfg& cfg, const lirec_model_params& P, const lirec
       g.epi.bias = enc.l1[s].bias;
       g.epi.act = LIREC_ACT_RELU;
       out_f32(g, w.r1[br][s], J);
-      if (w.sgn[br][s]) {                    // the gate of relu, 1 bit per element, for backward's scatter-reduce
-        g.epi.post = LIREC_POST_SIGN_MASK;
-        g.epi.aux = w.sgn[br][s];
-        g.epi.aux_ld = J / 32;
-      }
+      g.epi.post = LIREC_POST_SIGN_MASK;     // the gate of relu, 1 bit per element, for backward's scatter-reduce
+      g.epi.aux = w.sgn[br][s];
+      g.epi.aux_ld = J / 32;
       pr.push_back(g);
     }
   }
@@ -849,7 +847,6 @@ int backward(const lirec_model_cfg& cfg, const lirec_model_params& P, const lire
         const int inv = (s < 2) ? 0 : (s - 1);
         j.d_in = w.da2[br] + s * J;
         j.d_ld = 4 * J;
-        j.r1 = w.r1[br][s];
         j.sign = w.sgn[br][s];
         j.sign_ld = J / 32;
         j.J = J;
@@ -863,8 +860,7 @@ int backward(const lirec_model_cfg& cfg, const lirec_model_params& P, const lire
         j.ref_w = (br && use_refs) ? w.ref_w[inv] : nullptr;
         j.drop = mk_drop(p, B.seed, br ? DS_L1_CTX : DS_L1_INTS, 0);
         j.out = w.dz1T[br][s];
-        j.out_ld = 0;
-        j.out_t_pitch = (s < 2) ? d.ncP[br] : d.ntP[br];
+        j.out_pitch = (s < 2) ? d.ncP[br] : d.ntP[br];
       }
     }
     jobs.n = n;

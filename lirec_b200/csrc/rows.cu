@@ -184,53 +184,6 @@ expand_fwd_kernel(const ExpandFwdJobs jobs) {
   if (jb.flag_bf16_out && threadIdx.x == 0) jb.flag_bf16_out[o] = __float2bfloat16_rn(n > 0 ? 1.f : 0.f);
 }
 
-// ---------------------------------------------------------------------------
-// Backward of the expansion onto the unique rows of one bank slot:
-//   dZ1[u] = [r1[u] > 0] * sum_{i in inv(u)} keep(i) * w_i * d_in[o_i]
-// ---------------------------------------------------------------------------
-__global__ void __launch_bounds__(128)
-expand_bwd_kernel(const ExpandBwdJobs jobs) {
-  pdl_wait();
-  pdl_trigger();
-  const ExpandBwdJob& jb = jobs.job[blockIdx.y];
-  const int u = blockIdx.x;
-  if (u >= jb.n_unique) return;
-  const int J = jb.J;
-  const int beg = jb.inv_off[u], end = jb.inv_off[u + 1];
-  for (int j = threadIdx.x * 4; j < J; j += blockDim.x * 4) {
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-    for (int q = beg; q < end; ++q) {
-      const int i = jb.inv_idx[q];
-      int o = i;
-      float w = 1.0f;
-      if (jb.owner) {
-        o = jb.owner[i];
-        w = 1.0f / static_cast<float>(jb.seg_off[o + 1] - jb.seg_off[o]);
-      }
-      float4 g = ld4(jb.d_in + static_cast<int64_t>(o) * jb.d_ld + j);
-      if (jb.drop.p > 0.f) {
-        const uint32_t rkey = drop_row_key(jb.drop.seed, jb.drop.stream_id, static_cast<uint32_t>(i));
-        const uint32_t c = static_cast<uint32_t>(jb.drop.col_off + jb.slot * J + j);   // multiple of 4
-        const uint32_t thr = drop_threshold(jb.drop.p);
-        const uint32_t w0 = drop_word(rkey, c >> 1), w1 = drop_word(rkey, (c >> 1) + 1);
-        if ((w0 & 0xFFFFu) < thr) g.x = 0.f;
-        if ((w0 >> 16) < thr) g.y = 0.f;
-        if ((w1 & 0xFFFFu) < thr) g.z = 0.f;
-        if ((w1 >> 16) < thr) g.w = 0.f;
-      }
-      acc.x += w * g.x; acc.y += w * g.y; acc.z += w * g.z; acc.w += w * g.w;
-    }
-    const float4 r = ld4(jb.r1 + static_cast<int64_t>(u) * J + j);
-    if (!(r.x > 0.f)) acc.x = 0.f;
-    if (!(r.y > 0.f)) acc.y = 0.f;
-    if (!(r.z > 0.f)) acc.z = 0.f;
-    if (!(r.w > 0.f)) acc.w = 0.f;
-    __nv_bfloat16* orow = jb.out + static_cast<int64_t>(u) * jb.out_ld;
-    store_split4(orow + j, orow + J + j, acc);
-  }
-}
-
-
 // Per-reference (owner, 1 / segment length) of the context branch's three inverse CSRs, see rows.cuh.
 __global__ void __launch_bounds__(256)
 ref_tables_kernel(const RefTableJobs jobs) {
@@ -248,8 +201,11 @@ ref_tables_kernel(const RefTableJobs jobs) {
 }
 
 // ---------------------------------------------------------------------------
-// Same reduction, TRANSPOSED output: out[(j) * pitch + u] (hi rows [0, J), lo rows [J, 2J)), the
-// K-major B operand of the first-layer weight-gradient GEMM.  One CTA owns 64 consecutive unique rows
+// Backward of the expansion onto the unique rows of one bank slot:
+//   dZ1[u] = [r1[u] > 0] * sum_{i in inv(u)} keep(i) * w_i * d_in[o_i]
+// with the ReLU gate [r1 > 0] read from the 1-bit mask of the layer-1 GEMM (LIREC_POST_SIGN_MASK), written
+// TRANSPOSED: out[(j) * pitch + u] (hi rows [0, J), lo rows [J, 2J)), the K-major B operand of the
+// first-layer weight-gradient GEMM.  One CTA owns 64 consecutive unique rows
 // and walks the J columns in chunks of 64: thread t reduces 16 columns of row t/4, the chunk is
 // transposed through shared memory, and every output row segment is 64 rows x 2 B = one 128-byte line.
 // ---------------------------------------------------------------------------
@@ -310,18 +266,14 @@ expand_bwd_t_kernel(const ExpandBwdJobs jobs) {
     for (int k = 0; k < 16; ++k) acc[k] = 0.f;
     const int j = c0 + q4;
     uint2 gate = make_uint2(0u, 0u);       // issued ahead of the reference loop (c0 % 64 == 0: 8-byte aligned)
-    if (live && jb.sign) gate = *reinterpret_cast<const uint2*>(jb.sign + static_cast<int64_t>(u) * jb.sign_ld + (c0 >> 5));
-    // Latency hiding without registers: the ReLU gate of this chunk (read after the reference loop) and the
-    // gradient pieces of the NEXT chunk are pulled into L2 now; a row's 64 columns are two 128-byte lines, taken
-    // by the first two lanes of its quad.
-    if (live && (threadIdx.x & 3) < 2) {
+    if (live) gate = *reinterpret_cast<const uint2*>(jb.sign + static_cast<int64_t>(u) * jb.sign_ld + (c0 >> 5));
+    // Latency hiding without registers: the gradient pieces of the NEXT chunk are pulled into L2 now; a row's
+    // 64 columns are two 128-byte lines, taken by the first two lanes of its quad.
+    if (live && (threadIdx.x & 3) < 2 && c0 + EBT_COLS < c_end) {
       const int half = 32 * (threadIdx.x & 3);
-      if (!jb.sign) prefetch_l2(jb.r1 + static_cast<int64_t>(u) * J + c0 + half);
-      if (c0 + EBT_COLS < c_end) {
-        for (int q = beg; q < min(end, beg + 4); ++q)
-          if (q - q0 < EBT_REFS)
-            prefetch_l2(jb.d_in + static_cast<int64_t>(ref_out[q - q0]) * jb.d_ld + c0 + EBT_COLS + half);
-      }
+      for (int q = beg; q < min(end, beg + 4); ++q)
+        if (q - q0 < EBT_REFS)
+          prefetch_l2(jb.d_in + static_cast<int64_t>(ref_out[q - q0]) * jb.d_ld + c0 + EBT_COLS + half);
     }
     for (int q = beg; q < end; ++q) {
       int i, o;
@@ -358,7 +310,7 @@ expand_bwd_t_kernel(const ExpandBwdJobs jobs) {
         acc[4 * k + 2] += w * g[k].z; acc[4 * k + 3] += w * g[k].w;
       }
     }
-    if (live && jb.sign) {
+    if (live) {
       // ReLU gate from the 1-bit-per-element mask of the forward GEMM (8 bytes per row and chunk instead of 256)
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
@@ -366,16 +318,6 @@ expand_bwd_t_kernel(const ExpandBwdJobs jobs) {
 #pragma unroll
         for (int e = 0; e < 4; ++e)
           if (!((bits >> e) & 1u)) acc[4 * k + e] = 0.f;
-      }
-    } else if (live) {
-      const float* rp = jb.r1 + static_cast<int64_t>(u) * J + j;
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        const float4 r = ld4(rp + 16 * k);
-        if (!(r.x > 0.f)) acc[4 * k] = 0.f;
-        if (!(r.y > 0.f)) acc[4 * k + 1] = 0.f;
-        if (!(r.z > 0.f)) acc[4 * k + 2] = 0.f;
-        if (!(r.w > 0.f)) acc[4 * k + 3] = 0.f;
       }
     }
 #pragma unroll
@@ -393,7 +335,7 @@ expand_bwd_t_kernel(const ExpandBwdJobs jobs) {
       const int nrow = min(EBT_ROWS, jb.n_unique - u0);
 #pragma unroll
       for (int part = 0; part < 2; ++part) {
-        __nv_bfloat16* dst = jb.out + (static_cast<int64_t>(part) * J + c0 + col) * jb.out_t_pitch + u0 + r0;
+        __nv_bfloat16* dst = jb.out + (static_cast<int64_t>(part) * J + c0 + col) * jb.out_pitch + u0 + r0;
         const __nv_bfloat16* src = &tile[part][col][r0];
         if (r0 + 16 <= nrow) {
           reinterpret_cast<uint4*>(dst)[0] = reinterpret_cast<const uint4*>(src)[0];
@@ -474,23 +416,8 @@ transpose_bf16_kernel(const TransposeJobs jobs) {
 }
 
 // ---------------------------------------------------------------------------
-// fp32 -> hi/lo bf16 split with zero padding; fp32 -> bf16 cast
+// fp32 -> bf16 cast
 // ---------------------------------------------------------------------------
-__global__ void __launch_bounds__(256)
-split_kernel(const float* __restrict__ x, int64_t ld, int rows, int cols, __nv_bfloat16* __restrict__ out,
-             int64_t out_ld, int pad_cols) {
-  const int64_t total = static_cast<int64_t>(rows) * pad_cols;
-  for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < total;
-       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-    const int r = static_cast<int>(i / pad_cols), c = static_cast<int>(i % pad_cols);
-    const float v = (c < cols) ? x[r * ld + c] : 0.f;
-    __nv_bfloat16 h, l;
-    split_bf16(v, h, l);
-    out[r * out_ld + c] = h;
-    out[r * out_ld + pad_cols + c] = l;
-  }
-}
-
 __global__ void __launch_bounds__(256)
 cast_bf16_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ out, int64_t n) {
   const int64_t n4 = n / 4;
@@ -766,39 +693,27 @@ int ref_tables(const RefTableJobs& jobs, cudaStream_t stream) {
 }
 
 int expand_bwd(const ExpandBwdJobs& jobs, cudaStream_t stream) {
-  int max_u = 0;
+  int max_u = 0, max_j = 0;
   for (int i = 0; i < jobs.n; ++i) {
     const ExpandBwdJob& j = jobs.job[i];
-    LIREC_REQUIRE(j.J > 0 && j.J % 4 == 0 && j.d_ld % 4 == 0, "expand_bwd: J=%d d_ld=%lld", j.J,
+    LIREC_REQUIRE(j.J > 0 && j.J % EBT_COLS == 0 && j.d_ld % 4 == 0,
+                  "expand_bwd: J=%d must be a positive multiple of 64, d_ld=%lld a multiple of 4", j.J,
                   (long long)j.d_ld);
+    LIREC_REQUIRE(j.out_pitch % 8 == 0 && j.out_pitch >= j.n_unique && (reinterpret_cast<uintptr_t>(j.out) & 15) == 0,
+                  "expand_bwd: output needs 16-byte alignment and a pitch >= n_unique that is a multiple of 8");
+    LIREC_REQUIRE(j.sign && (reinterpret_cast<uintptr_t>(j.sign) & 7) == 0 && j.sign_ld % 2 == 0 &&
+                      j.sign_ld >= j.J / 32,
+                  "expand_bwd: sign mask must be non-NULL, 8-byte aligned, with an even pitch >= J / 32 words");
     max_u = std::max(max_u, j.n_unique);
+    max_j = std::max(max_j, j.J);
   }
   if (max_u == 0 || jobs.n == 0) return LIREC_OK;
-  int n_t = 0;
-  for (int i = 0; i < jobs.n; ++i) n_t += jobs.job[i].out_t_pitch > 0 ? 1 : 0;
-  LIREC_REQUIRE(n_t == 0 || n_t == jobs.n, "expand_bwd: natural and transposed outputs cannot be mixed");
-  if (n_t) {
-    for (int i = 0; i < jobs.n; ++i) {
-      const ExpandBwdJob& j = jobs.job[i];
-      LIREC_REQUIRE(j.J % EBT_COLS == 0 && j.out_t_pitch % 8 == 0 && j.out_t_pitch >= j.n_unique &&
-                        (reinterpret_cast<uintptr_t>(j.out) & 15) == 0,
-                    "expand_bwd: transposed output needs J %% 64 == 0 and a 16-byte aligned pitch");
-      LIREC_REQUIRE(!j.sign || ((reinterpret_cast<uintptr_t>(j.sign) & 7) == 0 && j.sign_ld % 2 == 0 &&
-                                j.sign_ld >= j.J / 32),
-                    "expand_bwd: sign mask must be 8-byte aligned with an even pitch >= J / 32 words");
-    }
-    int max_j = 0;
-    for (int i = 0; i < jobs.n; ++i) max_j = std::max(max_j, jobs.job[i].J);
-    // column split over grid.z: 4 at bench sizes; 8 (one 64-column chunk per CTA) when the whole launch is
-    // under ~2 k CTAs — measured on B200: 64-clip batches 41 -> 27 us, 1024-clip batches 141 -> 149 us
-    const int row_ctas = (max_u + EBT_ROWS - 1) / EBT_ROWS;
-    const int zsplit = (static_cast<long>(row_ctas) * jobs.n * EBT_ZSPLIT <= 2048) ? 2 * EBT_ZSPLIT : EBT_ZSPLIT;
-    dim3 grid(row_ctas, jobs.n, std::max(1, std::min(zsplit, max_j / EBT_COLS)));
-    LIREC_CUDA_OK(launch_pdl(expand_bwd_t_kernel, grid, dim3(256), 0, stream, jobs));
-  } else {
-    dim3 grid(max_u, jobs.n);
-    LIREC_CUDA_OK(launch_pdl(expand_bwd_kernel, grid, dim3(128), 0, stream, jobs));
-  }
+  // column split over grid.z: 4 at bench sizes; 8 (one 64-column chunk per CTA) when the whole launch is
+  // under ~2 k CTAs — measured on B200: 64-clip batches 41 -> 27 us, 1024-clip batches 141 -> 149 us
+  const int row_ctas = (max_u + EBT_ROWS - 1) / EBT_ROWS;
+  const int zsplit = (static_cast<long>(row_ctas) * jobs.n * EBT_ZSPLIT <= 2048) ? 2 * EBT_ZSPLIT : EBT_ZSPLIT;
+  dim3 grid(row_ctas, jobs.n, std::max(1, std::min(zsplit, max_j / EBT_COLS)));
+  LIREC_CUDA_OK(launch_pdl(expand_bwd_t_kernel, grid, dim3(256), 0, stream, jobs));
   LIREC_CUDA_OK(cudaGetLastError());
   note_launch();
   return LIREC_OK;
@@ -826,20 +741,6 @@ int transpose_bf16(const TransposeJobs& jobs, cudaStream_t stream) {
   }
   dim3 grid(std::min(max_tiles, 148 * 4), jobs.n);
   LIREC_CUDA_OK(launch_pdl(transpose_bf16_kernel, grid, dim3(256), 0, stream, jobs));
-  note_launch();
-  return LIREC_OK;
-}
-
-int split_f32(const float* x, int64_t ld, int rows, int cols, void* out, int64_t out_ld, int pad_cols,
-              cudaStream_t stream) {
-  LIREC_REQUIRE(pad_cols >= cols && out_ld >= 2 * pad_cols, "split_f32: pad_cols=%d cols=%d out_ld=%lld",
-                pad_cols, cols, (long long)out_ld);
-  if (rows <= 0) return LIREC_OK;
-  const int64_t total = static_cast<int64_t>(rows) * pad_cols;
-  const int grid = static_cast<int>(std::min<int64_t>((total + 255) / 256, 148 * 8));
-  split_kernel<<<grid, 256, 0, stream>>>(x, ld, rows, cols, reinterpret_cast<__nv_bfloat16*>(out), out_ld,
-                                         pad_cols);
-  LIREC_CUDA_OK(cudaGetLastError());
   note_launch();
   return LIREC_OK;
 }
@@ -894,24 +795,22 @@ extern "C" int lirec_rows_expand_fwd(const float* r1_txt, const float* r1_vis, c
   return rows::expand_fwd(jobs, static_cast<cudaStream_t>(stream));
 }
 
-extern "C" int lirec_rows_expand_bwd(const float* d_in, int64_t d_ld, const float* r1, int32_t J,
-                                     int32_t slot, const int32_t* inv_off, const int32_t* inv_idx,
+extern "C" int lirec_rows_expand_bwd(const float* d_in, int64_t d_ld, const uint32_t* sign, int64_t sign_ld,
+                                     int32_t J, int32_t slot, const int32_t* inv_off, const int32_t* inv_idx,
                                      int32_t n_unique, const int32_t* owner, const int32_t* seg_off,
-                                     lirec_dropout drop, void* out_split, int64_t out_ld,
-                                     int64_t out_t_pitch, void* stream) {
+                                     lirec_dropout drop, void* out_split, int64_t out_pitch, void* stream) {
   LIREC_ENTER();
   LIREC_REQUIRE((owner == nullptr) == (seg_off == nullptr), "expand_bwd: owner and seg_off go together");
   rows::ExpandBwdJobs jobs;
   jobs.n = 1;
   rows::ExpandBwdJob& j = jobs.job[0];
-  j.d_in = d_in; j.d_ld = d_ld; j.r1 = r1; j.J = J; j.slot = slot;
+  j.d_in = d_in; j.d_ld = d_ld; j.J = J; j.slot = slot;
+  j.sign = sign; j.sign_ld = sign_ld;
   j.inv_off = inv_off; j.inv_idx = inv_idx; j.n_unique = n_unique;
   j.owner = owner; j.seg_off = seg_off; j.drop = drop;
   j.ref_out = nullptr; j.ref_w = nullptr;
-  j.sign = nullptr; j.sign_ld = 0;
   j.out = reinterpret_cast<__nv_bfloat16*>(out_split);
-  j.out_ld = out_ld;
-  j.out_t_pitch = out_t_pitch;
+  j.out_pitch = out_pitch;
   return rows::expand_bwd(jobs, static_cast<cudaStream_t>(stream));
 }
 
@@ -931,9 +830,9 @@ extern "C" int lirec_gather_rows(const void* bank, int64_t bank_ld, int32_t n_ba
 }
 
 extern "C" int lirec_split_f32(const float* x, int64_t ld, int32_t rows_n, int32_t cols, void* out_split,
-                               int64_t out_ld, int32_t pad_cols, void* stream) {
+                               int64_t pitch, int32_t pad, void* stream) {
   LIREC_ENTER();
-  return rows::split_f32(x, ld, rows_n, cols, out_split, out_ld, pad_cols, static_cast<cudaStream_t>(stream));
+  return rows::split_f32_t(x, ld, rows_n, cols, out_split, pitch, pad, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int lirec_cast_bf16(const float* x, void* out, int64_t n, void* stream) {

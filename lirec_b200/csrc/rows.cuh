@@ -32,10 +32,9 @@ struct ExpandFwdJobs {
 struct ExpandBwdJob {
   const float* d_in;        // [n_out, d_ld] fp32 (column offset of the slot already applied)
   int64_t d_ld;
-  const float* r1;          // [n_unique, J]
-  const uint32_t* sign;     // optional (transposed form): bit (j & 31) of sign[u * sign_ld + (j >> 5)] = [r1[u, j] > 0],
-  int64_t sign_ld;          // as the layer-1 GEMM epilogue writes it (LIREC_POST_SIGN_MASK); read INSTEAD of r1
-  int32_t J, slot;
+  const uint32_t* sign;     // ReLU gate: bit (j & 31) of sign[u * sign_ld + (j >> 5)] = [r1[u, j] > 0], as the
+  int64_t sign_ld;          // layer-1 GEMM epilogue writes it (LIREC_POST_SIGN_MASK)
+  int32_t J, slot;          // J % 64 == 0
   const int32_t* inv_off;   // [n_unique + 1]
   const int32_t* inv_idx;   // table rows referencing each unique row
   int32_t n_unique;
@@ -44,9 +43,8 @@ struct ExpandBwdJob {
   const int32_t* ref_out;   // optional, parallel to inv_idx (ref_tables): owner[inv_idx[q]] ...
   const float* ref_w;       // ... and 1 / its segment length, so the kernel skips two dependent lookups
   lirec_dropout drop;
-  __nv_bfloat16* out;       // [n_unique, out_ld] hi|lo, or transposed [2J, out_t_pitch] (hi rows, lo rows)
-  int64_t out_ld;
-  int64_t out_t_pitch;      // > 0: transposed output with this row pitch (elements)
+  __nv_bfloat16* out;       // transposed [2J, out_pitch]: hi rows [0, J), lo rows [J, 2J)
+  int64_t out_pitch;        // row pitch (elements), >= n_unique
 };
 struct ExpandBwdJobs {
   ExpandBwdJob job[MAX_JOBS];
@@ -84,8 +82,6 @@ int seg_reduce(const float* x, const int32_t* seg_off, int nseg, int dim, int mo
                int64_t out_f32_ld, void* out_bf16, int64_t out_bf16_ld, cudaStream_t stream, const int32_t* row_idx = nullptr);
 int expand_fwd(const ExpandFwdJobs& jobs, cudaStream_t stream);
 int expand_bwd(const ExpandBwdJobs& jobs, cudaStream_t stream);
-int split_f32(const float* x, int64_t ld, int rows, int cols, void* out, int64_t out_ld, int pad_cols,
-              cudaStream_t stream);
 int cast_bf16(const float* x, void* out, int64_t n, cudaStream_t stream);
 int roi_max_pool(const float* maps, int T, int C, int H, int W, const int32_t* elem, int n_elem,
                  const int32_t* seg_off, int nseg, float* scratch, float* out_f32, int64_t out_f32_ld, void* out_bf16,

@@ -138,20 +138,23 @@ def rows_expand_fwd(r1, J, rows, seg_off, n_out, guard_zero, drop, out_split, ro
         _ext.ptr(row_flag_out), _ext.stream_ptr()))
 
 
-def rows_expand_bwd(d_in, d_ld, r1, J, slot, inv_off, inv_idx, n_unique, owner, seg_off, drop, out_split,
-                    d_in_col_off=0, transposed=False):
-    """transposed=False: out_split [n_unique, 2J]; True: out_split [2J, pitch] with pitch = out_split.stride(0)."""
+def rows_expand_bwd(d_in, d_ld, sign, J, slot, inv_off, inv_idx, n_unique, owner, seg_off, drop, out_split,
+                    d_in_col_off=0):
+    """sign: int32 [n_unique, >= J / 32] ReLU gate bits (LIREC_POST_SIGN_MASK layout); out_split: [2J, pitch] hi
+    rows then lo rows, pitch = out_split.stride(0)."""
     L = _ext.lib()
     _ext.check(L.lirec_rows_expand_bwd(
-        d_in.data_ptr() + 4 * d_in_col_off, d_ld, _ext.ptr(r1), J, slot, _ext.ptr(inv_off), _ext.ptr(inv_idx),
-        n_unique, _ext.ptr(owner), _ext.ptr(seg_off), drop, _ext.ptr(out_split), out_split.stride(0),
-        out_split.stride(0) if transposed else 0, _ext.stream_ptr()))
+        d_in.data_ptr() + 4 * d_in_col_off, d_ld, _ext.ptr(sign), sign.stride(0), J, slot, _ext.ptr(inv_off),
+        _ext.ptr(inv_idx), n_unique, _ext.ptr(owner), _ext.ptr(seg_off), drop, _ext.ptr(out_split),
+        out_split.stride(0), _ext.stream_ptr()))
 
 
-def split_f32(x, out_split, pad_cols):
+def split_f32(x, out_split, pad):
+    """x fp32 [rows, cols] -> out_split [2 * pad, pitch >= rows]: hi of x[r, c] at out_split[c, r], lo at
+    out_split[pad + c, r], rows [cols, pad) of each half zero."""
     L = _ext.lib()
     _ext.check(L.lirec_split_f32(_ext.ptr(x), x.stride(0), x.shape[0], x.shape[1], _ext.ptr(out_split),
-                                 out_split.stride(0), pad_cols, _ext.stream_ptr()))
+                                 out_split.stride(0), pad, _ext.stream_ptr()))
 
 
 def cast_bf16(x, out):

@@ -25,12 +25,13 @@ def test_header_symbols_exported(built_lib):
         assert hasattr(lib, name), "include/lirec_b200.h declares %s but the library does not export it" % name
 
 
-def test_binding_lists_every_symbol_of_abi_version_2(built_lib):
-    """Version 2: one entry point per operation (lirec_model_backward takes the nullable heads event,
-    lirec_adam_flat the coresident flag, lirec_seg_reduce_f32 the nullable row index)."""
+def test_binding_lists_every_symbol_of_abi_version_3(built_lib):
+    """Version 3: lirec_rows_expand_bwd reads the ReLU gate as the bit mask of LIREC_POST_SIGN_MASK and writes
+    only the transposed hi/lo form, and lirec_split_f32 writes the transposed split.  The symbol list is that
+    of version 2."""
     from lirec_b200 import _ext
     assert sorted(_ext.EXPORTED_SYMBOLS) == _declared_symbols()
-    assert _ext.lib().lirec_abi_version() == 2
+    assert _ext.lib().lirec_abi_version() == 3
 
 
 def test_sass_is_blackwell_native(built_lib):

@@ -70,7 +70,7 @@ def _expand_reference(r1, rows, seg_off, keep, J, guard):
 
 
 @pytest.mark.parametrize("p", [0.0, 0.3])
-def test_expand_forward_and_backward(p):
+def test_expand_forward_and_transposed_backward(p):
     from lirec_b200 import ops
     from oracle import dropout as od
     rng = np.random.default_rng(3)
@@ -101,37 +101,40 @@ def test_expand_forward_and_backward(p):
     empty = [c for c in range(n_out) if seg[c + 1] == seg[c]]
     assert empty and torch.isnan(out[empty].float()).all() and not torch.isnan(out[[c for c in range(n_out) if c not in empty]].float()).any()
 
-    # backward (context form): dZ1[u] = [r1[u] > 0] * sum_i keep_i * d[owner_i] / n(owner_i)
+    # backward: dZ1[u] = [r1[u] > 0] * sum_i keep_i * d[o_i] * w_i, context form (o_i = owner_i,
+    # w_i = 1 / n(owner_i)) and ints form (o_i = i, w_i = 1), written transposed [2J, pitch] (hi rows, lo rows)
     from lirec_b200.packing import _csr_inverse
     owner = np.repeat(np.arange(n_out), np.diff(seg)).astype(np.int32)
-    d = rng.standard_normal((n_out, 4 * J)).astype(np.float32)
-    dd = torch.from_numpy(d).cuda()
-    for slot, col, n_u in ((0, 0, n_clip), (1, 0, n_clip), (2, 1, n_track), (3, 2, n_track)):
-        off, idx = _csr_inverse(rows[:, col], n_u)
-        out = torch.zeros(n_u, 2 * J, device="cuda", dtype=torch.bfloat16)
-        ops.rows_expand_bwd(dd, 4 * J, r1d[slot], J, slot, torch.from_numpy(off).cuda(), torch.from_numpy(idx).cuda(),
-                            n_u, torch.from_numpy(owner).cuda(), segd, drop, out, d_in_col_off=slot * J)
-        ref = np.zeros((n_u, J))
-        for i in range(n_rows):
-            o = owner[i]
-            ref[rows[i, col]] += keep[i, slot * J:(slot + 1) * J] * d[o, slot * J:(slot + 1) * J] / (seg[o + 1] - seg[o])
-        ref *= (r1[slot] > 0)
-        got = (out[:, :J].double() + out[:, J:].double()).cpu().numpy()
-        np.testing.assert_allclose(got, ref, rtol=0, atol=2e-5 * np.abs(ref).max())
-        # transposed output (the K-major operand of the first-layer wgrad GEMM): same values, bit for bit
-        pitch = (n_u + 63) // 64 * 64
-        out_t = torch.zeros(2 * J, pitch, device="cuda", dtype=torch.bfloat16)
-        ops.rows_expand_bwd(dd, 4 * J, r1d[slot], J, slot, torch.from_numpy(off).cuda(), torch.from_numpy(idx).cuda(),
-                            n_u, torch.from_numpy(owner).cuda(), segd, drop, out_t, d_in_col_off=slot * J,
-                            transposed=True)
-        assert torch.equal(out_t[:, :n_u].t().contiguous(), out)
+    d_ctx = rng.standard_normal((n_out, 4 * J)).astype(np.float32)
+    d_ints = rng.standard_normal((n_rows, 4 * J)).astype(np.float32)
+    # the ReLU gate as the layer-1 GEMM writes it (LIREC_POST_SIGN_MASK): bit j & 31 of word u * J / 32 + (j >> 5)
+    sign = [torch.from_numpy(np.packbits(a > 0, axis=1, bitorder="little").view("<u4").view(np.int32)).cuda()
+            for a in r1]
+    for d, owner_np in ((d_ctx, owner), (d_ints, None)):
+        dd = torch.from_numpy(d).cuda()
+        owner_t, seg_t = (torch.from_numpy(owner_np).cuda(), segd) if owner_np is not None else (None, None)
+        for slot, col, n_u in ((0, 0, n_clip), (1, 0, n_clip), (2, 1, n_track), (3, 2, n_track)):
+            off, idx = _csr_inverse(rows[:, col], n_u)
+            pitch = (n_u + 63) // 64 * 64
+            out = torch.zeros(2 * J, pitch, device="cuda", dtype=torch.bfloat16)
+            ops.rows_expand_bwd(dd, 4 * J, sign[slot], J, slot, torch.from_numpy(off).cuda(),
+                                torch.from_numpy(idx).cuda(), n_u, owner_t, seg_t, drop, out, d_in_col_off=slot * J)
+            ref = np.zeros((n_u, J))
+            for i in range(n_rows):
+                o = owner_np[i] if owner_np is not None else i
+                n = seg[o + 1] - seg[o] if owner_np is not None else 1
+                ref[rows[i, col]] += keep[i, slot * J:(slot + 1) * J] * d[o, slot * J:(slot + 1) * J] / n
+            ref *= (r1[slot] > 0)
+            got = (out[:J, :n_u].double() + out[J:, :n_u].double()).t().cpu().numpy()
+            np.testing.assert_allclose(got, ref, rtol=0, atol=2e-5 * np.abs(ref).max())
 
 
-def test_split_and_cast():
+def test_transposed_split_and_cast():
     from lirec_b200 import ops
     x = torch.randn(37, 101, device="cuda") * 3
-    out = torch.full((37, 256), 7.0, device="cuda", dtype=torch.bfloat16)
-    ops.split_f32(x, out, 128)
+    out_t = torch.full((256, 40), 7.0, device="cuda", dtype=torch.bfloat16)   # transposed [2 * pad, pitch]
+    ops.split_f32(x, out_t, 128)
+    out = out_t[:, :37].t()                                                    # [rows, 2 * pad]: hi | lo
     assert torch.equal(out[:, :101], x.to(torch.bfloat16))
     assert (out[:, 101:128] == 0).all() and (out[:, 128 + 101:] == 0).all()
     rec = out[:, :101].double() + out[:, 128:128 + 101].double()
