@@ -306,6 +306,32 @@ int lirec_loss_rowmargin_fwd_bwd(const float* logits, int64_t ld, int32_t rows, 
                                  float scale, float* loss_per_row, float* d_logits,
                                  int64_t d_ld, void* stream);
 
+/* Multi-label sigmoid binary cross-entropy, forward + gradient (the reference has no BCE: parity is
+ * unpinned by construction; the tests' reference is torch's binary_cross_entropy_with_logits in fp64).
+ * Per element with target t and weight w:
+ *   l = w * (t * softplus(-x) + (1 - t) * softplus(x)),  dl/dx = w * (sigma(x) - t),
+ * softplus(x) = max(x,0) + log1p(exp(-|x|)), finite for any finite logit.  Masks are [rows or B, C]
+ * uint8; NULL means none.  Every element of the gradient rows a call owns is written.
+ *
+ * Row form: t_c = 1 for c == label or pos_mask[i,c] != 0; w_c = 0 for a non-target with
+ * neg_mask[i,c] == 0 (neg_mask NULL: every non-target is a negative).
+ *   loss_per_row[i] = scale * sum_c w_c * l_c;  rows with label < 0 get 0 and a zero gradient row. */
+int lirec_loss_bce_fwd_bwd(const float* logits, int64_t ld, int32_t rows, int32_t C, const int32_t* labels,
+                           const uint8_t* neg_mask, const uint8_t* pos_mask, float scale,
+                           float* loss_per_row, float* d_logits, int64_t d_ld, void* stream);
+
+/* Track form over the same inputs as lirec_loss_track_fwd_bwd, plus pos_mask [B, C] (NULL: none).
+ * t* is chosen exactly as there (arg-max, tr_correct, cat_distr) and written to assign[b].  The
+ * interaction positives are (t*, y) and (t*, c) for pos_mask[b,c] != 0; the negatives are the margin
+ * loss's sum-form negatives minus those positives; every other (slot, class) has weight 0.  The
+ * relationship positive is (t*, r0) when live, its negatives the margin loss's relationship negatives.
+ *   loss_per_clip[b] = lymbda / B * sum_ints l + 1 / B * sum_rels l
+ * cfg.margin is ignored; cfg.max_neg != 0 is LIREC_ERR_ARG (max-negative is a hinge idea).          */
+int lirec_loss_bce_track_fwd_bwd(const float* ints, const float* rels, const int32_t* cand_off, int32_t B,
+                                 const int32_t* labels, const int32_t* rels_label, const int32_t* gt_tracks,
+                                 const uint8_t* multilab, const uint8_t* pos_mask, lirec_track_loss_cfg cfg,
+                                 float* loss_per_clip, int32_t* assign, float* d_ints, float* d_rels, void* stream);
+
 /* Prediction arg-maxes of the evaluation loop (reference utils/evaluation.py:114-175, 179-271:
  * track assignment for the GT class (+ relationship), joint (t,c[,r]) arg-max, class / relationship
  * arg-max at the two GT slots), computed on the ragged logits so only 8 integers per clip go back to

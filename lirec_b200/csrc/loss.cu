@@ -31,43 +31,21 @@ __device__ __forceinline__ float block_sum(float v, float* red) {
 
 constexpr int MAX_SLOTS = 128;
 
-// MarginLoss (mlp/model.py:444-494) / MarginTrackRelsLoss (mlp/model.py:497-575).
-__global__ void __launch_bounds__(128)
-track_loss_kernel(const float* __restrict__ ints, const float* __restrict__ rels,
-                  const int32_t* __restrict__ cand_off, int B, const int32_t* __restrict__ labels,
-                  const int32_t* __restrict__ rels_label, const int32_t* __restrict__ gt_tracks,
-                  const uint8_t* __restrict__ multilab, lirec_track_loss_cfg cfg,
-                  float* __restrict__ loss_per_clip, int32_t* __restrict__ assign,
-                  float* __restrict__ d_ints, float* __restrict__ d_rels) {
-  pdl_wait();
-  pdl_trigger();
+// The weakly supervised track assignment t* of clip b over its n candidate slots, shared by the margin and
+// the BCE track losses: slot 0 under tr_correct, a counter-hash draw from the softmax scores under
+// cat_distr, otherwise the arg-max of sigma(ints[t,y]) (+ sigma(rels[t,r0])) with the lowest index winning
+// ties.  Called by every thread of the CTA; returns t* to all of them and writes assign[b].
+__device__ __forceinline__ int track_assign(const float* __restrict__ xi, const float* __restrict__ xr,
+                                            const int32_t* __restrict__ rels_lab, int n, int C, int R, int y, int r0,
+                                            int b, const lirec_track_loss_cfg& cfg, int32_t* __restrict__ assign) {
   __shared__ float s_score[MAX_SLOTS];
-  __shared__ float s_red[8];
   __shared__ int s_tstar;
-  const int b = blockIdx.x;
-  const int beg = cand_off[b], n = cand_off[b + 1] - beg;
-  const int C = cfg.n_classes, R = cfg.n_rels;
   const bool has_rels = R > 0;
-  const int y = labels[b];
-  const int gt0 = gt_tracks[2 * b], gt1 = gt_tracks[2 * b + 1];
-  // relationship class of the ground-truth pair(s); slots past the valid prefix carry the
-  // reference's pad label 0 (classification_dataloader.py:430)
-  int r0 = 0, r1 = 0;
-  if (has_rels) {
-    r0 = (gt0 < n) ? rels_label[beg + gt0] : 0;
-    r1 = (gt1 < n) ? rels_label[beg + gt1] : 0;
-  }
-  const float* xi = ints + static_cast<int64_t>(beg) * C;
-  const float* xr = has_rels ? rels + static_cast<int64_t>(beg) * R : nullptr;
-  float* gi = d_ints + static_cast<int64_t>(beg) * C;
-  float* gr = has_rels ? d_rels + static_cast<int64_t>(beg) * R : nullptr;
-  const float invB = 1.0f / static_cast<float>(B);
-
   // ---- per-slot assignment score: sigma(ints[t,y]) (+ sigma(rels[t,r0])) ----
   for (int t = threadIdx.x; t < n; t += blockDim.x) {
     float sc = sigmoidf(xi[static_cast<int64_t>(t) * C + y]);
     if (has_rels) {
-      const bool rel_on = rels_label[beg + t] != R;  // None-labelled slots are all -inf
+      const bool rel_on = rels_lab[t] != R;  // None-labelled slots are all -inf
       const float pr = (rel_on && r0 < R) ? sigmoidf(xr[static_cast<int64_t>(t) * R + r0]) : 0.f;
       sc = sc + pr;
     }
@@ -82,19 +60,19 @@ track_loss_kernel(const float* __restrict__ ints, const float* __restrict__ rels
       float mx = -INFINITY, mxr = -INFINITY;
       for (int t = 0; t < n; ++t) {
         mx = fmaxf(mx, xi[static_cast<int64_t>(t) * C + y]);
-        if (has_rels && r0 < R && rels_label[beg + t] != R) mxr = fmaxf(mxr, xr[static_cast<int64_t>(t) * R + r0]);
+        if (has_rels && r0 < R && rels_lab[t] != R) mxr = fmaxf(mxr, xr[static_cast<int64_t>(t) * R + r0]);
       }
       float zi = 0.f, zr = 0.f;
       for (int t = 0; t < n; ++t) {
         zi += expf(xi[static_cast<int64_t>(t) * C + y] - mx);
-        if (has_rels && r0 < R && rels_label[beg + t] != R) zr += expf(xr[static_cast<int64_t>(t) * R + r0] - mxr);
+        if (has_rels && r0 < R && rels_lab[t] != R) zr += expf(xr[static_cast<int64_t>(t) * R + r0] - mxr);
       }
       float total = 0.f;
       for (int t = 0; t < n; ++t) {
         float pt = expf(xi[static_cast<int64_t>(t) * C + y] - mx) / zi;
         if (has_rels) {
           float pr = 0.f;
-          if (r0 < R && rels_label[beg + t] != R && zr > 0.f) pr = expf(xr[static_cast<int64_t>(t) * R + r0] - mxr) / zr;
+          if (r0 < R && rels_lab[t] != R && zr > 0.f) pr = expf(xr[static_cast<int64_t>(t) * R + r0] - mxr) / zr;
           pt = 0.5f * (pt + pr);
         }
         s_p[t] = pt;
@@ -126,7 +104,39 @@ track_loss_kernel(const float* __restrict__ ints, const float* __restrict__ rels
     assign[b] = best;
   }
   __syncthreads();
-  const int ts = s_tstar;
+  return s_tstar;
+}
+
+// MarginLoss (mlp/model.py:444-494) / MarginTrackRelsLoss (mlp/model.py:497-575).
+__global__ void __launch_bounds__(128)
+track_loss_kernel(const float* __restrict__ ints, const float* __restrict__ rels,
+                  const int32_t* __restrict__ cand_off, int B, const int32_t* __restrict__ labels,
+                  const int32_t* __restrict__ rels_label, const int32_t* __restrict__ gt_tracks,
+                  const uint8_t* __restrict__ multilab, lirec_track_loss_cfg cfg,
+                  float* __restrict__ loss_per_clip, int32_t* __restrict__ assign,
+                  float* __restrict__ d_ints, float* __restrict__ d_rels) {
+  pdl_wait();
+  pdl_trigger();
+  __shared__ float s_red[8];
+  const int b = blockIdx.x;
+  const int beg = cand_off[b], n = cand_off[b + 1] - beg;
+  const int C = cfg.n_classes, R = cfg.n_rels;
+  const bool has_rels = R > 0;
+  const int y = labels[b];
+  const int gt0 = gt_tracks[2 * b], gt1 = gt_tracks[2 * b + 1];
+  // relationship class of the ground-truth pair(s); slots past the valid prefix carry the
+  // reference's pad label 0 (classification_dataloader.py:430)
+  int r0 = 0, r1 = 0;
+  if (has_rels) {
+    r0 = (gt0 < n) ? rels_label[beg + gt0] : 0;
+    r1 = (gt1 < n) ? rels_label[beg + gt1] : 0;
+  }
+  const float* xi = ints + static_cast<int64_t>(beg) * C;
+  const float* xr = has_rels ? rels + static_cast<int64_t>(beg) * R : nullptr;
+  float* gi = d_ints + static_cast<int64_t>(beg) * C;
+  float* gr = has_rels ? d_rels + static_cast<int64_t>(beg) * R : nullptr;
+  const float invB = 1.0f / static_cast<float>(B);
+  const int ts = track_assign(xi, xr, has_rels ? rels_label + beg : nullptr, n, C, R, y, r0, b, cfg, assign);
   const float pos = sigmoidf(xi[static_cast<int64_t>(ts) * C + y]);
   float pos_r = 0.f;
   bool pos_r_live = false;
@@ -302,6 +312,141 @@ ce_kernel(const float* __restrict__ logits, int64_t ld, int C, const int32_t* __
   const float w = (class_w ? class_w[y] : 1.0f) * scale;
   for (int c = threadIdx.x; c < C; c += blockDim.x) g[c] = w * (expf(x[c] - mx) / z - (c == y ? 1.f : 0.f));
   if (threadIdx.x == 0) loss_per_row[b] = w * (logf(z) + mx - x[y]);
+}
+
+// ---- sigmoid binary cross-entropy (multi-label) --------------------------------------------------------
+// Per element with target t and weight w:  l = w * (t ? softplus(-x) : softplus(x)),  dl/dx = w * (sigma(x) - t).
+// softplus(x) = max(x, 0) + log1p(exp(-|x|)) stays finite and exact for logits far outside [-88, 88].
+__device__ __forceinline__ float softplusf(float x) { return fmaxf(x, 0.f) + log1pf(expf(-fabsf(x))); }
+
+__device__ __forceinline__ float warp_sum(float v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+
+constexpr int BCE_ROWS_PER_CTA = 4;  // one warp per row: rows are short (C = 101 or R = 15)
+
+// Row form: target 1 on the label and on pos_mask, weight 0 on the non-targets that neg_mask excludes.
+//   loss_row = scale * sum_c w_c * BCE(x_c, t_c);  d/dx_c = scale * w_c * (sigma(x_c) - t_c)
+// Rows with label < 0 get loss 0 and a zero gradient row.
+__global__ void __launch_bounds__(32 * BCE_ROWS_PER_CTA)
+bce_rows_kernel(const float* __restrict__ logits, int64_t ld, int rows, int C, const int32_t* __restrict__ labels,
+                const uint8_t* __restrict__ neg_mask, const uint8_t* __restrict__ pos_mask, float scale,
+                float* __restrict__ loss_per_row, float* __restrict__ d_logits, int64_t d_ld) {
+  pdl_wait();
+  pdl_trigger();
+  const int lane = threadIdx.x & 31;
+  const int b = blockIdx.x * BCE_ROWS_PER_CTA + (threadIdx.x >> 5);
+  if (b >= rows) return;
+  const int y = labels[b];
+  float* g = d_logits + static_cast<int64_t>(b) * d_ld;
+  if (y < 0) {
+    for (int c = lane; c < C; c += 32) g[c] = 0.f;
+    if (lane == 0) loss_per_row[b] = 0.f;
+    return;
+  }
+  const float* x = logits + static_cast<int64_t>(b) * ld;
+  const uint8_t* nm = neg_mask ? neg_mask + static_cast<int64_t>(b) * C : nullptr;
+  const uint8_t* pm = pos_mask ? pos_mask + static_cast<int64_t>(b) * C : nullptr;
+  float l = 0.f;
+  for (int c = lane; c < C; c += 32) {
+    const float v = x[c];
+    const bool pos = (c == y) || (pm != nullptr && pm[c] != 0);
+    float gv = 0.f;
+    if (pos) {
+      l += softplusf(-v);
+      gv = scale * (sigmoidf(v) - 1.f);
+    } else if (nm == nullptr || nm[c] != 0) {
+      l += softplusf(v);
+      gv = scale * sigmoidf(v);
+    }
+    g[c] = gv;
+  }
+  l = warp_sum(l);
+  if (lane == 0) loss_per_row[b] = scale * l;
+}
+
+// Track form: one CTA per clip.  t* is the margin loss's assignment (track_assign); the positives are
+// (t*, y) and (t*, c) for pos_mask[b, c] != 0, the negatives are the margin loss's sum-form negatives
+// minus those positives, and every other (slot, class) has weight 0.  The relationship positive is
+// (t*, r0) when live, its negatives the margin loss's relationship negatives.
+//   loss_per_clip = lymbda / B * sum_ints l + 1 / B * sum_rels l
+__global__ void __launch_bounds__(128)
+bce_track_kernel(const float* __restrict__ ints, const float* __restrict__ rels,
+                 const int32_t* __restrict__ cand_off, int B, const int32_t* __restrict__ labels,
+                 const int32_t* __restrict__ rels_label, const int32_t* __restrict__ gt_tracks,
+                 const uint8_t* __restrict__ multilab, const uint8_t* __restrict__ pos_mask, lirec_track_loss_cfg cfg,
+                 float* __restrict__ loss_per_clip, int32_t* __restrict__ assign, float* __restrict__ d_ints,
+                 float* __restrict__ d_rels) {
+  pdl_wait();
+  pdl_trigger();
+  __shared__ float s_red[8];
+  const int b = blockIdx.x;
+  const int beg = cand_off[b], n = cand_off[b + 1] - beg;
+  const int C = cfg.n_classes, R = cfg.n_rels;
+  const bool has_rels = R > 0;
+  const int y = labels[b];
+  const int gt0 = gt_tracks[2 * b], gt1 = gt_tracks[2 * b + 1];
+  int r0 = 0, r1 = 0;
+  if (has_rels) {
+    r0 = (gt0 < n) ? rels_label[beg + gt0] : 0;
+    r1 = (gt1 < n) ? rels_label[beg + gt1] : 0;
+  }
+  const float* xi = ints + static_cast<int64_t>(beg) * C;
+  const float* xr = has_rels ? rels + static_cast<int64_t>(beg) * R : nullptr;
+  float* gi = d_ints + static_cast<int64_t>(beg) * C;
+  float* gr = has_rels ? d_rels + static_cast<int64_t>(beg) * R : nullptr;
+  const float invB = 1.0f / static_cast<float>(B);
+  const int ts = track_assign(xi, xr, has_rels ? rels_label + beg : nullptr, n, C, R, y, r0, b, cfg, assign);
+  const float wi = cfg.lymbda * invB, wr = invB;
+  const uint8_t* ml = multilab + static_cast<int64_t>(b) * C;
+  const uint8_t* pm = pos_mask ? pos_mask + static_cast<int64_t>(b) * C : nullptr;
+
+  float loss_i = 0.f, loss_r = 0.f;
+  for (int e = threadIdx.x; e < n * C; e += blockDim.x) {
+    const int t = e / C, c = e - t * C;
+    const bool pos = (t == ts) && (c == y || (pm != nullptr && pm[c] != 0));
+    bool neg = ml[c] != 0;
+    if (cfg.tr_correct) neg = neg && !(c == y && (t == gt0 || t == gt1));
+    else neg = neg && (c != y);
+    float g = 0.f;
+    if (pos) {
+      const float v = xi[e];
+      loss_i += softplusf(-v);
+      g = wi * (sigmoidf(v) - 1.f);
+    } else if (neg) {
+      const float v = xi[e];
+      loss_i += softplusf(v);
+      g = wi * sigmoidf(v);
+    }
+    gi[e] = g;
+  }
+  if (has_rels) {
+    const bool pos_r_live = (rels_label[beg + ts] != R) && (r0 < R);
+    for (int e = threadIdx.x; e < n * R; e += blockDim.x) {
+      const int t = e / R, r = e - t * R;
+      const int lab = rels_label[beg + t];
+      const bool pos = pos_r_live && t == ts && r == r0;
+      bool neg = lab != R;
+      if (cfg.tr_correct) neg = neg && (r != lab);
+      else neg = neg && (r != r0) && (r != r1);
+      float g = 0.f;
+      if (pos) {
+        const float v = xr[e];
+        loss_r += softplusf(-v);
+        g = wr * (sigmoidf(v) - 1.f);
+      } else if (neg) {
+        const float v = xr[e];
+        loss_r += softplusf(v);
+        g = wr * sigmoidf(v);
+      }
+      gr[e] = g;
+    }
+  }
+  loss_i = block_sum(loss_i, s_red);
+  if (has_rels) loss_r = block_sum(loss_r, s_red);
+  if (threadIdx.x == 0) loss_per_clip[b] = cfg.lymbda * loss_i * invB + loss_r * invB;
 }
 
 // Prediction arg-maxes of the evaluation loop (reference utils/evaluation.py:114-175, 179-271), one CTA
@@ -498,6 +643,42 @@ extern "C" int lirec_loss_ce_fwd_bwd(const float* logits, int64_t ld, int32_t ro
   loss::ce_kernel<<<rows, 128, 0, static_cast<cudaStream_t>(stream)>>>(logits, ld, C, labels, class_weights, scale,
                                                                       loss_per_row, d_logits, d_ld);
   LIREC_CUDA_OK(cudaGetLastError());
+  note_launch();
+  return LIREC_OK;
+}
+
+extern "C" int lirec_loss_bce_fwd_bwd(const float* logits, int64_t ld, int32_t rows, int32_t C, const int32_t* labels,
+                                      const uint8_t* neg_mask, const uint8_t* pos_mask, float scale,
+                                      float* loss_per_row, float* d_logits, int64_t d_ld, void* stream) {
+  LIREC_ENTER();
+  LIREC_REQUIRE(logits && labels && loss_per_row && d_logits && C > 0, "bce loss: bad arguments");
+  if (rows <= 0) return LIREC_OK;
+  const int grid = (rows + loss::BCE_ROWS_PER_CTA - 1) / loss::BCE_ROWS_PER_CTA;
+  LIREC_CUDA_OK(launch_pdl(loss::bce_rows_kernel, dim3(grid), dim3(32 * loss::BCE_ROWS_PER_CTA), 0,
+                           static_cast<cudaStream_t>(stream), logits, ld, rows, C, labels, neg_mask, pos_mask, scale,
+                           loss_per_row, d_logits, d_ld));
+  note_launch();
+  return LIREC_OK;
+}
+
+extern "C" int lirec_loss_bce_track_fwd_bwd(const float* ints, const float* rels, const int32_t* cand_off, int32_t B,
+                                            const int32_t* labels, const int32_t* rels_label, const int32_t* gt_tracks,
+                                            const uint8_t* multilab, const uint8_t* pos_mask, lirec_track_loss_cfg cfg,
+                                            float* loss_per_clip, int32_t* assign, float* d_ints, float* d_rels,
+                                            void* stream) {
+  LIREC_ENTER();
+  LIREC_REQUIRE(ints && cand_off && labels && gt_tracks && multilab && loss_per_clip && assign && d_ints,
+                "bce track loss: null pointer");
+  LIREC_REQUIRE(cfg.n_classes > 0 && cfg.n_rels >= 0, "bce track loss: n_classes=%d n_rels=%d", cfg.n_classes,
+                cfg.n_rels);
+  LIREC_REQUIRE(cfg.n_rels == 0 || (rels && rels_label && d_rels), "bce track loss: rel tensors missing");
+  LIREC_REQUIRE(!cfg.max_neg, "bce track loss: max_neg is a hinge variant, the BCE has no max-negative form");
+  LIREC_REQUIRE(cfg.max_slots > 0 && cfg.max_slots <= loss::MAX_SLOTS, "bce track loss: max_slots=%d (limit %d)",
+                cfg.max_slots, loss::MAX_SLOTS);
+  if (B <= 0) return LIREC_OK;
+  LIREC_CUDA_OK(launch_pdl(loss::bce_track_kernel, dim3(B), dim3(128), 0, static_cast<cudaStream_t>(stream), ints, rels,
+                           cand_off, B, labels, rels_label, gt_tracks, multilab, pos_mask, cfg, loss_per_clip, assign,
+                           d_ints, d_rels));
   note_launch();
   return LIREC_OK;
 }

@@ -131,21 +131,26 @@ class _PinnedRing:
         self.k = 0
 
     def stage(self, pb, copy_stream):
-        """Point `pb` (a host PackedBatch with `_host_arena`) at pinned copies of its arena / multilab."""
+        """Point `pb` (a host PackedBatch with `_host_arena`) at pinned copies of its arena / multilab (/ soft_pos)."""
         k = self.k
         self.k = (k + 1) % len(self.arena)
         if self.ev[k] is not None:
             self.ev[k].synchronize()                         # the slot's previous batch has crossed PCIe
         src = torch.from_numpy(pb._host_arena)
+        sp = pb.soft_pos                                     # --soft_gt: staged behind multilab in the same buffer
         n, m = src.numel(), pb.multilab.numel()
+        ms = m + (sp.numel() if sp is not None else 0)
         if self.arena[k] is None or self.arena[k].numel() < n:
             self.arena[k] = torch.empty(int(n * 1.25) + 1024, dtype=torch.int32).pin_memory()
-        if self.ml[k] is None or self.ml[k].numel() < m:
-            self.ml[k] = torch.empty(int(m * 1.25) + 1024, dtype=torch.uint8).pin_memory()
+        if self.ml[k] is None or self.ml[k].numel() < ms:
+            self.ml[k] = torch.empty(int(ms * 1.25) + 1024, dtype=torch.uint8).pin_memory()
         self.arena[k][:n].copy_(src)
         self.ml[k][:m].copy_(pb.multilab.reshape(-1))
         pb._arena, pb._layout = self.arena[k][:n], pb._host_layout
         pb.multilab = self.ml[k][:m].view(pb.multilab.shape)
+        if sp is not None:
+            self.ml[k][m:ms].copy_(sp.reshape(-1))
+            pb.soft_pos = self.ml[k][m:ms].view(sp.shape)
         self._last = k
         return pb
 

@@ -29,7 +29,7 @@ import numpy as np
 import torch
 from torch.utils.data import Dataset
 
-from lirec_b200.packing import PackedBatch
+from lirec_b200.packing import PackedBatch, soft_pos_of
 from lirec_b200.utils.arg_pars import opt
 
 
@@ -682,9 +682,19 @@ def collate_indexed(records, dataset, resident=False):
     mw = np.concatenate([r["multilab_weights"] for r in records]).reshape(B, -1) if "multilab_weights" in records[0] \
         else np.ones((B, dataset.n_classes))
     extras = {k: np.array([r[k] for r in records]) for k in ("just_zeros", "n_names", "hash_rel") if k in records[0]}
-    return collate_arrays(dataset, cand, counts, ctx if has_ctx else None, ctx_counts if has_ctx else None,
-                          [r["labels"] for r in records], rels_label, gt, mw, extras, T, records[0]["n_ctx_slots"],
-                          resident)
+    pb = collate_arrays(dataset, cand, counts, ctx if has_ctx else None, ctx_counts if has_ctx else None,
+                        [r["labels"] for r in records], rels_label, gt, mw, extras, T, records[0]["n_ctx_slots"],
+                        resident)
+    return _with_soft_pos(pb, records, dataset)
+
+
+def _with_soft_pos(pb, records, dataset):
+    """--soft_gt: attach the uint8 [B, C] multi-hot of the records' soft labels (`pb.soft_pos`), the positives of
+    the BCE losses.  Without soft labels the batch is left exactly as it is."""
+    if "soft_labels" in records[0]:
+        pb.soft_pos = soft_pos_of(np.stack([np.asarray(r["soft_labels"]).reshape(-1) for r in records]),
+                                  dataset.n_classes)
+    return pb
 
 
 def collate_arrays(dataset, cand, counts, ctx, ctx_counts, labels, rels_label, gt, multilab, extras, n_slots,
@@ -810,7 +820,7 @@ def collate_indexed_numpy(records, dataset, resident=False):
         n_slots=dataset._max_n_tripl if track_models else 1,
         n_ctx_slots=records[0]["n_ctx_slots"], extras=extras)
     pb.extras["bank_rows"] = (clip_src.astype(np.int32), track_src.astype(np.int32))
-    return pb
+    return _with_soft_pos(pb, records, dataset)
 
 
 STAGE_TRACE = None      # measurement aid (bench.py, LIREC_BENCH_DEBUG): a list that ResidentBanks.stage appends its phase times to

@@ -21,7 +21,7 @@ from lirec_b200.utils.arg_pars import opt
 
 __all__ = ["Modalities", "MidFusionMultiClip", "MidFusionMultiClipMaxTracks", "GatingUnit",
            "MultiTaskCrossEntropyLoss", "MultiTaskMaxMargin", "MaxMarginCrossEntropyLoss", "MarginLoss",
-           "MarginTrackRelsLoss", "create_model", "ModelOutput", "FlatAdam"]
+           "MarginTrackRelsLoss", "MultiLabelBCELoss", "TrackBCELoss", "create_model", "ModelOutput", "FlatAdam"]
 
 _SLOTS = ("txt", "vis", "tracks1", "tracks2")
 _SECOND = ("txt2", "vis2", "tracks12", "tracks22")
@@ -531,12 +531,19 @@ def _rel_term(loss_mod, pb, n_sel, run):
 
 
 def dp_empty_shard_collectives(loss_mod, device):
-    """The collectives a loss would have issued on a rank that holds an EmptyShard this step."""
-    if int(getattr(loss_mod, "_dp_world", 1) or 1) > 1 and isinstance(loss_mod, (MultiTaskMaxMargin,
-                                                                                 MultiTaskCrossEntropyLoss)):
-        if isinstance(loss_mod, MultiTaskCrossEntropyLoss) or opt.ctx == 1:
-            import torch.distributed as dist
-            dist.all_reduce(torch.zeros(1, dtype=torch.float32, device=device))
+    """The collectives a loss would have issued on a rank that holds an EmptyShard this step: the one all_reduce of
+    `_rel_term`, issued by the multi-task losses whenever their relationship term runs."""
+    if int(getattr(loss_mod, "_dp_world", 1) or 1) <= 1:
+        return
+    if isinstance(loss_mod, MultiTaskCrossEntropyLoss):
+        rel_term = not opt.mod_check and opt.ctx == 1      # the model has relationship logits (Modalities has none)
+    elif isinstance(loss_mod, MultiLabelBCELoss):
+        rel_term = bool(loss_mod.n_rels) and opt.ctx == 1
+    else:
+        rel_term = isinstance(loss_mod, MultiTaskMaxMargin) and opt.ctx == 1
+    if rel_term:
+        import torch.distributed as dist
+        dist.all_reduce(torch.zeros(1, dtype=torch.float32, device=device))
 
 
 class MaxMarginCrossEntropyLoss(_FusedLoss):
@@ -588,10 +595,15 @@ class _TrackLoss(_FusedLoss):
     def set_rank(self, rank):
         self._seed_rank = int(rank)            # tr_cat_distr draws differ per data-parallel rank
 
+    def _draw_seed(self):
+        """Counter-hash seed of this step's tr_cat_distr draw (per loss call and data-parallel rank)."""
+        self._draws = getattr(self, "_draws", 0) + 1
+        return int(opt.seed) * 0x9E3779B1 + self._draws * 0xC2B2AE35 + getattr(self, "_seed_rank", 0) * 0x27D4EB2F
+
     def _run(self, x, args, n_rels, lymbda):
         assert opt.tr_maximize
         assert not (opt.tr_cat_distr and opt.tr_correct)                 # model.py:469, 539
-        self._draws = getattr(self, "_draws", 0) + 1
+        seed = self._draw_seed()
         pb = _batch_of(x, args)
         li, lr = x.ragged_inters, x.ragged_rels if n_rels else None
         if li is None:
@@ -601,8 +613,7 @@ class _TrackLoss(_FusedLoss):
             li, lr, pb["cand_off"], pb["labels"], pb["rels_label"] if n_rels else None, pb["gt_tracks"],
             pb.multilab, self.m, lymbda, n_rels, tr_correct=opt.tr_correct,
             max_neg=bool(opt.tr_max_neg and opt.tr_sum_max_flag), max_slots=pb.n_slots,
-            cat_distr=bool(opt.tr_cat_distr),
-            seed=(int(opt.seed) * 0x9E3779B1 + self._draws * 0xC2B2AE35 + getattr(self, "_seed_rank", 0) * 0x27D4EB2F))
+            cat_distr=bool(opt.tr_cat_distr), seed=seed)
         self.last_assignment = assign
         return terms, d_i, (d_r if n_rels else None)
 
@@ -663,6 +674,81 @@ class MultiTaskCrossEntropyLoss(_FusedLoss):
             if t is not None:
                 terms.append(t)
         return torch.cat(terms), d_i, d_r
+
+
+def _soft_pos(pb):
+    """The batch's soft-label positives (uint8 [B, C]) under --soft_gt, None otherwise."""
+    if not opt.soft_gt:
+        return None
+    sp = getattr(pb, "soft_pos", None)
+    if sp is None:
+        raise RuntimeError("--soft_gt is set but the batch carries no soft labels (soft_pos): only the index-only "
+                           "MovieGraphs dataset (and the synthetic annotation world) builds them; refusing to train "
+                           "the BCE loss on the hard labels alone")
+    return sp
+
+
+class MultiLabelBCELoss(_FusedLoss):
+    """Multi-label sigmoid BCE for Modalities / MidFusionMultiClip (lirec_loss_bce_fwd_bwd).  Interaction rows:
+    target 1 on the label (and, under --soft_gt, on the co-occurring interactions of the batch's `soft_pos`),
+    target 0 on the classes multilab_weights keeps as negatives, the rest left out.  Without a relationship
+    term (n_rels == 0) the interaction term is a mean over the clips, like MaxMarginCrossEntropyLoss; with one it
+    is weighted by lymbda and gated by opt.ints, and the relationship term (one-hot target, no mask) is the mean
+    over the rows whose label is not None, like MultiTaskMaxMargin."""
+
+    def __init__(self, n_rels=0):
+        super().__init__()
+        self.n_rels = n_rels
+
+    def terms_and_grads(self, x, args):
+        pb = _batch_of(x, args)
+        terms, d_i, d_r = [], None, None
+        if not self.n_rels or opt.ints == 1:
+            li = x.ragged_inters
+            w = (opt.lymbda if self.n_rels else 1.0) / li.shape[0]
+            t, d_i = ops.loss_bce(li, pb["labels"], pb.multilab, _soft_pos(pb), w)
+            terms.append(t)
+        if self.n_rels and opt.ctx == 1:
+            lr = x.ragged_rels
+            host = pb.host if pb.device is not None else pb
+            n_sel = int((host["rels_label"] != self.n_rels).sum())
+
+            def run(scale):
+                sel = pb["rels_label"].clone()
+                sel[sel == self.n_rels] = -1                     # rows labelled None are skipped
+                return ops.loss_bce(lr, sel, None, None, scale)
+            t, d_r = _rel_term(self, pb, n_sel, run)
+            if t is not None:
+                terms.append(t)
+        return torch.cat(terms), d_i, d_r
+
+
+class TrackBCELoss(_TrackLoss):
+    """Sigmoid BCE over the weakly supervised track assignment of MidFusionMultiClipMaxTracks
+    (lirec_loss_bce_track_fwd_bwd): t* is the margin losses' assignment (same arg-max, tr_correct slot and
+    tr_cat_distr draw for the same step); (t*, label) and, under --soft_gt, (t*, soft positives) are the
+    targets, the margin losses' negatives the zeros.  n_rels > 0 adds the relationship term, weighting the
+    interaction term by lymbda as MarginTrackRelsLoss does."""
+
+    def __init__(self, n_rels=0):
+        super().__init__()
+        self.n_rels = n_rels
+
+    def terms_and_grads(self, x, args):
+        assert opt.tr_maximize
+        assert not (opt.tr_cat_distr and opt.tr_correct)
+        seed = self._draw_seed()
+        pb = _batch_of(x, args)
+        n_rels = self.n_rels
+        li, lr = x.ragged_inters, x.ragged_rels if n_rels else None
+        if li is None:
+            raise ValueError("TrackBCELoss needs interaction logits (opt.ints == 1)")
+        terms, assign, d_i, d_r = ops.loss_bce_track(
+            li, lr, pb["cand_off"], pb["labels"], pb["rels_label"] if n_rels else None, pb["gt_tracks"],
+            pb.multilab, _soft_pos(pb), opt.lymbda if n_rels else 1.0, n_rels, tr_correct=opt.tr_correct,
+            max_slots=pb.n_slots, cat_distr=bool(opt.tr_cat_distr), seed=seed)
+        self.last_assignment = assign
+        return terms, d_i, (d_r if n_rels else None)
 
 
 def train_step(model, loss, x, seed=None):
@@ -769,8 +855,25 @@ class FlatAdam(torch.optim.Optimizer):
         self._t = int(steps[0]) if steps else 0
 
 
+def _check_loss_choice():
+    """--loss against the rest of the configuration (host only, before any device work)."""
+    kind = getattr(opt, "loss", "margin")
+    if kind not in ("margin", "bce", "ce"):
+        raise ValueError("--loss must be margin, bce or ce (got %r)" % (kind,))
+    if kind == "ce" and opt.tr_maximize:
+        raise ValueError("--loss ce has no track-assignment form: use margin or bce with --tr_maximize")
+    if kind == "ce" and not opt.mod_check and opt.ints == 0:
+        raise ValueError("--loss ce needs interaction logits (opt.ints == 1): MultiTaskCrossEntropyLoss always has an "
+                         "interaction term")
+    if kind == "bce" and opt.tr_max_neg:
+        raise ValueError("--loss bce has no max-negative form (--tr_max_neg is a hinge variant)")
+    return kind
+
+
 def create_model(n_classes, n_rels=0):
-    """Reference: mlp/model.py:578-609 — same selection logic and return triple."""
+    """Reference: mlp/model.py:578-609 — same selection logic and return triple.  --loss bce / ce swap in the
+    multi-label BCE or the softmax cross-entropy for the reference's max-margin losses."""
+    loss_kind = _check_loss_choice()
     if opt.device != "cuda":
         raise RuntimeError("lirec_b200 runs on a B200 only (opt.device='%s'); no CPU fallback" % opt.device)
     if opt.tr_maximize:
@@ -781,7 +884,11 @@ def create_model(n_classes, n_rels=0):
         model = Modalities(n_classes=n_classes)
     model = model.to(opt.device)
 
-    if opt.tr_maximize:
+    if loss_kind == "bce":
+        loss = (TrackBCELoss if opt.tr_maximize else MultiLabelBCELoss)(n_rels=n_rels if opt.rels_multitask else 0)
+    elif loss_kind == "ce":
+        loss = MultiTaskCrossEntropyLoss(n_classes, n_rels=n_rels if opt.rels_multitask else 0)
+    elif opt.tr_maximize:
         loss = MarginTrackRelsLoss(n_rels=n_rels) if opt.rels_multitask else MarginLoss()
     else:
         loss = MultiTaskMaxMargin(n_rels=n_rels) if opt.rels_multitask else MaxMarginCrossEntropyLoss()

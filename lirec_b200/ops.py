@@ -12,7 +12,7 @@ from ._ext import (ACT_NONE, ACT_RELU, ACT_TANH, OUT_F32, OUT_SPLIT, OUT_SPLIT_T
                    POST_NONE, POST_SIGN_MASK)
 
 __all__ = ["gemm_problem", "gemm_grouped", "seg_reduce", "seg_softmax_pool", "seg_softmax_pool_bwd", "SegSoftmaxPool", "rows_expand_fwd", "rows_expand_bwd", "split_f32",
-           "cast_bf16", "gather_rows", "roi_max_pool", "loss_track", "loss_rowmargin", "loss_ce", "predict_tracks", "adam_flat", "dp_exchange", "dp_reduce_adam_bcast", "dp_reduce_adam_bcast_peer", "dropout_desc"]
+           "cast_bf16", "gather_rows", "roi_max_pool", "loss_track", "loss_rowmargin", "loss_ce", "loss_bce", "loss_bce_track", "predict_tracks", "adam_flat", "dp_exchange", "dp_reduce_adam_bcast", "dp_reduce_adam_bcast_peer", "dropout_desc"]
 
 
 def dropout_desc(p=0.0, seed=0, stream_id=0, col_off=0):
@@ -222,6 +222,40 @@ def loss_ce(logits, labels, class_weights, scale):
                                                 _ext.ptr(class_weights), float(scale), _ext.ptr(loss), _ext.ptr(d),
                                                 d.stride(0), _ext.stream_ptr()))
     return loss, d
+
+
+def loss_bce(logits, labels, neg_mask, pos_mask, scale):
+    """Multi-label sigmoid BCE rows, forward + gradient (lirec_loss_bce_fwd_bwd): target 1 on the label and on
+    pos_mask, non-targets with neg_mask == 0 left out (masks uint8 [rows, C] or None). labels < 0 are skipped."""
+    rows, Cc = logits.shape
+    loss = torch.empty(rows, dtype=torch.float32, device=logits.device)
+    d = torch.empty_like(logits)
+    _ext.check(_ext.lib().lirec_loss_bce_fwd_bwd(
+        _ext.ptr(logits), logits.stride(0), rows, Cc, _ext.ptr(labels), _ext.ptr(neg_mask), _ext.ptr(pos_mask),
+        float(scale), _ext.ptr(loss), _ext.ptr(d), d.stride(0), _ext.stream_ptr()))
+    return loss, d
+
+
+def loss_bce_track(ints, rels, cand_off, labels, rels_label, gt_tracks, multilab, pos_mask, lymbda, n_rels,
+                   tr_correct=False, max_slots=20, cat_distr=False, seed=0):
+    """Fused BCE over the weakly supervised track assignment (lirec_loss_bce_track_fwd_bwd); t* is chosen as in
+    loss_track. Returns (loss_per_clip, assign, d_ints, d_rels)."""
+    B = cand_off.numel() - 1
+    Ni, Cc = ints.shape
+    cfg = _ext.TrackLossCfg()
+    cfg.margin, cfg.lymbda = 0.0, float(lymbda)
+    cfg.n_classes, cfg.n_rels = int(Cc), int(n_rels)
+    cfg.tr_correct, cfg.max_neg, cfg.max_slots = int(tr_correct), 0, int(max_slots)
+    cfg.cat_distr, cfg.seed = int(cat_distr), int(seed) & 0xFFFFFFFF
+    loss = torch.empty(B, dtype=torch.float32, device=ints.device)
+    assign = torch.empty(B, dtype=torch.int32, device=ints.device)
+    d_ints = torch.empty_like(ints)
+    d_rels = torch.empty_like(rels) if n_rels > 0 else None
+    _ext.check(_ext.lib().lirec_loss_bce_track_fwd_bwd(
+        _ext.ptr(ints), _ext.ptr(rels) if n_rels > 0 else None, _ext.ptr(cand_off), B, _ext.ptr(labels),
+        _ext.ptr(rels_label) if n_rels > 0 else None, _ext.ptr(gt_tracks), _ext.ptr(multilab), _ext.ptr(pos_mask), cfg,
+        _ext.ptr(loss), _ext.ptr(assign), _ext.ptr(d_ints), _ext.ptr(d_rels), _ext.stream_ptr()))
+    return loss, assign, d_ints, d_rels
 
 
 def loss_rowmargin(logits, labels, weights, margin, scale):

@@ -97,6 +97,7 @@ class PackedBatch:
         self.n_clip_ints = 0
         self.n_track_ints = 0
         self.multilab = None        # uint8 [B, C]
+        self.soft_pos = None        # uint8 [B, C] multi-hot of the soft labels (--soft_gt), else None
         self.tables = {}            # name -> int32 array/tensor
         self.extras = {}            # pass-through keys (just_zeros, n_names, hash_rel, soft_labels ...)
         self.device = None
@@ -258,6 +259,8 @@ class PackedBatch:
     # ---- device staging --------------------------------------------------------------------
     def h2d_bytes(self):
         n = self.clip_bank.numel() * 2 + self.track_bank.numel() * 2 + self.multilab.numel()
+        if self.soft_pos is not None:
+            n += self.soft_pos.numel()
         for v in self.tables.values():
             n += v.size * 4
         return int(n)
@@ -284,6 +287,8 @@ class PackedBatch:
             self.clip_bank = self.clip_bank.pin_memory()
             self.track_bank = self.track_bank.pin_memory()
             self.multilab = self.multilab.pin_memory()
+            if self.soft_pos is not None:
+                self.soft_pos = self.soft_pos.pin_memory()
             self._pin_bank_rows()
             return self
         names = [k for k in _INT_TABLES if k in self.tables]
@@ -299,6 +304,8 @@ class PackedBatch:
         self.clip_bank = self.clip_bank.pin_memory()
         self.track_bank = self.track_bank.pin_memory()
         self.multilab = self.multilab.pin_memory()
+        if self.soft_pos is not None:
+            self.soft_pos = self.soft_pos.pin_memory()
         self._pin_bank_rows()
         return self
 
@@ -317,6 +324,8 @@ class PackedBatch:
             d.clip_bank = self.clip_bank.to(device, non_blocking=non_blocking)
             d.track_bank = self.track_bank.to(device, non_blocking=non_blocking)
         d.multilab = self.multilab.to(device, non_blocking=non_blocking)
+        if self.soft_pos is not None:
+            d.soft_pos = self.soft_pos.to(device, non_blocking=non_blocking)
         d.tables = _DeviceTables(arena, self._layout)
         d._n_cand = int(self._layout["cand_rows"][2][0])
         if self.has_ctx:
@@ -332,7 +341,7 @@ class PackedBatch:
         assert self.device is None
         d = PackedBatch()
         for k in ("B", "n_slots", "n_ctx_slots", "n_classes", "has_ctx", "n_clip_ints", "n_track_ints", "multilab",
-                  "tables"):
+                  "soft_pos", "tables"):
             setattr(d, k, getattr(self, k))
         d.extras = dict(self.extras)
         if getattr(self, "_host_arena", None) is not None:
@@ -348,6 +357,8 @@ class PackedBatch:
         allocated on a copy stream)."""
         for t in (self._arena_dev, self.clip_bank, self.track_bank, self.multilab) + tuple(getattr(self, "_bank_idx", ())):
             t.record_stream(stream)
+        if self.soft_pos is not None:
+            self.soft_pos.record_stream(stream)
         return self
 
     # ---- dense (reference-format) view -------------------------------------------------------
@@ -479,6 +490,20 @@ def pack_dense_batch(batch, kind, n_slots=None):
         mw = np.ones((B, int(batch.get("n_classes", 101))))
     mw = mw.numpy() if isinstance(mw, torch.Tensor) else np.asarray(mw)
     extras = {k: batch[k] for k in ("just_zeros", "n_names", "hash_rel", "soft_labels") if k in batch}
-    return PackedBatch.from_tables(np.vstack(clip_rows), np.vstack(tr_rows), n_clip_ints, n_track_ints,
-                                   cand_off, cand_tbl, ctx_off, ctx_tbl, labels, rels_label, gt_tracks, mw,
-                                   n_slots=n_slots or T, n_ctx_slots=S, extras=extras)
+    pb = PackedBatch.from_tables(np.vstack(clip_rows), np.vstack(tr_rows), n_clip_ints, n_track_ints,
+                                 cand_off, cand_tbl, ctx_off, ctx_tbl, labels, rels_label, gt_tracks, mw,
+                                 n_slots=n_slots or T, n_ctx_slots=S, extras=extras)
+    if "soft_labels" in batch:
+        sl = batch["soft_labels"]
+        pb.soft_pos = soft_pos_of(sl.numpy() if isinstance(sl, torch.Tensor) else sl, pb.n_classes)
+    return pb
+
+
+def soft_pos_of(soft_labels, n_classes):
+    """uint8 [B, C] multi-hot of the soft-label class ids [B, K] (the dataset's `soft_labels`: the clip's label
+    and the interactions that co-occur with it in time, padded with -1) — the extra positives of the BCE losses."""
+    sl = np.asarray(soft_labels).reshape(len(soft_labels), -1).astype(np.int64)
+    out = np.zeros((sl.shape[0], int(n_classes)), dtype=np.uint8)
+    rows, cols = np.nonzero(sl >= 0)
+    out[rows, sl[rows, cols]] = 1
+    return torch.from_numpy(out)

@@ -123,6 +123,10 @@ _FLAGS = [
     ("--resident_banks", dict(default=1, type=int, help="1 (default): the split's pooled feature banks stay in HBM "
                                                         "(< 1 GB for MovieGraphs) and batches ship index tables; "
                                                         "0: every batch carries its feature rows host -> device")),
+    ("--loss", dict(default="margin", choices=("margin", "bce", "ce"),
+                    help="margin: the reference's max-margin losses; bce: multi-label sigmoid BCE (row and track "
+                         "forms; --soft_gt adds the co-occurring interactions as positives); ce: softmax "
+                         "cross-entropy (row models only)")),
     ("--world_movies", dict(default=6, type=int)),
     ("--world_scenes", dict(default=40, type=int)),
 ]
