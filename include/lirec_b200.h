@@ -479,6 +479,30 @@ int lirec_adam_flat(float* param, const float* grad, float* exp_avg, float* exp_
                     void* param_bf16, int64_t n, float lr, float beta1, float beta2, float eps,
                     float weight_decay, int32_t step, float grad_scale, int32_t coresident, void* stream);
 
+/* LAMB (You et al., "Large Batch Optimization for Deep Learning", ICLR 2020) over the same flat buffers, for
+ * large-batch training.  Tensor l is floats [tensor_begin[l], tensor_begin[l] + tensor_len[l]) of the buffers
+ * (DEVICE arrays [n_tensors]; the tensors are disjoint and lie inside [0, n)).  Per element, step t:
+ *   g = grad_scale * grad;  m = b1*m + (1-b1)*g;  v = b2*v + (1-b2)*g*g
+ *   u = (m / bc1) / (sqrt(v) / sqrt(bc2) + eps) + weight_decay * w            (decoupled weight decay)
+ *   r_l = ||w_l|| / ||u_l|| if both norms > 0, else 1                          (norms over the old w)
+ *   w = w - lr * r_l * u;  param_bf16 = rn_bf16(w)  (param_bf16 may be NULL)
+ * with bc1 = 1 - b1^t, bc2 = 1 - b2^t in double.  No ratio clamp, no exclusions; NaN and Inf propagate.
+ * The betas come as their complements one_minus_beta1 = 1 - b1, one_minus_beta2 = 1 - b2 (each in (0, 1]): fp32
+ * holds 1 - b to full precision where 1 - fp32(0.999) is 1.3e-5 off 0.001; b = 1 - (1 - b) is formed in double.
+ * Two launches: moments + per-chunk partial norms, then trust ratios + update.  Each tensor is cut into chunks of
+ * LIREC_LAMB_CHUNK floats; the norms are summed in a fixed order (fp64 across chunks, no atomics), so results are
+ * bitwise reproducible.  `partials` is caller-owned device scratch of n_partials chunk entries of two doubles,
+ * n_partials >= LIREC_LAMB_PARTIALS(n, n_tensors).  trust_out (optional, DEVICE [n_tensors]) receives every r_l.
+ * A tensor of length <= 0 is empty: nothing is read or written for it and its r_l is 1.  Floats outside every
+ * tensor (the padding between segments) are neither read into a norm nor written.                           */
+#define LIREC_LAMB_CHUNK 8192
+#define LIREC_LAMB_PARTIALS(n, n_tensors) ((n) / LIREC_LAMB_CHUNK + (n_tensors))
+int lirec_lamb_flat(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, void* param_bf16,
+                    const int64_t* tensor_begin, const int64_t* tensor_len, int32_t n_tensors, int64_t n,
+                    double* partials, int64_t n_partials, float lr, float one_minus_beta1,
+                    float one_minus_beta2, float eps, float weight_decay, int32_t step, float grad_scale,
+                    float* trust_out, void* stream);
+
 /* ---- data parallel: in-switch gradient exchange, bucket by bucket --------
  * Replaces ncclAllReduce(flat gradient) of a data-parallel step (the reference is single-process, SURVEY.md
  * §2.3; the optimizer stays torch.optim.Adam's arithmetic, mlp/model.py:599-601, through lirec_adam_flat on the

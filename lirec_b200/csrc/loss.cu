@@ -595,6 +595,199 @@ adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restric
   }
 }
 
+// ---- LAMB (You et al., ICLR 2020) over the flat buffer: Adam moments, decoupled weight decay, per-tensor trust ratio
+// Every tensor l of the table is cut into chunks of LIREC_LAMB_CHUNK floats that never cross its end; chunks are
+// numbered tensor by tensor in table order.  One CTA per chunk in both passes:
+//   lamb_moments_kernel: m, v <- Adam moments of g = grad_scale * grad; u = lamb_u(m, v, w);
+//                        partials[chunk] = (sum w^2, sum u^2) over the chunk
+//   lamb_apply_kernel  : r_l = ||w_l|| / ||u_l|| from tensor l's partials (1 unless both are > 0);
+//                        w <- w - lr * r_l * u, bf16 shadow <- rn_bf16(w)
+// Pass 2 recomputes u from the stored moments and the old w with the same helper, so the norm is the norm of the u
+// that is applied.  Sums run in a fixed order that depends only on the chunk size and the CTA size, never on the
+// grid: per thread over its elements, a shuffle butterfly, the warps in order; across chunks in fp64, contiguous runs
+// of chunks per thread in chunk order, then the same butterfly and warp order.  No float atomics.
+constexpr int LAMB_THREADS = 256;
+
+// u of one element.  Explicit round-to-nearest intrinsics: the compiler may not contract or reorder them, so both
+// passes compute the same bits.
+__device__ __forceinline__ float lamb_u(float m, float v, float w, float inv_bc1, float inv_bc2_sqrt, float eps,
+                                        float wd) {
+  const float den = __fadd_rn(__fmul_rn(__fsqrt_rn(v), inv_bc2_sqrt), eps);
+  return __fadd_rn(__fdiv_rn(__fmul_rn(m, inv_bc1), den), __fmul_rn(wd, w));
+}
+
+__device__ __forceinline__ int64_t lamb_chunks(int64_t len) {
+  return len > 0 ? (len + LIREC_LAMB_CHUNK - 1) / LIREC_LAMB_CHUNK : 1;  // an empty tensor keeps one (empty) chunk
+}
+
+struct LambChunk {
+  int l;              // tensor, -1 past the last chunk
+  int64_t k;          // chunk within the tensor
+  int64_t base, cnt;  // the tensor's first chunk and its chunk count
+};
+
+// The tensor that owns chunk c: a block-wide scan of the chunk counts, 256 table entries at a time.  All threads.
+__device__ LambChunk lamb_locate(const int64_t* __restrict__ len, int n_tensors, int64_t c) {
+  __shared__ long long s_warp[LAMB_THREADS / 32];
+  __shared__ LambChunk s_hit;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (threadIdx.x == 0) s_hit.l = -1;
+  long long carry = 0;
+  for (int t0 = 0; t0 < n_tensors; t0 += LAMB_THREADS) {
+    const int l = t0 + static_cast<int>(threadIdx.x);
+    const long long cnt = l < n_tensors ? lamb_chunks(len[l]) : 0;
+    long long x = cnt;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const long long y = __shfl_up_sync(0xffffffffu, x, o);
+      if (lane >= o) x += y;
+    }
+    if (lane == 31) s_warp[warp] = x;
+    __syncthreads();
+    long long before = carry, total = 0;
+#pragma unroll
+    for (int w = 0; w < LAMB_THREADS / 32; ++w) {
+      if (w < warp) before += s_warp[w];
+      total += s_warp[w];
+    }
+    const long long excl = before + x - cnt;
+    if (l < n_tensors && c >= excl && c < excl + cnt) s_hit = LambChunk{l, c - excl, excl, cnt};
+    carry += total;
+    __syncthreads();
+    if (s_hit.l >= 0 || c < carry) break;
+  }
+  return s_hit;
+}
+
+__device__ __forceinline__ double2 lamb_block_sum2(double a, double b) {
+  __shared__ double2 s_red[LAMB_THREADS / 32];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    a += __shfl_xor_sync(0xffffffffu, a, o);
+    b += __shfl_xor_sync(0xffffffffu, b, o);
+  }
+  if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = make_double2(a, b);
+  __syncthreads();
+  double2 t = make_double2(0.0, 0.0);
+#pragma unroll
+  for (int w = 0; w < LAMB_THREADS / 32; ++w) {
+    t.x += s_red[w].x;
+    t.y += s_red[w].y;
+  }
+  return t;
+}
+
+// [off, off + n) of the flat buffers: the chunk this CTA owns.
+__device__ __forceinline__ int lamb_chunk_span(const int64_t* __restrict__ begin, const int64_t* __restrict__ len,
+                                               const LambChunk& ch, int64_t* off) {
+  const int64_t l = len[ch.l];
+  *off = begin[ch.l] + ch.k * LIREC_LAMB_CHUNK;
+  return l > 0 ? static_cast<int>(min(static_cast<int64_t>(LIREC_LAMB_CHUNK), l - ch.k * LIREC_LAMB_CHUNK)) : 0;
+}
+
+__global__ void __launch_bounds__(LAMB_THREADS)
+lamb_moments_kernel(const float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
+                    float* __restrict__ v, const int64_t* __restrict__ begin, const int64_t* __restrict__ len,
+                    int n_tensors, double2* __restrict__ partials, float beta1, float beta2, float c1, float c2,
+                    float eps, float wd, float inv_bc1, float inv_bc2_sqrt, float grad_scale) {
+  pdl_wait();
+  pdl_trigger();
+  const LambChunk ch = lamb_locate(len, n_tensors, blockIdx.x);
+  if (ch.l < 0) return;
+  int64_t off;
+  const int n = lamb_chunk_span(begin, len, ch, &off);
+  const float* pc = p + off; const float* gc = g + off; float* mc = m + off; float* vc = v + off;
+  const bool vec = ((reinterpret_cast<uintptr_t>(pc) | reinterpret_cast<uintptr_t>(gc) |
+                     reinterpret_cast<uintptr_t>(mc) | reinterpret_cast<uintptr_t>(vc)) & 15) == 0;
+  const int n4 = vec ? n / 4 : 0;
+  float sw = 0.f, su = 0.f;
+  for (int i = threadIdx.x; i < n4; i += LAMB_THREADS) {
+    const float4 pv = reinterpret_cast<const float4*>(pc)[i];
+    const float4 gr = reinterpret_cast<const float4*>(gc)[i];
+    float4 mv = reinterpret_cast<const float4*>(mc)[i];
+    float4 vv = reinterpret_cast<const float4*>(vc)[i];
+    const float* pp = &pv.x; const float* gg = &gr.x; float* mm = &mv.x; float* vp = &vv.x;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const float gv = gg[k] * grad_scale;
+      mm[k] = beta1 * mm[k] + c1 * gv;
+      vp[k] = beta2 * vp[k] + c2 * gv * gv;
+      const float u = lamb_u(mm[k], vp[k], pp[k], inv_bc1, inv_bc2_sqrt, eps, wd);
+      sw += pp[k] * pp[k];
+      su += u * u;
+    }
+    reinterpret_cast<float4*>(mc)[i] = mv;
+    reinterpret_cast<float4*>(vc)[i] = vv;
+  }
+  for (int i = 4 * n4 + threadIdx.x; i < n; i += LAMB_THREADS) {
+    const float pv = pc[i];
+    const float gv = gc[i] * grad_scale;
+    const float mv = beta1 * mc[i] + c1 * gv;
+    const float vv = beta2 * vc[i] + c2 * gv * gv;
+    mc[i] = mv;
+    vc[i] = vv;
+    const float u = lamb_u(mv, vv, pv, inv_bc1, inv_bc2_sqrt, eps, wd);
+    sw += pv * pv;
+    su += u * u;
+  }
+  const double2 s = lamb_block_sum2(sw, su);
+  if (threadIdx.x == 0) partials[blockIdx.x] = s;
+}
+
+__global__ void __launch_bounds__(LAMB_THREADS)
+lamb_apply_kernel(float* __restrict__ p, const float* __restrict__ m, const float* __restrict__ v,
+                  __nv_bfloat16* __restrict__ pb, const int64_t* __restrict__ begin, const int64_t* __restrict__ len,
+                  int n_tensors, const double2* __restrict__ partials, float* __restrict__ trust_out, float lr,
+                  float eps, float wd, float inv_bc1, float inv_bc2_sqrt) {
+  pdl_wait();
+  pdl_trigger();
+  const LambChunk ch = lamb_locate(len, n_tensors, blockIdx.x);
+  if (ch.l < 0) return;
+  // trust ratio of the tensor: thread t sums a contiguous run of its chunks' partials in chunk order
+  const int64_t run = (ch.cnt + LAMB_THREADS - 1) / LAMB_THREADS;
+  const int64_t j0 = min(ch.cnt, run * threadIdx.x), j1 = min(ch.cnt, j0 + run);
+  double sw = 0.0, su = 0.0;
+  for (int64_t j = j0; j < j1; ++j) {
+    const double2 q = partials[ch.base + j];
+    sw += q.x;
+    su += q.y;
+  }
+  const double2 s = lamb_block_sum2(sw, su);
+  const double r = (s.x > 0.0 && s.y > 0.0) ? sqrt(s.x) / sqrt(s.y) : 1.0;
+  if (trust_out && ch.k == 0 && threadIdx.x == 0) trust_out[ch.l] = static_cast<float>(r);
+  const float step = static_cast<float>(static_cast<double>(lr) * r);
+
+  int64_t off;
+  const int n = lamb_chunk_span(begin, len, ch, &off);
+  float* pc = p + off; const float* mc = m + off; const float* vc = v + off;
+  __nv_bfloat16* bc = pb ? pb + off : nullptr;
+  const bool vec = ((reinterpret_cast<uintptr_t>(pc) | reinterpret_cast<uintptr_t>(mc) |
+                     reinterpret_cast<uintptr_t>(vc)) & 15) == 0 && (reinterpret_cast<uintptr_t>(bc) & 7) == 0;
+  const int n4 = vec ? n / 4 : 0;
+  for (int i = threadIdx.x; i < n4; i += LAMB_THREADS) {
+    float4 pv = reinterpret_cast<const float4*>(pc)[i];
+    const float4 mv = reinterpret_cast<const float4*>(mc)[i];
+    const float4 vv = reinterpret_cast<const float4*>(vc)[i];
+    float* pp = &pv.x; const float* mm = &mv.x; const float* vp = &vv.x;
+#pragma unroll
+    for (int k = 0; k < 4; ++k)
+      pp[k] = __fsub_rn(pp[k], __fmul_rn(step, lamb_u(mm[k], vp[k], pp[k], inv_bc1, inv_bc2_sqrt, eps, wd)));
+    reinterpret_cast<float4*>(pc)[i] = pv;
+    if (bc) {
+      const __nv_bfloat162 lo = __floats2bfloat162_rn(pv.x, pv.y), hi = __floats2bfloat162_rn(pv.z, pv.w);
+      uint2 w;
+      w.x = *reinterpret_cast<const uint32_t*>(&lo);
+      w.y = *reinterpret_cast<const uint32_t*>(&hi);
+      reinterpret_cast<uint2*>(bc)[i] = w;
+    }
+  }
+  for (int i = 4 * n4 + threadIdx.x; i < n; i += LAMB_THREADS) {
+    const float pv = __fsub_rn(pc[i], __fmul_rn(step, lamb_u(mc[i], vc[i], pc[i], inv_bc1, inv_bc2_sqrt, eps, wd)));
+    pc[i] = pv;
+    if (bc) bc[i] = __float2bfloat16_rn(pv);
+  }
+}
+
 }  // namespace loss
 }  // namespace lirec
 
@@ -716,5 +909,44 @@ extern "C" int lirec_adam_flat(float* param, const float* grad, float* exp_avg, 
                            exp_avg, exp_avg_sq, reinterpret_cast<__nv_bfloat16*>(param_bf16), n, lr, beta1, beta2, eps,
                            weight_decay, bc1, sqrtf(bc2), grad_scale));
   note_launch();
+  return LIREC_OK;
+}
+
+extern "C" int lirec_lamb_flat(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, void* param_bf16,
+                               const int64_t* tensor_begin, const int64_t* tensor_len, int32_t n_tensors, int64_t n,
+                               double* partials, int64_t n_partials, float lr, float one_minus_beta1,
+                               float one_minus_beta2, float eps, float weight_decay, int32_t step, float grad_scale,
+                               float* trust_out, void* stream) {
+  LIREC_ENTER();
+  LIREC_REQUIRE(param && grad && exp_avg && exp_avg_sq && tensor_begin && tensor_len && partials,
+                "lamb: null pointer");
+  LIREC_REQUIRE(step >= 1, "lamb: step=%d (the first step is 1)", step);
+  LIREC_REQUIRE(n_tensors >= 1 && n >= 1, "lamb: n_tensors=%d n=%lld", n_tensors, static_cast<long long>(n));
+  const int64_t chunks = LIREC_LAMB_PARTIALS(n, n_tensors);
+  LIREC_REQUIRE(n_partials >= chunks, "lamb: partials hold %lld chunks, %lld needed", static_cast<long long>(n_partials),
+                static_cast<long long>(chunks));
+  LIREC_REQUIRE(chunks <= 0x7fffffff, "lamb: %lld chunks", static_cast<long long>(chunks));
+  LIREC_REQUIRE(one_minus_beta1 > 0.f && one_minus_beta1 <= 1.f && one_minus_beta2 > 0.f && one_minus_beta2 <= 1.f,
+                "lamb: 1 - beta1 = %g, 1 - beta2 = %g (each in (0, 1])", one_minus_beta1, one_minus_beta2);
+  // beta = 1 - (1 - beta) in double: the complement carries the digits that an fp32 beta near 1 drops
+  // (fp32 1 - fp32(0.999) is 1.3e-5 off 0.001), and beta formed from it is exact to fp32 rounding
+  const double b1 = 1.0 - static_cast<double>(one_minus_beta1), b2 = 1.0 - static_cast<double>(one_minus_beta2);
+  // bias corrections in double like lirec_adam_flat
+  const double bc1 = 1.0 - pow(b1, static_cast<double>(step));
+  const double bc2 = 1.0 - pow(b2, static_cast<double>(step));
+  const float inv_bc1 = static_cast<float>(1.0 / bc1), inv_bc2_sqrt = static_cast<float>(1.0 / sqrt(bc2));
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  double2* part = reinterpret_cast<double2*>(partials);
+  // one CTA per chunk; the bound leaves at most n_tensors CTAs without a chunk, and they return at once
+  const dim3 grid(static_cast<unsigned>(chunks));
+  LIREC_CUDA_OK(launch_pdl(loss::lamb_moments_kernel, grid, dim3(loss::LAMB_THREADS), 0, s, param, grad, exp_avg,
+                           exp_avg_sq, tensor_begin, tensor_len, n_tensors, part, static_cast<float>(b1),
+                           static_cast<float>(b2), one_minus_beta1, one_minus_beta2, eps, weight_decay, inv_bc1,
+                           inv_bc2_sqrt, grad_scale));
+  LIREC_CUDA_OK(launch_pdl(loss::lamb_apply_kernel, grid, dim3(loss::LAMB_THREADS), 0, s, param, exp_avg, exp_avg_sq,
+                           reinterpret_cast<__nv_bfloat16*>(param_bf16), tensor_begin, tensor_len, n_tensors,
+                           static_cast<const double2*>(part), trust_out, lr, eps, weight_decay, inv_bc1,
+                           inv_bc2_sqrt));
+  note_launch(2);
   return LIREC_OK;
 }

@@ -312,14 +312,14 @@ def reduce_and_step(model, optimizer, fused=None, local_clips=None, global_clips
         fused.step(local_clips, global_clips)
         return
     if world_size() > 1:
-        from lirec_b200.mlp.model import FlatAdam
-        if isinstance(optimizer, FlatAdam):
+        from lirec_b200.mlp.model import _FlatOptimizer
+        if isinstance(optimizer, _FlatOptimizer):        # FlatAdam, FlatLamb: the average rides in grad_scale
             optimizer.step(grad_scale=allreduce_flat_grad(model._flat_grad, local_clips, global_clips))
         else:
             allreduce_flat_grad(model._flat_grad, local_clips, global_clips, average_in_place=True)
             optimizer.step()
     else:
-        step = getattr(optimizer, "_step_impl", None)       # FlatAdam: skip the Optimizer.step hook wrapper
+        step = getattr(optimizer, "_step_impl", None)       # FlatAdam / FlatLamb: skip the Optimizer.step hook wrapper
         if step is not None:
             step()
         else:

@@ -21,7 +21,8 @@ from lirec_b200.utils.arg_pars import opt
 
 __all__ = ["Modalities", "MidFusionMultiClip", "MidFusionMultiClipMaxTracks", "GatingUnit",
            "MultiTaskCrossEntropyLoss", "MultiTaskMaxMargin", "MaxMarginCrossEntropyLoss", "MarginLoss",
-           "MarginTrackRelsLoss", "MultiLabelBCELoss", "TrackBCELoss", "create_model", "ModelOutput", "FlatAdam"]
+           "MarginTrackRelsLoss", "MultiLabelBCELoss", "TrackBCELoss", "create_model", "ModelOutput", "FlatAdam",
+           "FlatLamb"]
 
 _SLOTS = ("txt", "vis", "tracks1", "tracks2")
 _SECOND = ("txt2", "vis2", "tracks12", "tracks22")
@@ -782,15 +783,15 @@ def train_step(model, loss, x, seed=None):
 # =================================================================================================
 # optimizer + factory
 # =================================================================================================
-class FlatAdam(torch.optim.Optimizer):
-    """torch.optim.Adam semantics (coupled L2, reference mlp/model.py:599-601) as ONE fused kernel
-    over the model's flat buffers; also refreshes the bf16 weight shadow.  state_dict() has the
-    layout of torch.optim.Adam (per-parameter 'step', 'exp_avg', 'exp_avg_sq')."""
+class _FlatOptimizer(torch.optim.Optimizer):
+    """What FlatAdam and FlatLamb share: Adam moments in two flat buffers laid out like the model's flat parameter
+    buffer, per-parameter state views into them, and torch.optim.Adam's state_dict layout (per-parameter 'step',
+    'exp_avg', 'exp_avg_sq').  Subclasses launch their kernel in _launch(step, grad_scale)."""
 
-    def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0):
+    def __init__(self, model, defaults):
         self.model = model
         model._sync_flat()
-        super().__init__(model._param_list, dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay))
+        super().__init__(model._param_list, defaults)
         self._m = torch.zeros_like(model._flat)
         self._v = torch.zeros_like(model._flat)
         self._t = 0
@@ -801,13 +802,11 @@ class FlatAdam(torch.optim.Optimizer):
 
     def _step_impl(self, grad_scale=1.0):
         """The step itself, without torch.optim.Optimizer's per-call hook / profiler wrapper (lirec_b200's
-        own loop calls this directly: ~25 us of host time per step at 64-clip batches)."""
-        m = self.model
-        g = self.param_groups[0]
+        own loop calls this directly: ~25 us of host time per step at 64-clip batches).  grad_scale multiplies
+        the gradients (the data-parallel 1/world average)."""
         self._t += 1
-        ops.adam_flat(m._flat, m._flat_grad, self._m, self._v, m._flat_bf16, g["lr"], g["betas"][0],
-                      g["betas"][1], g["eps"], g["weight_decay"], self._t, grad_scale)
-        m.mark_bf16_fresh()
+        self._launch(self.param_groups[0], grad_scale)
+        self.model.mark_bf16_fresh()
 
     def step(self, closure=None, grad_scale=1.0):
         self._step_impl(grad_scale)
@@ -833,7 +832,7 @@ class FlatAdam(torch.optim.Optimizer):
         return super().state_dict()
 
     def load_state_dict(self, state_dict):
-        """Accepts a torch.optim.Adam / FlatAdam state (reference checkpoints: mlp/train.py:84-106):
+        """Accepts a torch.optim.Adam / FlatAdam / FlatLamb state (reference checkpoints: mlp/train.py:84-106):
         the moments are copied into the flat buffers, which the per-parameter state keeps aliasing."""
         super().load_state_dict(state_dict)
         m, steps = self.model, []
@@ -851,8 +850,49 @@ class FlatAdam(torch.optim.Optimizer):
                 steps.append(step)
                 self.state[p] = {"step": torch.tensor(step), "exp_avg": mv, "exp_avg_sq": vv}
         if len(set(steps)) > 1:
-            raise RuntimeError("FlatAdam needs one common step count for all parameters, got %s" % sorted(set(steps)))
+            raise RuntimeError("%s needs one common step count for all parameters, got %s"
+                               % (type(self).__name__, sorted(set(steps))))
         self._t = int(steps[0]) if steps else 0
+
+
+class FlatAdam(_FlatOptimizer):
+    """torch.optim.Adam semantics (coupled L2, reference mlp/model.py:599-601) as ONE fused kernel
+    over the model's flat buffers; also refreshes the bf16 weight shadow.  state_dict() has the
+    layout of torch.optim.Adam (per-parameter 'step', 'exp_avg', 'exp_avg_sq')."""
+
+    def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0):
+        super().__init__(model, dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay))
+
+    def _launch(self, g, grad_scale):
+        m = self.model
+        ops.adam_flat(m._flat, m._flat_grad, self._m, self._v, m._flat_bf16, g["lr"], g["betas"][0],
+                      g["betas"][1], g["eps"], g["weight_decay"], self._t, grad_scale)
+
+
+class FlatLamb(_FlatOptimizer):
+    """LAMB (You et al., "Large Batch Optimization for Deep Learning", ICLR 2020) for large global batches: Adam's
+    moments, decoupled weight decay, and a trust ratio ||w|| / ||update|| per nn.Parameter, as two fused kernels
+    over the model's flat buffers (lirec_lamb_flat); also refreshes the bf16 weight shadow.  lr is read from
+    param_groups[0] every step, so torch LR schedulers apply.  state_dict() has torch.optim.Adam's layout."""
+
+    def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-6, weight_decay=0.0):
+        super().__init__(model, dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay))
+        dev = model._flat.device
+        self._begin = torch.tensor(model._offsets, dtype=torch.int64, device=dev)
+        self._len = torch.tensor([p.numel() for p in model._param_list], dtype=torch.int64, device=dev)
+        self._partials = ops.lamb_partials(model._flat.numel(), len(model._param_list), device=dev)
+        self._trust = torch.ones(len(model._param_list), dtype=torch.float32, device=dev)
+
+    def _launch(self, g, grad_scale):
+        m = self.model
+        ops.lamb_flat(m._flat, m._flat_grad, self._m, self._v, m._flat_bf16, self._begin, self._len, self._partials,
+                      g["lr"], g["betas"][0], g["betas"][1], g["eps"], g["weight_decay"], self._t, grad_scale,
+                      trust_out=self._trust)
+
+    def last_trust_ratios(self):
+        """Device float32 tensor [n_parameters]: the trust ratio each parameter got in the last step (1 before the
+        first), in model.parameters() order."""
+        return self._trust
 
 
 def _check_loss_choice():
@@ -870,10 +910,20 @@ def _check_loss_choice():
     return kind
 
 
+def _check_optimizer_choice():
+    """--optimizer (host only, before any device work)."""
+    kind = getattr(opt, "optimizer", "adam")
+    if kind not in ("adam", "lamb"):
+        raise ValueError("--optimizer must be adam or lamb (got %r)" % (kind,))
+    return kind
+
+
 def create_model(n_classes, n_rels=0):
     """Reference: mlp/model.py:578-609 — same selection logic and return triple.  --loss bce / ce swap in the
-    multi-label BCE or the softmax cross-entropy for the reference's max-margin losses."""
+    multi-label BCE or the softmax cross-entropy for the reference's max-margin losses; --optimizer lamb swaps in
+    FlatLamb for Adam."""
     loss_kind = _check_loss_choice()
+    optimizer_kind = _check_optimizer_choice()
     if opt.device != "cuda":
         raise RuntimeError("lirec_b200 runs on a B200 only (opt.device='%s'); no CPU fallback" % opt.device)
     if opt.tr_maximize:
@@ -893,7 +943,9 @@ def create_model(n_classes, n_rels=0):
     else:
         loss = MultiTaskMaxMargin(n_rels=n_rels) if opt.rels_multitask else MaxMarginCrossEntropyLoss()
 
-    if getattr(opt, "fused_adam", 0):
+    if optimizer_kind == "lamb":
+        optimizer = FlatLamb(model, lr=opt.lr, weight_decay=opt.weight_decay)
+    elif getattr(opt, "fused_adam", 0):
         optimizer = FlatAdam(model, lr=opt.lr, weight_decay=opt.weight_decay)
     else:
         model._sync_flat()

@@ -12,7 +12,7 @@ from ._ext import (ACT_NONE, ACT_RELU, ACT_TANH, OUT_F32, OUT_SPLIT, OUT_SPLIT_T
                    POST_NONE, POST_SIGN_MASK)
 
 __all__ = ["gemm_problem", "gemm_grouped", "seg_reduce", "seg_softmax_pool", "seg_softmax_pool_bwd", "SegSoftmaxPool", "rows_expand_fwd", "rows_expand_bwd", "split_f32",
-           "cast_bf16", "gather_rows", "roi_max_pool", "loss_track", "loss_rowmargin", "loss_ce", "loss_bce", "loss_bce_track", "predict_tracks", "adam_flat", "dp_exchange", "dp_reduce_adam_bcast", "dp_reduce_adam_bcast_peer", "dropout_desc"]
+           "cast_bf16", "gather_rows", "roi_max_pool", "loss_track", "loss_rowmargin", "loss_ce", "loss_bce", "loss_bce_track", "predict_tracks", "adam_flat", "lamb_partials", "lamb_flat", "dp_exchange", "dp_reduce_adam_bcast", "dp_reduce_adam_bcast_peer", "dropout_desc"]
 
 
 def dropout_desc(p=0.0, seed=0, stream_id=0, col_off=0):
@@ -294,6 +294,34 @@ def adam_flat(param, grad, exp_avg, exp_avg_sq, param_bf16, lr, beta1, beta2, ep
                                  float(lr), float(beta1), float(beta2),
                                  float(eps), float(weight_decay), int(step), float(grad_scale), int(bool(coresident)),
                                  sp))
+
+
+def lamb_partials(n, n_tensors, device=None):
+    """Scratch of lirec_lamb_flat for flat buffers of n floats cut into n_tensors tensors (LIREC_LAMB_PARTIALS)."""
+    return torch.empty(int(n) // _ext.LAMB_CHUNK + int(n_tensors), 2, dtype=torch.float64, device=device)
+
+
+def lamb_flat(param, grad, exp_avg, exp_avg_sq, param_bf16, tensor_begin, tensor_len, partials, lr, beta1, beta2, eps,
+              weight_decay, step, grad_scale=1.0, trust_out=None, stream=None):
+    """Fused LAMB step over the flat buffers (lirec_lamb_flat).  tensor_begin / tensor_len: int64 device tensors
+    [n_tensors] in floats; partials: lamb_partials(param.numel(), n_tensors); trust_out: optional float32 device
+    tensor [n_tensors] that receives the trust ratios.  The entry point takes 1 - beta, formed here in double."""
+    n_tensors = tensor_begin.numel()
+    if any(t.numel() != param.numel() for t in (grad, exp_avg, exp_avg_sq)):
+        raise ValueError("lamb_flat: param, grad, exp_avg and exp_avg_sq must have one size")
+    for t in (tensor_begin, tensor_len):
+        if t.dtype != torch.int64 or t.numel() != n_tensors or not t.is_contiguous():
+            raise ValueError("lamb_flat: tensor_begin / tensor_len must be contiguous int64 tensors of one length")
+    if partials.dtype != torch.float64 or not partials.is_contiguous():
+        raise ValueError("lamb_flat: partials must be a contiguous float64 tensor (ops.lamb_partials)")
+    if trust_out is not None and (trust_out.dtype != torch.float32 or trust_out.numel() < n_tensors):
+        raise ValueError("lamb_flat: trust_out must be float32 with one entry per tensor")
+    sp = _ext.stream_ptr() if stream is None else C.c_void_p(stream.cuda_stream)
+    _ext.check(_ext.lib().lirec_lamb_flat(
+        _ext.ptr(param), _ext.ptr(grad), _ext.ptr(exp_avg), _ext.ptr(exp_avg_sq), _ext.ptr(param_bf16),
+        _ext.ptr(tensor_begin), _ext.ptr(tensor_len), int(n_tensors), int(param.numel()), _ext.ptr(partials),
+        int(partials.numel() // 2), float(lr), 1.0 - float(beta1), 1.0 - float(beta2), float(eps), float(weight_decay),
+        int(step), float(grad_scale), _ext.ptr(trust_out), sp))
 
 
 def dp_reduce_adam_bcast(grad_mc, param, param_mc, bf16_mc, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, weight_decay,

@@ -127,6 +127,10 @@ _FLAGS = [
                     help="margin: the reference's max-margin losses; bce: multi-label sigmoid BCE (row and track "
                          "forms; --soft_gt adds the co-occurring interactions as positives); ce: softmax "
                          "cross-entropy (row models only)")),
+    ("--optimizer", dict(default="adam", choices=("adam", "lamb"),
+                         help="adam: the reference's Adam (torch.optim.Adam, or the fused kernel with --fused_adam); "
+                              "lamb: fused LAMB (layer-wise trust ratio, decoupled --weight_decay) for large global "
+                              "batches, whatever --fused_adam says")),
     ("--world_movies", dict(default=6, type=int)),
     ("--world_scenes", dict(default=40, type=int)),
 ]
