@@ -17,6 +17,9 @@ namespace loss {
 
 __device__ __forceinline__ float sigmoidf(float x) { return 1.0f / (1.0f + expf(-x)); }
 
+// softplus(x) = max(x, 0) + log1p(exp(-|x|)) stays finite and exact for logits far outside [-88, 88].
+__device__ __forceinline__ float softplusf(float x) { return fmaxf(x, 0.f) + log1pf(expf(-fabsf(x))); }
+
 __device__ __forceinline__ float block_sum(float v, float* red) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -26,6 +29,18 @@ __device__ __forceinline__ float block_sum(float v, float* red) {
   __syncthreads();
   float t = 0.f;
   for (int w = 0; w < (blockDim.x >> 5); ++w) t += red[w];  // fixed order: deterministic
+  return t;
+}
+
+__device__ __forceinline__ float block_max(float v, float* red) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  __syncthreads();
+  if (lane == 0) red[warp] = v;
+  __syncthreads();
+  float t = red[0];
+  for (int w = 1; w < (blockDim.x >> 5); ++w) t = fmaxf(t, red[w]);
   return t;
 }
 
@@ -107,14 +122,37 @@ __device__ __forceinline__ int track_assign(const float* __restrict__ xi, const 
   return s_tstar;
 }
 
-// MarginLoss (mlp/model.py:444-494) / MarginTrackRelsLoss (mlp/model.py:497-575).
-__global__ void __launch_bounds__(128)
-track_loss_kernel(const float* __restrict__ ints, const float* __restrict__ rels,
-                  const int32_t* __restrict__ cand_off, int B, const int32_t* __restrict__ labels,
-                  const int32_t* __restrict__ rels_label, const int32_t* __restrict__ gt_tracks,
-                  const uint8_t* __restrict__ multilab, lirec_track_loss_cfg cfg,
-                  float* __restrict__ loss_per_clip, int32_t* __restrict__ assign,
-                  float* __restrict__ d_ints, float* __restrict__ d_rels) {
+// The negatives of the track losses, shared by the margin loss's sum and max forms and by the BCE.
+// Interaction (t, c): a class that multilab keeps for the clip, other than the label; under tr_correct the
+// label is a positive only on the ground-truth slots, and a negative on every other slot.
+__device__ __forceinline__ bool int_negative(const uint8_t* __restrict__ ml, int t, int c, int y, int gt0, int gt1,
+                                             bool tr_correct) {
+  return ml[c] != 0 && (tr_correct ? !(c == y && (t == gt0 || t == gt1)) : c != y);
+}
+
+// Relationship (t, r) of a slot labelled lab: none when lab is None (R); otherwise every class other than lab
+// under tr_correct, and other than the ground-truth pairs' classes r0 and r1 without it.
+__device__ __forceinline__ bool rel_negative(int lab, int r, int R, int r0, int r1, bool tr_correct) {
+  return lab != R && (tr_correct ? r != lab : (r != r0 && r != r1));
+}
+
+// One CTA per clip; t* is track_assign's.  Both forms sum over the same negatives (int_negative, rel_negative).
+//   hinge (kBce = false): MarginLoss (mlp/model.py:444-494) / MarginTrackRelsLoss (mlp/model.py:497-575): one hinge
+//     m - sigma(x[t*, y]) + sigma(x[neg]) per negative, or under max_neg one per slot on its hardest negative.
+//   BCE (kBce = true): the positives are (t*, y) and (t*, c) for pos_mask[b, c] != 0, the negatives minus those
+//     positives are the zeros, and every other (slot, class) has weight 0.  The relationship positive is
+//     (t*, r0) when live.
+//   loss_per_clip = lymbda / B * sum_ints l + 1 / B * sum_rels l
+template <bool kBce>
+__device__ __forceinline__ void track_loss_body(const float* __restrict__ ints, const float* __restrict__ rels,
+                                                const int32_t* __restrict__ cand_off, int B,
+                                                const int32_t* __restrict__ labels,
+                                                const int32_t* __restrict__ rels_label,
+                                                const int32_t* __restrict__ gt_tracks,
+                                                const uint8_t* __restrict__ multilab,
+                                                const uint8_t* __restrict__ pos_mask, const lirec_track_loss_cfg& cfg,
+                                                float* __restrict__ loss_per_clip, int32_t* __restrict__ assign,
+                                                float* __restrict__ d_ints, float* __restrict__ d_rels) {
   pdl_wait();
   pdl_trigger();
   __shared__ float s_red[8];
@@ -137,26 +175,34 @@ track_loss_kernel(const float* __restrict__ ints, const float* __restrict__ rels
   float* gr = has_rels ? d_rels + static_cast<int64_t>(beg) * R : nullptr;
   const float invB = 1.0f / static_cast<float>(B);
   const int ts = track_assign(xi, xr, has_rels ? rels_label + beg : nullptr, n, C, R, y, r0, b, cfg, assign);
-  const float pos = sigmoidf(xi[static_cast<int64_t>(ts) * C + y]);
-  float pos_r = 0.f;
-  bool pos_r_live = false;
-  if (has_rels) {
-    pos_r_live = (rels_label[beg + ts] != R) && (r0 < R);
+  const bool pos_r_live = has_rels && (rels_label[beg + ts] != R) && (r0 < R);
+  float pos = 0.f, pos_r = 0.f;  // the hinge's positive scores
+  if constexpr (!kBce) {
+    pos = sigmoidf(xi[static_cast<int64_t>(ts) * C + y]);
     pos_r = pos_r_live ? sigmoidf(xr[static_cast<int64_t>(ts) * R + r0]) : 0.f;
   }
   const float mi = cfg.margin - pos, mr = cfg.margin - pos_r;
   const float wi = cfg.lymbda * invB, wr = invB;
 
   float loss_i = 0.f, cnt_i = 0.f, loss_r = 0.f, cnt_r = 0.f;
-  if (!cfg.max_neg) {
-    // ---- sum over every unmasked (slot, class) negative ----
+  if (kBce || !cfg.max_neg) {
+    // ---- sum over every (slot, class) negative, and the BCE's positives ----
     for (int e = threadIdx.x; e < n * C; e += blockDim.x) {
       const int t = e / C, c = e - t * C;
-      bool neg = multilab[static_cast<int64_t>(b) * C + c] != 0;
-      if (cfg.tr_correct) neg = neg && !(c == y && (t == gt0 || t == gt1));
-      else neg = neg && (c != y);
       float g = 0.f;
-      if (neg) {
+      if constexpr (kBce) {
+        const bool pos = (t == ts) && (c == y || (pos_mask != nullptr && pos_mask[static_cast<int64_t>(b) * C + c] != 0));
+        const bool neg = int_negative(multilab + static_cast<int64_t>(b) * C, t, c, y, gt0, gt1, cfg.tr_correct);
+        if (pos) {
+          const float v = xi[e];
+          loss_i += softplusf(-v);
+          g = wi * (sigmoidf(v) - 1.f);
+        } else if (neg) {
+          const float v = xi[e];
+          loss_i += softplusf(v);
+          g = wi * sigmoidf(v);
+        }
+      } else if (int_negative(multilab + static_cast<int64_t>(b) * C, t, c, y, gt0, gt1, cfg.tr_correct)) {
         const float s = sigmoidf(xi[e]);
         const float h = mi + s;
         if (h > 0.f) { loss_i += h; cnt_i += 1.f; g = wi * s * (1.f - s); }
@@ -166,12 +212,20 @@ track_loss_kernel(const float* __restrict__ ints, const float* __restrict__ rels
     if (has_rels) {
       for (int e = threadIdx.x; e < n * R; e += blockDim.x) {
         const int t = e / R, r = e - t * R;
-        const int lab = rels_label[beg + t];
-        bool neg = lab != R;
-        if (cfg.tr_correct) neg = neg && (r != lab);
-        else neg = neg && (r != r0) && (r != r1);
         float g = 0.f;
-        if (neg) {
+        if constexpr (kBce) {
+          const bool pos = pos_r_live && t == ts && r == r0;
+          const bool neg = rel_negative(rels_label[beg + t], r, R, r0, r1, cfg.tr_correct);
+          if (pos) {
+            const float v = xr[e];
+            loss_r += softplusf(-v);
+            g = wr * (sigmoidf(v) - 1.f);
+          } else if (neg) {
+            const float v = xr[e];
+            loss_r += softplusf(v);
+            g = wr * sigmoidf(v);
+          }
+        } else if (rel_negative(rels_label[beg + t], r, R, r0, r1, cfg.tr_correct)) {
           const float s = sigmoidf(xr[e]);
           const float h = mr + s;
           if (h > 0.f) { loss_r += h; cnt_r += 1.f; g = wr * s * (1.f - s); }
@@ -179,7 +233,7 @@ track_loss_kernel(const float* __restrict__ ints, const float* __restrict__ rels
         gr[e] = g;
       }
     }
-  } else {
+  } else if constexpr (!kBce) {
     // ---- max-negative variant: one hinge per slot on its hardest negative; the
     // reference also adds relu(m - pos) for every EMPTY slot (model.py:485-486,558-562)
     for (int e = threadIdx.x; e < n * C; e += blockDim.x) gi[e] = 0.f;
@@ -191,10 +245,7 @@ track_loss_kernel(const float* __restrict__ ints, const float* __restrict__ rels
       int bc = -1;
       if (t < n) {
         for (int c = 0; c < C; ++c) {
-          bool neg = multilab[static_cast<int64_t>(b) * C + c] != 0;
-          if (cfg.tr_correct) neg = neg && !(c == y && (t == gt0 || t == gt1));
-          else neg = neg && (c != y);
-          if (!neg) continue;
+          if (!int_negative(multilab + static_cast<int64_t>(b) * C, t, c, y, gt0, gt1, cfg.tr_correct)) continue;
           const float s = sigmoidf(xi[static_cast<int64_t>(t) * C + c]);
           if (s > best) { best = s; bc = c; }
         }
@@ -209,13 +260,10 @@ track_loss_kernel(const float* __restrict__ ints, const float* __restrict__ rels
         int br = -1;
         if (t < n) {
           const int lab = rels_label[beg + t];
-          if (lab != R) {
-            for (int r = 0; r < R; ++r) {
-              const bool neg = cfg.tr_correct ? (r != lab) : (r != r0 && r != r1);
-              if (!neg) continue;
-              const float s = sigmoidf(xr[static_cast<int64_t>(t) * R + r]);
-              if (s > bestr) { bestr = s; br = r; }
-            }
+          for (int r = 0; r < R; ++r) {
+            if (!rel_negative(lab, r, R, r0, r1, cfg.tr_correct)) continue;
+            const float s = sigmoidf(xr[static_cast<int64_t>(t) * R + r]);
+            if (s > bestr) { bestr = s; br = r; }
           }
         }
         const float hr = mr + bestr;
@@ -227,18 +275,42 @@ track_loss_kernel(const float* __restrict__ ints, const float* __restrict__ rels
     }
   }
   loss_i = block_sum(loss_i, s_red);
-  cnt_i = block_sum(cnt_i, s_red);
+  if constexpr (!kBce) cnt_i = block_sum(cnt_i, s_red);
   if (has_rels) {
     loss_r = block_sum(loss_r, s_red);
-    cnt_r = block_sum(cnt_r, s_red);
+    if constexpr (!kBce) cnt_r = block_sum(cnt_r, s_red);
   }
-  __syncthreads();
+  if constexpr (!kBce) __syncthreads();
   if (threadIdx.x == 0) {
-    // the positive receives minus the number of active hinges
-    gi[static_cast<int64_t>(ts) * C + y] += -cnt_i * wi * pos * (1.f - pos);
-    if (has_rels && pos_r_live) gr[static_cast<int64_t>(ts) * R + r0] += -cnt_r * wr * pos_r * (1.f - pos_r);
+    if constexpr (!kBce) {
+      // the positive receives minus the number of active hinges
+      gi[static_cast<int64_t>(ts) * C + y] += -cnt_i * wi * pos * (1.f - pos);
+      if (has_rels && pos_r_live) gr[static_cast<int64_t>(ts) * R + r0] += -cnt_r * wr * pos_r * (1.f - pos_r);
+    }
     loss_per_clip[b] = cfg.lymbda * loss_i * invB + loss_r * invB;
   }
+}
+
+__global__ void __launch_bounds__(128)
+track_loss_kernel(const float* __restrict__ ints, const float* __restrict__ rels,
+                  const int32_t* __restrict__ cand_off, int B, const int32_t* __restrict__ labels,
+                  const int32_t* __restrict__ rels_label, const int32_t* __restrict__ gt_tracks,
+                  const uint8_t* __restrict__ multilab, lirec_track_loss_cfg cfg,
+                  float* __restrict__ loss_per_clip, int32_t* __restrict__ assign,
+                  float* __restrict__ d_ints, float* __restrict__ d_rels) {
+  track_loss_body<false>(ints, rels, cand_off, B, labels, rels_label, gt_tracks, multilab, nullptr, cfg,
+                         loss_per_clip, assign, d_ints, d_rels);
+}
+
+__global__ void __launch_bounds__(128)
+bce_track_kernel(const float* __restrict__ ints, const float* __restrict__ rels,
+                 const int32_t* __restrict__ cand_off, int B, const int32_t* __restrict__ labels,
+                 const int32_t* __restrict__ rels_label, const int32_t* __restrict__ gt_tracks,
+                 const uint8_t* __restrict__ multilab, const uint8_t* __restrict__ pos_mask, lirec_track_loss_cfg cfg,
+                 float* __restrict__ loss_per_clip, int32_t* __restrict__ assign, float* __restrict__ d_ints,
+                 float* __restrict__ d_rels) {
+  track_loss_body<true>(ints, rels, cand_off, B, labels, rels_label, gt_tracks, multilab, pos_mask, cfg,
+                        loss_per_clip, assign, d_ints, d_rels);
 }
 
 // Row-wise hinge: MaxMarginCrossEntropyLoss (model.py:422-441) and both terms of
@@ -300,12 +372,7 @@ ce_kernel(const float* __restrict__ logits, int64_t ld, int C, const int32_t* __
   const float* x = logits + static_cast<int64_t>(b) * ld;
   float mx = -INFINITY;
   for (int c = threadIdx.x; c < C; c += blockDim.x) mx = fmaxf(mx, x[c]);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (lane == 0) s_red[warp] = mx;
-  __syncthreads();
-  mx = fmaxf(fmaxf(s_red[0], s_red[1]), fmaxf(s_red[2], s_red[3]));
+  mx = block_max(mx, s_red);
   float z = 0.f;
   for (int c = threadIdx.x; c < C; c += blockDim.x) z += expf(x[c] - mx);
   z = block_sum(z, s_red);
@@ -316,9 +383,6 @@ ce_kernel(const float* __restrict__ logits, int64_t ld, int C, const int32_t* __
 
 // ---- sigmoid binary cross-entropy (multi-label) --------------------------------------------------------
 // Per element with target t and weight w:  l = w * (t ? softplus(-x) : softplus(x)),  dl/dx = w * (sigma(x) - t).
-// softplus(x) = max(x, 0) + log1p(exp(-|x|)) stays finite and exact for logits far outside [-88, 88].
-__device__ __forceinline__ float softplusf(float x) { return fmaxf(x, 0.f) + log1pf(expf(-fabsf(x))); }
-
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -365,88 +429,6 @@ bce_rows_kernel(const float* __restrict__ logits, int64_t ld, int rows, int C, c
   }
   l = warp_sum(l);
   if (lane == 0) loss_per_row[b] = scale * l;
-}
-
-// Track form: one CTA per clip.  t* is the margin loss's assignment (track_assign); the positives are
-// (t*, y) and (t*, c) for pos_mask[b, c] != 0, the negatives are the margin loss's sum-form negatives
-// minus those positives, and every other (slot, class) has weight 0.  The relationship positive is
-// (t*, r0) when live, its negatives the margin loss's relationship negatives.
-//   loss_per_clip = lymbda / B * sum_ints l + 1 / B * sum_rels l
-__global__ void __launch_bounds__(128)
-bce_track_kernel(const float* __restrict__ ints, const float* __restrict__ rels,
-                 const int32_t* __restrict__ cand_off, int B, const int32_t* __restrict__ labels,
-                 const int32_t* __restrict__ rels_label, const int32_t* __restrict__ gt_tracks,
-                 const uint8_t* __restrict__ multilab, const uint8_t* __restrict__ pos_mask, lirec_track_loss_cfg cfg,
-                 float* __restrict__ loss_per_clip, int32_t* __restrict__ assign, float* __restrict__ d_ints,
-                 float* __restrict__ d_rels) {
-  pdl_wait();
-  pdl_trigger();
-  __shared__ float s_red[8];
-  const int b = blockIdx.x;
-  const int beg = cand_off[b], n = cand_off[b + 1] - beg;
-  const int C = cfg.n_classes, R = cfg.n_rels;
-  const bool has_rels = R > 0;
-  const int y = labels[b];
-  const int gt0 = gt_tracks[2 * b], gt1 = gt_tracks[2 * b + 1];
-  int r0 = 0, r1 = 0;
-  if (has_rels) {
-    r0 = (gt0 < n) ? rels_label[beg + gt0] : 0;
-    r1 = (gt1 < n) ? rels_label[beg + gt1] : 0;
-  }
-  const float* xi = ints + static_cast<int64_t>(beg) * C;
-  const float* xr = has_rels ? rels + static_cast<int64_t>(beg) * R : nullptr;
-  float* gi = d_ints + static_cast<int64_t>(beg) * C;
-  float* gr = has_rels ? d_rels + static_cast<int64_t>(beg) * R : nullptr;
-  const float invB = 1.0f / static_cast<float>(B);
-  const int ts = track_assign(xi, xr, has_rels ? rels_label + beg : nullptr, n, C, R, y, r0, b, cfg, assign);
-  const float wi = cfg.lymbda * invB, wr = invB;
-  const uint8_t* ml = multilab + static_cast<int64_t>(b) * C;
-  const uint8_t* pm = pos_mask ? pos_mask + static_cast<int64_t>(b) * C : nullptr;
-
-  float loss_i = 0.f, loss_r = 0.f;
-  for (int e = threadIdx.x; e < n * C; e += blockDim.x) {
-    const int t = e / C, c = e - t * C;
-    const bool pos = (t == ts) && (c == y || (pm != nullptr && pm[c] != 0));
-    bool neg = ml[c] != 0;
-    if (cfg.tr_correct) neg = neg && !(c == y && (t == gt0 || t == gt1));
-    else neg = neg && (c != y);
-    float g = 0.f;
-    if (pos) {
-      const float v = xi[e];
-      loss_i += softplusf(-v);
-      g = wi * (sigmoidf(v) - 1.f);
-    } else if (neg) {
-      const float v = xi[e];
-      loss_i += softplusf(v);
-      g = wi * sigmoidf(v);
-    }
-    gi[e] = g;
-  }
-  if (has_rels) {
-    const bool pos_r_live = (rels_label[beg + ts] != R) && (r0 < R);
-    for (int e = threadIdx.x; e < n * R; e += blockDim.x) {
-      const int t = e / R, r = e - t * R;
-      const int lab = rels_label[beg + t];
-      const bool pos = pos_r_live && t == ts && r == r0;
-      bool neg = lab != R;
-      if (cfg.tr_correct) neg = neg && (r != lab);
-      else neg = neg && (r != r0) && (r != r1);
-      float g = 0.f;
-      if (pos) {
-        const float v = xr[e];
-        loss_r += softplusf(-v);
-        g = wr * (sigmoidf(v) - 1.f);
-      } else if (neg) {
-        const float v = xr[e];
-        loss_r += softplusf(v);
-        g = wr * sigmoidf(v);
-      }
-      gr[e] = g;
-    }
-  }
-  loss_i = block_sum(loss_i, s_red);
-  if (has_rels) loss_r = block_sum(loss_r, s_red);
-  if (threadIdx.x == 0) loss_per_clip[b] = cfg.lymbda * loss_i * invB + loss_r * invB;
 }
 
 // Prediction arg-maxes of the evaluation loop (reference utils/evaluation.py:114-175, 179-271), one CTA
@@ -793,19 +775,30 @@ lamb_apply_kernel(float* __restrict__ p, const float* __restrict__ m, const floa
 
 using namespace lirec;
 
+// The arguments both track-loss entry points take; `what` names the loss in the error.
+static int check_track_loss_args(const char* what, const float* ints, const float* rels, const int32_t* cand_off,
+                                 const int32_t* labels, const int32_t* rels_label, const int32_t* gt_tracks,
+                                 const uint8_t* multilab, const lirec_track_loss_cfg& cfg, const float* loss_per_clip,
+                                 const int32_t* assign, const float* d_ints, const float* d_rels) {
+  LIREC_REQUIRE(ints && cand_off && labels && gt_tracks && multilab && loss_per_clip && assign && d_ints,
+                "%s: null pointer", what);
+  LIREC_REQUIRE(cfg.n_classes > 0 && cfg.n_rels >= 0, "%s: n_classes=%d n_rels=%d", what, cfg.n_classes,
+                cfg.n_rels);
+  LIREC_REQUIRE(cfg.n_rels == 0 || (rels && rels_label && d_rels), "%s: rel tensors missing", what);
+  LIREC_REQUIRE(cfg.max_slots > 0 && cfg.max_slots <= loss::MAX_SLOTS, "%s: max_slots=%d (limit %d)", what,
+                cfg.max_slots, loss::MAX_SLOTS);
+  return LIREC_OK;
+}
+
 extern "C" int lirec_loss_track_fwd_bwd(const float* ints, const float* rels, const int32_t* cand_off,
                                         int32_t B, const int32_t* labels, const int32_t* rels_label,
                                         const int32_t* gt_tracks, const uint8_t* multilab,
                                         lirec_track_loss_cfg cfg, float* loss_per_clip, int32_t* assign,
                                         float* d_ints, float* d_rels, void* stream) {
   LIREC_ENTER();
-  LIREC_REQUIRE(ints && cand_off && labels && gt_tracks && multilab && loss_per_clip && assign && d_ints,
-                "track loss: null pointer");
-  LIREC_REQUIRE(cfg.n_classes > 0 && cfg.n_rels >= 0, "track loss: n_classes=%d n_rels=%d", cfg.n_classes,
-                cfg.n_rels);
-  LIREC_REQUIRE(cfg.n_rels == 0 || (rels && rels_label && d_rels), "track loss: rel tensors missing");
-  LIREC_REQUIRE(cfg.max_slots > 0 && cfg.max_slots <= loss::MAX_SLOTS, "track loss: max_slots=%d (limit %d)",
-                cfg.max_slots, loss::MAX_SLOTS);
+  const int rc = check_track_loss_args("track loss", ints, rels, cand_off, labels, rels_label, gt_tracks, multilab,
+                                       cfg, loss_per_clip, assign, d_ints, d_rels);
+  if (rc != LIREC_OK) return rc;
   if (B <= 0) return LIREC_OK;
   LIREC_CUDA_OK(launch_pdl(loss::track_loss_kernel, dim3(B), dim3(128), 0, static_cast<cudaStream_t>(stream), ints, rels,
                            cand_off, B, labels, rels_label, gt_tracks, multilab, cfg, loss_per_clip, assign, d_ints,
@@ -860,14 +853,10 @@ extern "C" int lirec_loss_bce_track_fwd_bwd(const float* ints, const float* rels
                                             float* loss_per_clip, int32_t* assign, float* d_ints, float* d_rels,
                                             void* stream) {
   LIREC_ENTER();
-  LIREC_REQUIRE(ints && cand_off && labels && gt_tracks && multilab && loss_per_clip && assign && d_ints,
-                "bce track loss: null pointer");
-  LIREC_REQUIRE(cfg.n_classes > 0 && cfg.n_rels >= 0, "bce track loss: n_classes=%d n_rels=%d", cfg.n_classes,
-                cfg.n_rels);
-  LIREC_REQUIRE(cfg.n_rels == 0 || (rels && rels_label && d_rels), "bce track loss: rel tensors missing");
+  const int rc = check_track_loss_args("bce track loss", ints, rels, cand_off, labels, rels_label, gt_tracks,
+                                       multilab, cfg, loss_per_clip, assign, d_ints, d_rels);
+  if (rc != LIREC_OK) return rc;
   LIREC_REQUIRE(!cfg.max_neg, "bce track loss: max_neg is a hinge variant, the BCE has no max-negative form");
-  LIREC_REQUIRE(cfg.max_slots > 0 && cfg.max_slots <= loss::MAX_SLOTS, "bce track loss: max_slots=%d (limit %d)",
-                cfg.max_slots, loss::MAX_SLOTS);
   if (B <= 0) return LIREC_OK;
   LIREC_CUDA_OK(launch_pdl(loss::bce_track_kernel, dim3(B), dim3(128), 0, static_cast<cudaStream_t>(stream), ints, rels,
                            cand_off, B, labels, rels_label, gt_tracks, multilab, pos_mask, cfg, loss_per_clip, assign,

@@ -498,6 +498,10 @@ class _FusedLoss(nn.Module):
     def terms_and_grads(self, x, args):
         raise NotImplementedError
 
+    def has_rel_term(self):
+        """Whether terms_and_grads runs the relationship term of the multi-task losses (`_rel_term`)."""
+        return False
+
     def forward(self, x, args):
         terms, d_i, d_r = self.terms_and_grads(x, args)
         grads, logits = [], []
@@ -531,18 +535,24 @@ def _rel_term(loss_mod, pb, n_sel, run):
     return t * scale, d * scale
 
 
+def _labelled_rel_term(loss_mod, pb, kernel):
+    """`_rel_term` over the rows whose relationship label is not None (`loss_mod.n_rels`): `kernel(labels, scale)`
+    launches the fused row kernel on the batch's labels with None mapped to -1, which it skips, and returns
+    (terms, d_rels).  The count of labelled rows comes from the host copy of the batch."""
+    host = pb.host if pb.device is not None else pb
+    n_sel = int((host["rels_label"] != loss_mod.n_rels).sum())
+
+    def run(scale):
+        sel = pb["rels_label"].clone()
+        sel[sel == loss_mod.n_rels] = -1                 # rows labelled None are skipped (model.py:369, 406)
+        return kernel(sel, scale)
+    return _rel_term(loss_mod, pb, n_sel, run)
+
+
 def dp_empty_shard_collectives(loss_mod, device):
     """The collectives a loss would have issued on a rank that holds an EmptyShard this step: the one all_reduce of
-    `_rel_term`, issued by the multi-task losses whenever their relationship term runs."""
-    if int(getattr(loss_mod, "_dp_world", 1) or 1) <= 1:
-        return
-    if isinstance(loss_mod, MultiTaskCrossEntropyLoss):
-        rel_term = not opt.mod_check and opt.ctx == 1      # the model has relationship logits (Modalities has none)
-    elif isinstance(loss_mod, MultiLabelBCELoss):
-        rel_term = bool(loss_mod.n_rels) and opt.ctx == 1
-    else:
-        rel_term = isinstance(loss_mod, MultiTaskMaxMargin) and opt.ctx == 1
-    if rel_term:
+    `_rel_term`, issued whenever the loss has a relationship term."""
+    if int(getattr(loss_mod, "_dp_world", 1) or 1) > 1 and loss_mod.has_rel_term():
         import torch.distributed as dist
         dist.all_reduce(torch.zeros(1, dtype=torch.float32, device=device))
 
@@ -569,6 +579,9 @@ class MultiTaskMaxMargin(_FusedLoss):
         self.m = opt.margin
         self.n_rels = n_rels
 
+    def has_rel_term(self):
+        return opt.ctx == 1
+
     def terms_and_grads(self, x, args):
         pb = _batch_of(x, args)
         terms, d_i, d_r = [], None, None
@@ -576,23 +589,17 @@ class MultiTaskMaxMargin(_FusedLoss):
             li = x.ragged_inters
             t, d_i = ops.loss_rowmargin(li, pb["labels"], pb.multilab, self.m, opt.lymbda / li.shape[0])
             terms.append(t)
-        if opt.ctx == 1:
+        if self.has_rel_term():
             lr = x.ragged_rels
-            host = pb.host if pb.device is not None else pb
-            lab = host["rels_label"]
-            n_sel = int((lab != self.n_rels).sum())
-
-            def run(scale):
-                sel = pb["rels_label"].clone()
-                sel[sel == self.n_rels] = -1                     # rows labelled None are skipped (model.py:406)
-                return ops.loss_rowmargin(lr, sel, None, self.m, scale)
-            t, d_r = _rel_term(self, pb, n_sel, run)
+            t, d_r = _labelled_rel_term(self, pb, lambda sel, scale: ops.loss_rowmargin(lr, sel, None, self.m, scale))
             if t is not None:
                 terms.append(t)
         return torch.cat(terms), d_i, d_r
 
 
 class _TrackLoss(_FusedLoss):
+    n_rels = 0
+
     def set_rank(self, rank):
         self._seed_rank = int(rank)            # tr_cat_distr draws differ per data-parallel rank
 
@@ -601,20 +608,22 @@ class _TrackLoss(_FusedLoss):
         self._draws = getattr(self, "_draws", 0) + 1
         return int(opt.seed) * 0x9E3779B1 + self._draws * 0xC2B2AE35 + getattr(self, "_seed_rank", 0) * 0x27D4EB2F
 
-    def _run(self, x, args, n_rels, lymbda):
+    def _run(self, x, args, kernel, lymbda, **kw):
+        """terms_and_grads of a track loss: `kernel` is ops.loss_track or ops.loss_bce_track, `lymbda` the weight of
+        the interaction term and `kw` the kernel's own arguments."""
         assert opt.tr_maximize
         assert not (opt.tr_cat_distr and opt.tr_correct)                 # model.py:469, 539
         seed = self._draw_seed()
         pb = _batch_of(x, args)
+        n_rels = self.n_rels
         li, lr = x.ragged_inters, x.ragged_rels if n_rels else None
         if li is None:
-            raise ValueError("the track-assignment losses need interaction logits: opt.ints == 0 only works with "
-                             "MultiTaskMaxMargin, as in the reference (mlp/model.py:455, 507 dereference x['inters'])")
-        terms, assign, d_i, d_r = ops.loss_track(
+            raise ValueError("the track-assignment losses need interaction logits (opt.ints == 1), as in the "
+                             "reference (mlp/model.py:455, 507 dereference x['inters'])")
+        terms, assign, d_i, d_r = kernel(
             li, lr, pb["cand_off"], pb["labels"], pb["rels_label"] if n_rels else None, pb["gt_tracks"],
-            pb.multilab, self.m, lymbda, n_rels, tr_correct=opt.tr_correct,
-            max_neg=bool(opt.tr_max_neg and opt.tr_sum_max_flag), max_slots=pb.n_slots,
-            cat_distr=bool(opt.tr_cat_distr), seed=seed)
+            pb.multilab, lymbda=lymbda, n_rels=n_rels, tr_correct=opt.tr_correct, max_slots=pb.n_slots,
+            cat_distr=bool(opt.tr_cat_distr), seed=seed, **kw)
         self.last_assignment = assign
         return terms, d_i, (d_r if n_rels else None)
 
@@ -626,8 +635,9 @@ class MarginLoss(_TrackLoss):
         super().__init__()
         self.m = opt.tr_margin
 
-    def terms_and_grads(self, input, args):
-        return self._run(input, args, 0, 1.0)
+    def terms_and_grads(self, x, args):
+        return self._run(x, args, ops.loss_track, 1.0, margin=self.m,
+                         max_neg=bool(opt.tr_max_neg and opt.tr_sum_max_flag))
 
 
 class MarginTrackRelsLoss(_TrackLoss):
@@ -639,7 +649,8 @@ class MarginTrackRelsLoss(_TrackLoss):
         self.n_rels = n_rels
 
     def terms_and_grads(self, x, args):
-        return self._run(x, args, self.n_rels, opt.lymbda)
+        return self._run(x, args, ops.loss_track, opt.lymbda, margin=self.m,
+                         max_neg=bool(opt.tr_max_neg and opt.tr_sum_max_flag))
 
 
 class MultiTaskCrossEntropyLoss(_FusedLoss):
@@ -652,6 +663,9 @@ class MultiTaskCrossEntropyLoss(_FusedLoss):
         self.n_classes, self.n_rels = n_classes, n_rels
         self.weights = None if weights is None else torch.tensor(weights).float()
 
+    def has_rel_term(self):
+        return not opt.mod_check and opt.ctx == 1          # the model has relationship logits (Modalities has none)
+
     def terms_and_grads(self, x, args):
         pb = _batch_of(x, args)
         host = pb.host if pb.device is not None else pb
@@ -663,15 +677,9 @@ class MultiTaskCrossEntropyLoss(_FusedLoss):
         denom = float(self.weights[torch.as_tensor(host["labels"]).long()].sum()) if w is not None else li.shape[0]
         t, d_i = ops.loss_ce(li, lab_i, w, 1.0 / denom)
         terms, d_r = [t], None
-        if x.ragged_rels is not None:
-            lab = host["rels_label"]
-            n_sel = int((lab != self.n_rels).sum())
-
-            def run(scale):
-                sel = pb["rels_label"].clone()
-                sel[sel == self.n_rels] = -1                     # rows labelled None are skipped (model.py:369)
-                return ops.loss_ce(x.ragged_rels, sel, None, scale)
-            t, d_r = _rel_term(self, pb, n_sel, run)
+        if self.has_rel_term():
+            lr = x.ragged_rels
+            t, d_r = _labelled_rel_term(self, pb, lambda sel, scale: ops.loss_ce(lr, sel, None, scale))
             if t is not None:
                 terms.append(t)
         return torch.cat(terms), d_i, d_r
@@ -701,6 +709,9 @@ class MultiLabelBCELoss(_FusedLoss):
         super().__init__()
         self.n_rels = n_rels
 
+    def has_rel_term(self):
+        return bool(self.n_rels) and opt.ctx == 1
+
     def terms_and_grads(self, x, args):
         pb = _batch_of(x, args)
         terms, d_i, d_r = [], None, None
@@ -709,16 +720,9 @@ class MultiLabelBCELoss(_FusedLoss):
             w = (opt.lymbda if self.n_rels else 1.0) / li.shape[0]
             t, d_i = ops.loss_bce(li, pb["labels"], pb.multilab, _soft_pos(pb), w)
             terms.append(t)
-        if self.n_rels and opt.ctx == 1:
+        if self.has_rel_term():
             lr = x.ragged_rels
-            host = pb.host if pb.device is not None else pb
-            n_sel = int((host["rels_label"] != self.n_rels).sum())
-
-            def run(scale):
-                sel = pb["rels_label"].clone()
-                sel[sel == self.n_rels] = -1                     # rows labelled None are skipped
-                return ops.loss_bce(lr, sel, None, None, scale)
-            t, d_r = _rel_term(self, pb, n_sel, run)
+            t, d_r = _labelled_rel_term(self, pb, lambda sel, scale: ops.loss_bce(lr, sel, None, None, scale))
             if t is not None:
                 terms.append(t)
         return torch.cat(terms), d_i, d_r
@@ -736,20 +740,8 @@ class TrackBCELoss(_TrackLoss):
         self.n_rels = n_rels
 
     def terms_and_grads(self, x, args):
-        assert opt.tr_maximize
-        assert not (opt.tr_cat_distr and opt.tr_correct)
-        seed = self._draw_seed()
-        pb = _batch_of(x, args)
-        n_rels = self.n_rels
-        li, lr = x.ragged_inters, x.ragged_rels if n_rels else None
-        if li is None:
-            raise ValueError("TrackBCELoss needs interaction logits (opt.ints == 1)")
-        terms, assign, d_i, d_r = ops.loss_bce_track(
-            li, lr, pb["cand_off"], pb["labels"], pb["rels_label"] if n_rels else None, pb["gt_tracks"],
-            pb.multilab, _soft_pos(pb), opt.lymbda if n_rels else 1.0, n_rels, tr_correct=opt.tr_correct,
-            max_slots=pb.n_slots, cat_distr=bool(opt.tr_cat_distr), seed=seed)
-        self.last_assignment = assign
-        return terms, d_i, (d_r if n_rels else None)
+        return self._run(x, args, ops.loss_bce_track, opt.lymbda if self.n_rels else 1.0,
+                         pos_mask=_soft_pos(_batch_of(x, args)))
 
 
 def train_step(model, loss, x, seed=None):

@@ -191,26 +191,33 @@ def gather_rows(bank, idx, out=None):
     return out
 
 
-def loss_track(ints, rels, cand_off, labels, rels_label, gt_tracks, multilab, margin, lymbda, n_rels,
-               tr_correct=False, max_neg=False, max_slots=20, cat_distr=False, seed=0):
-    """Fused MarginLoss / MarginTrackRelsLoss. Returns (loss_per_clip, assign, d_ints, d_rels)."""
+def _track_loss_cfg_and_outputs(ints, rels, cand_off, margin, lymbda, n_rels, tr_correct, max_neg, max_slots,
+                                cat_distr, seed):
+    """The TrackLossCfg of both track losses and their outputs (loss_per_clip, assign, d_ints, d_rels)."""
     B = cand_off.numel() - 1
-    Ni, Cc = ints.shape
     cfg = _ext.TrackLossCfg()
     cfg.margin, cfg.lymbda = float(margin), float(lymbda)
-    cfg.n_classes, cfg.n_rels = int(Cc), int(n_rels)
+    cfg.n_classes, cfg.n_rels = int(ints.shape[1]), int(n_rels)
     cfg.tr_correct, cfg.max_neg, cfg.max_slots = int(tr_correct), int(max_neg), int(max_slots)
     cfg.cat_distr, cfg.seed = int(cat_distr), int(seed) & 0xFFFFFFFF
     loss = torch.empty(B, dtype=torch.float32, device=ints.device)
     assign = torch.empty(B, dtype=torch.int32, device=ints.device)
     d_ints = torch.empty_like(ints)
     d_rels = torch.empty_like(rels) if n_rels > 0 else None
-    L = _ext.lib()
-    _ext.check(L.lirec_loss_track_fwd_bwd(
-        _ext.ptr(ints), _ext.ptr(rels) if n_rels > 0 else None, _ext.ptr(cand_off), B, _ext.ptr(labels),
+    return cfg, (loss, assign, d_ints, d_rels)
+
+
+def loss_track(ints, rels, cand_off, labels, rels_label, gt_tracks, multilab, margin, lymbda, n_rels,
+               tr_correct=False, max_neg=False, max_slots=20, cat_distr=False, seed=0):
+    """Fused MarginLoss / MarginTrackRelsLoss. Returns (loss_per_clip, assign, d_ints, d_rels)."""
+    cfg, out = _track_loss_cfg_and_outputs(ints, rels, cand_off, margin, lymbda, n_rels, tr_correct, max_neg,
+                                           max_slots, cat_distr, seed)
+    loss, assign, d_ints, d_rels = out
+    _ext.check(_ext.lib().lirec_loss_track_fwd_bwd(
+        _ext.ptr(ints), _ext.ptr(rels) if n_rels > 0 else None, _ext.ptr(cand_off), loss.numel(), _ext.ptr(labels),
         _ext.ptr(rels_label) if n_rels > 0 else None, _ext.ptr(gt_tracks), _ext.ptr(multilab), cfg,
         _ext.ptr(loss), _ext.ptr(assign), _ext.ptr(d_ints), _ext.ptr(d_rels), _ext.stream_ptr()))
-    return loss, assign, d_ints, d_rels
+    return out
 
 
 def loss_ce(logits, labels, class_weights, scale):
@@ -240,22 +247,14 @@ def loss_bce_track(ints, rels, cand_off, labels, rels_label, gt_tracks, multilab
                    tr_correct=False, max_slots=20, cat_distr=False, seed=0):
     """Fused BCE over the weakly supervised track assignment (lirec_loss_bce_track_fwd_bwd); t* is chosen as in
     loss_track. Returns (loss_per_clip, assign, d_ints, d_rels)."""
-    B = cand_off.numel() - 1
-    Ni, Cc = ints.shape
-    cfg = _ext.TrackLossCfg()
-    cfg.margin, cfg.lymbda = 0.0, float(lymbda)
-    cfg.n_classes, cfg.n_rels = int(Cc), int(n_rels)
-    cfg.tr_correct, cfg.max_neg, cfg.max_slots = int(tr_correct), 0, int(max_slots)
-    cfg.cat_distr, cfg.seed = int(cat_distr), int(seed) & 0xFFFFFFFF
-    loss = torch.empty(B, dtype=torch.float32, device=ints.device)
-    assign = torch.empty(B, dtype=torch.int32, device=ints.device)
-    d_ints = torch.empty_like(ints)
-    d_rels = torch.empty_like(rels) if n_rels > 0 else None
+    cfg, out = _track_loss_cfg_and_outputs(ints, rels, cand_off, 0.0, lymbda, n_rels, tr_correct, False, max_slots,
+                                           cat_distr, seed)
+    loss, assign, d_ints, d_rels = out
     _ext.check(_ext.lib().lirec_loss_bce_track_fwd_bwd(
-        _ext.ptr(ints), _ext.ptr(rels) if n_rels > 0 else None, _ext.ptr(cand_off), B, _ext.ptr(labels),
+        _ext.ptr(ints), _ext.ptr(rels) if n_rels > 0 else None, _ext.ptr(cand_off), loss.numel(), _ext.ptr(labels),
         _ext.ptr(rels_label) if n_rels > 0 else None, _ext.ptr(gt_tracks), _ext.ptr(multilab), _ext.ptr(pos_mask), cfg,
         _ext.ptr(loss), _ext.ptr(assign), _ext.ptr(d_ints), _ext.ptr(d_rels), _ext.stream_ptr()))
-    return loss, assign, d_ints, d_rels
+    return out
 
 
 def loss_rowmargin(logits, labels, weights, margin, scale):
