@@ -503,6 +503,23 @@ int lirec_lamb_flat(float* param, const float* grad, float* exp_avg, float* exp_
                     float one_minus_beta2, float eps, float weight_decay, int32_t step, float grad_scale,
                     float* trust_out, void* stream);
 
+/* Global-norm gradient clipping over the flat gradient buffer, in place: torch.nn.utils.clip_grad_norm_(params,
+ * max_norm) with norm_type 2, applied to the gradient an optimizer is about to consume.  Same tensor table as
+ * lirec_lamb_flat (DEVICE arrays tensor_begin / tensor_len [n_tensors], disjoint, inside [0, n)):
+ *   norm = || grad_scale * grad ||_2 over every tensor          (grad_scale: the data-parallel 1/world average)
+ *   coef = min(max_norm / (norm + 1e-6), 1) in fp32             (a NaN norm gives a NaN coef, an Inf norm 0)
+ *   grad = grad * coef                                          (grad_scale is NOT applied: the optimizer does)
+ * When coef is exactly 1 the buffer is not written.  Three launches: per-chunk sums of squares (fp32 within a
+ * thread, fp64 across the CTA), one CTA that sums them in a fixed order in fp64 (each tensor's chunks in order, then
+ * the tensors in table order), and the scale; no host sync, no float atomics, bitwise reproducible.  `partials` is
+ * the same caller-owned scratch as lirec_lamb_flat's (n_partials entries of two doubles, n_partials >=
+ * LIREC_LAMB_PARTIALS(n, n_tensors)).  norm_out (DEVICE float, required) receives the pre-clip norm;
+ * tensor_norms_out (optional, DEVICE [n_tensors]) the pre-clip norm of every tensor.  max_norm must be finite and
+ * > 0.  Floats outside every tensor are neither read nor written.                                                 */
+int lirec_grad_clip_flat(float* grad, const int64_t* tensor_begin, const int64_t* tensor_len, int32_t n_tensors,
+                         int64_t n, double* partials, int64_t n_partials, float max_norm, float grad_scale,
+                         float* norm_out, float* tensor_norms_out, void* stream);
+
 /* ---- data parallel: in-switch gradient exchange, bucket by bucket --------
  * Replaces ncclAllReduce(flat gradient) of a data-parallel step (the reference is single-process, SURVEY.md
  * §2.3; the optimizer stays torch.optim.Adam's arithmetic, mlp/model.py:599-601, through lirec_adam_flat on the

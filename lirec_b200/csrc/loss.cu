@@ -577,47 +577,34 @@ adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restric
   }
 }
 
-// ---- LAMB (You et al., ICLR 2020) over the flat buffer: Adam moments, decoupled weight decay, per-tensor trust ratio
-// Every tensor l of the table is cut into chunks of LIREC_LAMB_CHUNK floats that never cross its end; chunks are
-// numbered tensor by tensor in table order.  One CTA per chunk in both passes:
-//   lamb_moments_kernel: m, v <- Adam moments of g = grad_scale * grad; u = lamb_u(m, v, w);
-//                        partials[chunk] = (sum w^2, sum u^2) over the chunk
-//   lamb_apply_kernel  : r_l = ||w_l|| / ||u_l|| from tensor l's partials (1 unless both are > 0);
-//                        w <- w - lr * r_l * u, bf16 shadow <- rn_bf16(w)
-// Pass 2 recomputes u from the stored moments and the old w with the same helper, so the norm is the norm of the u
-// that is applied.  Sums run in a fixed order that depends only on the chunk size and the CTA size, never on the
-// grid: per thread over its elements, a shuffle butterfly, the warps in order; across chunks in fp64, contiguous runs
-// of chunks per thread in chunk order, then the same butterfly and warp order.  No float atomics.
-constexpr int LAMB_THREADS = 256;
+// ---- Chunked passes over a tensor table of the flat buffer (LAMB, gradient clipping)
+// Every tensor l of the table (floats [begin[l], begin[l] + len[l])) is cut into chunks of LIREC_LAMB_CHUNK floats
+// that never cross its end; chunks are numbered tensor by tensor in table order, and one CTA of CHUNK_THREADS owns
+// one chunk.  Floats outside every tensor (the padding between segments) are never touched.  Sums run in a fixed
+// order that depends only on the chunk size and the CTA size, never on the grid: per thread over its elements, a
+// shuffle butterfly, the warps in order; across chunks in fp64.  No float atomics.
+constexpr int CHUNK_THREADS = 256;
 
-// u of one element.  Explicit round-to-nearest intrinsics: the compiler may not contract or reorder them, so both
-// passes compute the same bits.
-__device__ __forceinline__ float lamb_u(float m, float v, float w, float inv_bc1, float inv_bc2_sqrt, float eps,
-                                        float wd) {
-  const float den = __fadd_rn(__fmul_rn(__fsqrt_rn(v), inv_bc2_sqrt), eps);
-  return __fadd_rn(__fdiv_rn(__fmul_rn(m, inv_bc1), den), __fmul_rn(wd, w));
-}
-
-__device__ __forceinline__ int64_t lamb_chunks(int64_t len) {
+__device__ __forceinline__ int64_t flat_chunks(int64_t len) {
   return len > 0 ? (len + LIREC_LAMB_CHUNK - 1) / LIREC_LAMB_CHUNK : 1;  // an empty tensor keeps one (empty) chunk
 }
 
-struct LambChunk {
+struct FlatChunk {
   int l;              // tensor, -1 past the last chunk
   int64_t k;          // chunk within the tensor
   int64_t base, cnt;  // the tensor's first chunk and its chunk count
 };
 
 // The tensor that owns chunk c: a block-wide scan of the chunk counts, 256 table entries at a time.  All threads.
-__device__ LambChunk lamb_locate(const int64_t* __restrict__ len, int n_tensors, int64_t c) {
-  __shared__ long long s_warp[LAMB_THREADS / 32];
-  __shared__ LambChunk s_hit;
+__device__ FlatChunk flat_locate(const int64_t* __restrict__ len, int n_tensors, int64_t c) {
+  __shared__ long long s_warp[CHUNK_THREADS / 32];
+  __shared__ FlatChunk s_hit;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   if (threadIdx.x == 0) s_hit.l = -1;
   long long carry = 0;
-  for (int t0 = 0; t0 < n_tensors; t0 += LAMB_THREADS) {
+  for (int t0 = 0; t0 < n_tensors; t0 += CHUNK_THREADS) {
     const int l = t0 + static_cast<int>(threadIdx.x);
-    const long long cnt = l < n_tensors ? lamb_chunks(len[l]) : 0;
+    const long long cnt = l < n_tensors ? flat_chunks(len[l]) : 0;
     long long x = cnt;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
@@ -628,12 +615,12 @@ __device__ LambChunk lamb_locate(const int64_t* __restrict__ len, int n_tensors,
     __syncthreads();
     long long before = carry, total = 0;
 #pragma unroll
-    for (int w = 0; w < LAMB_THREADS / 32; ++w) {
+    for (int w = 0; w < CHUNK_THREADS / 32; ++w) {
       if (w < warp) before += s_warp[w];
       total += s_warp[w];
     }
     const long long excl = before + x - cnt;
-    if (l < n_tensors && c >= excl && c < excl + cnt) s_hit = LambChunk{l, c - excl, excl, cnt};
+    if (l < n_tensors && c >= excl && c < excl + cnt) s_hit = FlatChunk{l, c - excl, excl, cnt};
     carry += total;
     __syncthreads();
     if (s_hit.l >= 0 || c < carry) break;
@@ -641,8 +628,8 @@ __device__ LambChunk lamb_locate(const int64_t* __restrict__ len, int n_tensors,
   return s_hit;
 }
 
-__device__ __forceinline__ double2 lamb_block_sum2(double a, double b) {
-  __shared__ double2 s_red[LAMB_THREADS / 32];
+__device__ __forceinline__ double2 flat_block_sum2(double a, double b) {
+  __shared__ double2 s_red[CHUNK_THREADS / 32];
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     a += __shfl_xor_sync(0xffffffffu, a, o);
@@ -652,7 +639,7 @@ __device__ __forceinline__ double2 lamb_block_sum2(double a, double b) {
   __syncthreads();
   double2 t = make_double2(0.0, 0.0);
 #pragma unroll
-  for (int w = 0; w < LAMB_THREADS / 32; ++w) {
+  for (int w = 0; w < CHUNK_THREADS / 32; ++w) {
     t.x += s_red[w].x;
     t.y += s_red[w].y;
   }
@@ -660,30 +647,48 @@ __device__ __forceinline__ double2 lamb_block_sum2(double a, double b) {
 }
 
 // [off, off + n) of the flat buffers: the chunk this CTA owns.
-__device__ __forceinline__ int lamb_chunk_span(const int64_t* __restrict__ begin, const int64_t* __restrict__ len,
-                                               const LambChunk& ch, int64_t* off) {
+__device__ __forceinline__ int flat_chunk_span(const int64_t* __restrict__ begin, const int64_t* __restrict__ len,
+                                               const FlatChunk& ch, int64_t* off) {
   const int64_t l = len[ch.l];
   *off = begin[ch.l] + ch.k * LIREC_LAMB_CHUNK;
   return l > 0 ? static_cast<int>(min(static_cast<int64_t>(LIREC_LAMB_CHUNK), l - ch.k * LIREC_LAMB_CHUNK)) : 0;
 }
 
-__global__ void __launch_bounds__(LAMB_THREADS)
+// ---- LAMB (You et al., ICLR 2020) over the flat buffer: Adam moments, decoupled weight decay, per-tensor trust ratio
+// One CTA per chunk in both passes:
+//   lamb_moments_kernel: m, v <- Adam moments of g = grad_scale * grad; u = lamb_u(m, v, w);
+//                        partials[chunk] = (sum w^2, sum u^2) over the chunk
+//   lamb_apply_kernel  : r_l = ||w_l|| / ||u_l|| from tensor l's partials (1 unless both are > 0);
+//                        w <- w - lr * r_l * u, bf16 shadow <- rn_bf16(w)
+// Pass 2 recomputes u from the stored moments and the old w with the same helper, so the norm is the norm of the u
+// that is applied.  Across chunks, thread t sums a contiguous run of the tensor's partials in chunk order, then the
+// block sum.
+
+// u of one element.  Explicit round-to-nearest intrinsics: the compiler may not contract or reorder them, so both
+// passes compute the same bits.
+__device__ __forceinline__ float lamb_u(float m, float v, float w, float inv_bc1, float inv_bc2_sqrt, float eps,
+                                        float wd) {
+  const float den = __fadd_rn(__fmul_rn(__fsqrt_rn(v), inv_bc2_sqrt), eps);
+  return __fadd_rn(__fdiv_rn(__fmul_rn(m, inv_bc1), den), __fmul_rn(wd, w));
+}
+
+__global__ void __launch_bounds__(CHUNK_THREADS)
 lamb_moments_kernel(const float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                     float* __restrict__ v, const int64_t* __restrict__ begin, const int64_t* __restrict__ len,
                     int n_tensors, double2* __restrict__ partials, float beta1, float beta2, float c1, float c2,
                     float eps, float wd, float inv_bc1, float inv_bc2_sqrt, float grad_scale) {
   pdl_wait();
   pdl_trigger();
-  const LambChunk ch = lamb_locate(len, n_tensors, blockIdx.x);
+  const FlatChunk ch = flat_locate(len, n_tensors, blockIdx.x);
   if (ch.l < 0) return;
   int64_t off;
-  const int n = lamb_chunk_span(begin, len, ch, &off);
+  const int n = flat_chunk_span(begin, len, ch, &off);
   const float* pc = p + off; const float* gc = g + off; float* mc = m + off; float* vc = v + off;
   const bool vec = ((reinterpret_cast<uintptr_t>(pc) | reinterpret_cast<uintptr_t>(gc) |
                      reinterpret_cast<uintptr_t>(mc) | reinterpret_cast<uintptr_t>(vc)) & 15) == 0;
   const int n4 = vec ? n / 4 : 0;
   float sw = 0.f, su = 0.f;
-  for (int i = threadIdx.x; i < n4; i += LAMB_THREADS) {
+  for (int i = threadIdx.x; i < n4; i += CHUNK_THREADS) {
     const float4 pv = reinterpret_cast<const float4*>(pc)[i];
     const float4 gr = reinterpret_cast<const float4*>(gc)[i];
     float4 mv = reinterpret_cast<const float4*>(mc)[i];
@@ -701,7 +706,7 @@ lamb_moments_kernel(const float* __restrict__ p, const float* __restrict__ g, fl
     reinterpret_cast<float4*>(mc)[i] = mv;
     reinterpret_cast<float4*>(vc)[i] = vv;
   }
-  for (int i = 4 * n4 + threadIdx.x; i < n; i += LAMB_THREADS) {
+  for (int i = 4 * n4 + threadIdx.x; i < n; i += CHUNK_THREADS) {
     const float pv = pc[i];
     const float gv = gc[i] * grad_scale;
     const float mv = beta1 * mc[i] + c1 * gv;
@@ -712,21 +717,21 @@ lamb_moments_kernel(const float* __restrict__ p, const float* __restrict__ g, fl
     sw += pv * pv;
     su += u * u;
   }
-  const double2 s = lamb_block_sum2(sw, su);
+  const double2 s = flat_block_sum2(sw, su);
   if (threadIdx.x == 0) partials[blockIdx.x] = s;
 }
 
-__global__ void __launch_bounds__(LAMB_THREADS)
+__global__ void __launch_bounds__(CHUNK_THREADS)
 lamb_apply_kernel(float* __restrict__ p, const float* __restrict__ m, const float* __restrict__ v,
                   __nv_bfloat16* __restrict__ pb, const int64_t* __restrict__ begin, const int64_t* __restrict__ len,
                   int n_tensors, const double2* __restrict__ partials, float* __restrict__ trust_out, float lr,
                   float eps, float wd, float inv_bc1, float inv_bc2_sqrt) {
   pdl_wait();
   pdl_trigger();
-  const LambChunk ch = lamb_locate(len, n_tensors, blockIdx.x);
+  const FlatChunk ch = flat_locate(len, n_tensors, blockIdx.x);
   if (ch.l < 0) return;
   // trust ratio of the tensor: thread t sums a contiguous run of its chunks' partials in chunk order
-  const int64_t run = (ch.cnt + LAMB_THREADS - 1) / LAMB_THREADS;
+  const int64_t run = (ch.cnt + CHUNK_THREADS - 1) / CHUNK_THREADS;
   const int64_t j0 = min(ch.cnt, run * threadIdx.x), j1 = min(ch.cnt, j0 + run);
   double sw = 0.0, su = 0.0;
   for (int64_t j = j0; j < j1; ++j) {
@@ -734,19 +739,19 @@ lamb_apply_kernel(float* __restrict__ p, const float* __restrict__ m, const floa
     sw += q.x;
     su += q.y;
   }
-  const double2 s = lamb_block_sum2(sw, su);
+  const double2 s = flat_block_sum2(sw, su);
   const double r = (s.x > 0.0 && s.y > 0.0) ? sqrt(s.x) / sqrt(s.y) : 1.0;
   if (trust_out && ch.k == 0 && threadIdx.x == 0) trust_out[ch.l] = static_cast<float>(r);
   const float step = static_cast<float>(static_cast<double>(lr) * r);
 
   int64_t off;
-  const int n = lamb_chunk_span(begin, len, ch, &off);
+  const int n = flat_chunk_span(begin, len, ch, &off);
   float* pc = p + off; const float* mc = m + off; const float* vc = v + off;
   __nv_bfloat16* bc = pb ? pb + off : nullptr;
   const bool vec = ((reinterpret_cast<uintptr_t>(pc) | reinterpret_cast<uintptr_t>(mc) |
                      reinterpret_cast<uintptr_t>(vc)) & 15) == 0 && (reinterpret_cast<uintptr_t>(bc) & 7) == 0;
   const int n4 = vec ? n / 4 : 0;
-  for (int i = threadIdx.x; i < n4; i += LAMB_THREADS) {
+  for (int i = threadIdx.x; i < n4; i += CHUNK_THREADS) {
     float4 pv = reinterpret_cast<const float4*>(pc)[i];
     const float4 mv = reinterpret_cast<const float4*>(mc)[i];
     const float4 vv = reinterpret_cast<const float4*>(vc)[i];
@@ -763,11 +768,114 @@ lamb_apply_kernel(float* __restrict__ p, const float* __restrict__ m, const floa
       reinterpret_cast<uint2*>(bc)[i] = w;
     }
   }
-  for (int i = 4 * n4 + threadIdx.x; i < n; i += LAMB_THREADS) {
+  for (int i = 4 * n4 + threadIdx.x; i < n; i += CHUNK_THREADS) {
     const float pv = __fsub_rn(pc[i], __fmul_rn(step, lamb_u(mc[i], vc[i], pc[i], inv_bc1, inv_bc2_sqrt, eps, wd)));
     pc[i] = pv;
     if (bc) bc[i] = __float2bfloat16_rn(pv);
   }
+}
+
+// ---- Global-norm gradient clipping over the flat gradient buffer (torch.nn.utils.clip_grad_norm_, norm_type 2)
+//   clip_norm_kernel : one CTA per chunk; partials[chunk] = sum (grad_scale * g)^2 over the chunk
+//   clip_coef_kernel : one CTA; each tensor's partials summed in chunk order (fp64), then the tensors in table order
+//                      (fp64); norm = sqrt(total), coef = min(max_norm / (norm + 1e-6), 1) in fp32
+//   clip_scale_kernel: one CTA per chunk; g <- g * coef, and nothing at all when coef is exactly 1
+__global__ void __launch_bounds__(CHUNK_THREADS)
+clip_norm_kernel(const float* __restrict__ g, const int64_t* __restrict__ begin, const int64_t* __restrict__ len,
+                 int n_tensors, double* __restrict__ partials, float grad_scale) {
+  pdl_wait();
+  pdl_trigger();
+  const FlatChunk ch = flat_locate(len, n_tensors, blockIdx.x);
+  if (ch.l < 0) return;
+  int64_t off;
+  const int n = flat_chunk_span(begin, len, ch, &off);
+  const float* gc = g + off;
+  const int n4 = (reinterpret_cast<uintptr_t>(gc) & 15) == 0 ? n / 4 : 0;
+  float s = 0.f;
+  for (int i = threadIdx.x; i < n4; i += CHUNK_THREADS) {
+    const float4 gr = reinterpret_cast<const float4*>(gc)[i];
+    const float* gg = &gr.x;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const float x = __fmul_rn(gg[k], grad_scale);
+      s = __fmaf_rn(x, x, s);
+    }
+  }
+  for (int i = 4 * n4 + threadIdx.x; i < n; i += CHUNK_THREADS) {
+    const float x = __fmul_rn(gc[i], grad_scale);
+    s = __fmaf_rn(x, x, s);
+  }
+  const double2 t = flat_block_sum2(s, 0.0);
+  if (threadIdx.x == 0) partials[blockIdx.x] = t.x;
+}
+
+// Warp w takes tensor t0 + w of each group of CHUNK_THREADS / 32 tensors: lane k sums a contiguous run of the
+// tensor's partials in chunk order, then a shuffle butterfly; thread 0 adds the group's tensors in table order.
+__global__ void __launch_bounds__(CHUNK_THREADS)
+clip_coef_kernel(const int64_t* __restrict__ len, int n_tensors, const double* __restrict__ partials, float max_norm,
+                 float* __restrict__ norm_out, float* __restrict__ tensor_norms_out, float* __restrict__ coef_out) {
+  constexpr int WARPS = CHUNK_THREADS / 32;
+  __shared__ double s_tensor[WARPS];
+  pdl_wait();
+  pdl_trigger();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  double total = 0.0;
+  int64_t group_base = 0;  // first chunk of tensor t0
+  for (int t0 = 0; t0 < n_tensors; t0 += WARPS) {
+    const int l = t0 + warp, t1 = min(t0 + WARPS, n_tensors);
+    int64_t base = group_base, cnt = 0, group = 0;
+    for (int j = t0; j < t1; ++j) {
+      const int64_t c = flat_chunks(len[j]);
+      if (j < l) base += c;
+      if (j == l) cnt = c;
+      group += c;
+    }
+    double s = 0.0;
+    if (l < n_tensors) {
+      const int64_t run = (cnt + 31) / 32;
+      const int64_t j0 = min(cnt, run * lane), j1 = min(cnt, j0 + run);
+      for (int64_t j = j0; j < j1; ++j) s += partials[base + j];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+      if (lane == 0 && tensor_norms_out) tensor_norms_out[l] = static_cast<float>(sqrt(s));
+    }
+    if (lane == 0) s_tensor[warp] = s;
+    __syncthreads();
+    if (threadIdx.x == 0)
+      for (int w = 0; w < t1 - t0; ++w) total += s_tensor[w];
+    __syncthreads();
+    group_base += group;
+  }
+  if (threadIdx.x == 0) {
+    const float norm = static_cast<float>(sqrt(total));
+    const float coef = __fdiv_rn(max_norm, __fadd_rn(norm, 1e-6f));
+    *norm_out = norm;
+    *coef_out = coef > 1.f ? 1.f : coef;  // torch.clamp(max=1) keeps a NaN, where fminf(NaN, 1) would give 1
+  }
+}
+
+__global__ void __launch_bounds__(CHUNK_THREADS)
+clip_scale_kernel(float* __restrict__ g, const int64_t* __restrict__ begin, const int64_t* __restrict__ len,
+                  int n_tensors, const float* __restrict__ coef) {
+  pdl_wait();
+  pdl_trigger();
+  const float c = *coef;
+  if (c == 1.f) return;  // not clipped: the buffer stays as it is, bitwise what g * 1 gives
+  const FlatChunk ch = flat_locate(len, n_tensors, blockIdx.x);
+  if (ch.l < 0) return;
+  int64_t off;
+  const int n = flat_chunk_span(begin, len, ch, &off);
+  float* gc = g + off;
+  const int n4 = (reinterpret_cast<uintptr_t>(gc) & 15) == 0 ? n / 4 : 0;
+  for (int i = threadIdx.x; i < n4; i += CHUNK_THREADS) {
+    float4 gr = reinterpret_cast<const float4*>(gc)[i];
+    gr.x = __fmul_rn(gr.x, c);
+    gr.y = __fmul_rn(gr.y, c);
+    gr.z = __fmul_rn(gr.z, c);
+    gr.w = __fmul_rn(gr.w, c);
+    reinterpret_cast<float4*>(gc)[i] = gr;
+  }
+  for (int i = 4 * n4 + threadIdx.x; i < n; i += CHUNK_THREADS) gc[i] = __fmul_rn(gc[i], c);
 }
 
 }  // namespace loss
@@ -928,14 +1036,42 @@ extern "C" int lirec_lamb_flat(float* param, const float* grad, float* exp_avg, 
   double2* part = reinterpret_cast<double2*>(partials);
   // one CTA per chunk; the bound leaves at most n_tensors CTAs without a chunk, and they return at once
   const dim3 grid(static_cast<unsigned>(chunks));
-  LIREC_CUDA_OK(launch_pdl(loss::lamb_moments_kernel, grid, dim3(loss::LAMB_THREADS), 0, s, param, grad, exp_avg,
+  LIREC_CUDA_OK(launch_pdl(loss::lamb_moments_kernel, grid, dim3(loss::CHUNK_THREADS), 0, s, param, grad, exp_avg,
                            exp_avg_sq, tensor_begin, tensor_len, n_tensors, part, static_cast<float>(b1),
                            static_cast<float>(b2), one_minus_beta1, one_minus_beta2, eps, weight_decay, inv_bc1,
                            inv_bc2_sqrt, grad_scale));
-  LIREC_CUDA_OK(launch_pdl(loss::lamb_apply_kernel, grid, dim3(loss::LAMB_THREADS), 0, s, param, exp_avg, exp_avg_sq,
+  LIREC_CUDA_OK(launch_pdl(loss::lamb_apply_kernel, grid, dim3(loss::CHUNK_THREADS), 0, s, param, exp_avg, exp_avg_sq,
                            reinterpret_cast<__nv_bfloat16*>(param_bf16), tensor_begin, tensor_len, n_tensors,
                            static_cast<const double2*>(part), trust_out, lr, eps, weight_decay, inv_bc1,
                            inv_bc2_sqrt));
   note_launch(2);
+  return LIREC_OK;
+}
+
+extern "C" int lirec_grad_clip_flat(float* grad, const int64_t* tensor_begin, const int64_t* tensor_len,
+                                    int32_t n_tensors, int64_t n, double* partials, int64_t n_partials,
+                                    float max_norm, float grad_scale, float* norm_out, float* tensor_norms_out,
+                                    void* stream) {
+  LIREC_ENTER();
+  LIREC_REQUIRE(grad && tensor_begin && tensor_len && partials && norm_out, "grad clip: null pointer");
+  LIREC_REQUIRE(n_tensors >= 1 && n >= 1, "grad clip: n_tensors=%d n=%lld", n_tensors, static_cast<long long>(n));
+  const int64_t chunks = LIREC_LAMB_PARTIALS(n, n_tensors);
+  LIREC_REQUIRE(n_partials >= chunks, "grad clip: partials hold %lld chunks, %lld needed",
+                static_cast<long long>(n_partials), static_cast<long long>(chunks));
+  LIREC_REQUIRE(chunks <= 0x7fffffff, "grad clip: %lld chunks", static_cast<long long>(chunks));
+  LIREC_REQUIRE(std::isfinite(max_norm) && max_norm > 0.f, "grad clip: max_norm=%g (finite and > 0)", max_norm);
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  // the chunk sums take the first `chunks` doubles of the partials; the clip coefficient travels from the norm pass
+  // to the scale pass in the double after them (the entries hold two doubles each, so it exists)
+  float* coef = reinterpret_cast<float*>(partials + chunks);
+  const dim3 grid(static_cast<unsigned>(chunks));
+  LIREC_CUDA_OK(launch_pdl(loss::clip_norm_kernel, grid, dim3(loss::CHUNK_THREADS), 0, s,
+                           static_cast<const float*>(grad), tensor_begin, tensor_len, n_tensors, partials,
+                           grad_scale));
+  LIREC_CUDA_OK(launch_pdl(loss::clip_coef_kernel, dim3(1), dim3(loss::CHUNK_THREADS), 0, s, tensor_len, n_tensors,
+                           static_cast<const double*>(partials), max_norm, norm_out, tensor_norms_out, coef));
+  LIREC_CUDA_OK(launch_pdl(loss::clip_scale_kernel, grid, dim3(loss::CHUNK_THREADS), 0, s, grad, tensor_begin,
+                           tensor_len, n_tensors, static_cast<const float*>(coef)));
+  note_launch(3);
   return LIREC_OK;
 }

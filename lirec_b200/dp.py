@@ -305,22 +305,43 @@ class SwitchReduceAdam:
         m.mark_bf16_fresh()          # FlatAdam materialises the per-parameter step counters lazily
 
 
-def reduce_and_step(model, optimizer, fused=None, local_clips=None, global_clips=None):
+def _clip(model, max_norm, grad_scale=1.0):
+    from lirec_b200.mlp import model as M
+    return M.clip_grad_norm_flat_(model, max_norm, grad_scale=grad_scale)
+
+
+def reduce_and_step(model, optimizer, fused=None, local_clips=None, global_clips=None, max_norm=0.0):
     """Gradient exchange + optimizer step of one data-parallel iteration: the in-switch fused kernel when
-    `fused` (SwitchReduceAdam.attach) is available, else NCCL all_reduce + the optimizer's own step."""
+    `fused` (SwitchReduceAdam.attach) is available, else NCCL all_reduce + the optimizer's own step.
+    max_norm > 0 clips the reduced gradient to that global L2 norm between the exchange and the step
+    (mlp.model.clip_grad_norm_flat_; the norm of the averaged gradient, identical on every rank) and returns the
+    pre-clip norm as a 0-d device tensor; otherwise returns None.  The fused step updates parameters before the
+    global norm exists, so it cannot clip."""
     if fused is not None:
+        if max_norm:
+            raise ValueError("reduce_and_step: gradient clipping needs the unfused step (do not attach "
+                             "SwitchReduceAdam with --clip_grad_norm)")
         fused.step(local_clips, global_clips)
-        return
+        return None
+    norm = None
     if world_size() > 1:
         from lirec_b200.mlp.model import _FlatOptimizer
         if isinstance(optimizer, _FlatOptimizer):        # FlatAdam, FlatLamb: the average rides in grad_scale
-            optimizer.step(grad_scale=allreduce_flat_grad(model._flat_grad, local_clips, global_clips))
+            scale = allreduce_flat_grad(model._flat_grad, local_clips, global_clips)
+            if max_norm:
+                norm = _clip(model, max_norm, scale)
+            optimizer.step(grad_scale=scale)
         else:
             allreduce_flat_grad(model._flat_grad, local_clips, global_clips, average_in_place=True)
+            if max_norm:
+                norm = _clip(model, max_norm)
             optimizer.step()
     else:
+        if max_norm:
+            norm = _clip(model, max_norm)
         step = getattr(optimizer, "_step_impl", None)       # FlatAdam / FlatLamb: skip the Optimizer.step hook wrapper
         if step is not None:
             step()
         else:
             optimizer.step()
+    return norm

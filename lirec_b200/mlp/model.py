@@ -10,6 +10,7 @@ storage is re-pointed into one flat fp32 buffer (plus a flat gradient buffer and
 that the kernels read and write in place.  There is no PyTorch or CPU fallback.
 """
 import ctypes as C
+import math
 
 import numpy as np
 import torch
@@ -22,7 +23,7 @@ from lirec_b200.utils.arg_pars import opt
 __all__ = ["Modalities", "MidFusionMultiClip", "MidFusionMultiClipMaxTracks", "GatingUnit",
            "MultiTaskCrossEntropyLoss", "MultiTaskMaxMargin", "MaxMarginCrossEntropyLoss", "MarginLoss",
            "MarginTrackRelsLoss", "MultiLabelBCELoss", "TrackBCELoss", "create_model", "ModelOutput", "FlatAdam",
-           "FlatLamb"]
+           "FlatLamb", "clip_grad_norm_flat_"]
 
 _SLOTS = ("txt", "vis", "tracks1", "tracks2")
 _SECOND = ("txt2", "vis2", "tracks12", "tracks22")
@@ -146,6 +147,8 @@ class _HotPath(nn.Module):
         self._gate_dim = out_dim_ints
         self._flat = self._flat_grad = self._flat_bf16 = None
         self._param_list = None
+        self._table = self._clip_partials = None
+        self._last_grad_norm = None              # pre-clip gradient norm of the last clip_grad_norm_flat_ (device)
         self._versions = None
         self._dirty = True
         self._step = 0
@@ -190,9 +193,20 @@ class _HotPath(nn.Module):
         self._flat, self._offsets, self._param_list = flat, offsets, params
         self._flat_grad = torch.zeros_like(flat)
         self._flat_bf16 = torch.zeros(total, dtype=torch.bfloat16, device=dev)
+        self._table = self._clip_partials = None
         self._versions = None
         self._dirty = False
         self._build_structs()
+
+    def _tensor_table(self):
+        """(begin, len): int64 device tensors [n_parameters], the float offset and length of every parameter in the
+        flat buffers, in model.parameters() order (the tensor table of lirec_lamb_flat / lirec_grad_clip_flat).
+        Built once per flat layout (_sync_flat must have run)."""
+        if self._table is None:
+            dev = self._flat.device
+            self._table = (torch.tensor(self._offsets, dtype=torch.int64, device=dev),
+                           torch.tensor([p.numel() for p in self._param_list], dtype=torch.int64, device=dev))
+        return self._table
 
     def _apply(self, fn, *args, **kwargs):
         self._dirty = True                    # parameters may have been re-allocated (model.to(...))
@@ -870,8 +884,7 @@ class FlatLamb(_FlatOptimizer):
     def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-6, weight_decay=0.0):
         super().__init__(model, dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay))
         dev = model._flat.device
-        self._begin = torch.tensor(model._offsets, dtype=torch.int64, device=dev)
-        self._len = torch.tensor([p.numel() for p in model._param_list], dtype=torch.int64, device=dev)
+        self._begin, self._len = model._tensor_table()
         self._partials = ops.lamb_partials(model._flat.numel(), len(model._param_list), device=dev)
         self._trust = torch.ones(len(model._param_list), dtype=torch.float32, device=dev)
 
@@ -885,6 +898,37 @@ class FlatLamb(_FlatOptimizer):
         """Device float32 tensor [n_parameters]: the trust ratio each parameter got in the last step (1 before the
         first), in model.parameters() order."""
         return self._trust
+
+
+@torch.no_grad()
+def clip_grad_norm_flat_(model, max_norm, grad_scale=1.0, tensor_norms=None):
+    """torch.nn.utils.clip_grad_norm_(model.parameters(), max_norm) with norm_type 2, over the model's flat gradient
+    buffer in three fused launches (lirec_grad_clip_flat) and without a host sync: norm = ||grad_scale * g|| over
+    every parameter, then g *= min(max_norm / (norm + 1e-6), 1) in place; nothing is written when the factor is 1.
+    grad_scale is the factor the optimizer still applies to the gradients (the data-parallel 1/world average that
+    FlatAdam and FlatLamb take in their step): the norm is the norm of the scaled gradient, the buffer is multiplied
+    by the clip factor alone.  As in torch, a NaN norm turns the gradients into NaN, and an Inf norm gives a factor of
+    0.  Returns the pre-clip total norm as a 0-d float32 device tensor; tensor_norms (optional float32 device tensor
+    [n_parameters]) receives every parameter's pre-clip norm, in model.parameters() order."""
+    max_norm = float(max_norm)
+    if not (math.isfinite(max_norm) and max_norm > 0.0):
+        raise ValueError("clip_grad_norm_flat_: max_norm must be finite and > 0 (got %r)" % (max_norm,))
+    if model._flat_grad is None:
+        raise RuntimeError("clip_grad_norm_flat_: the model has no flat gradient buffer yet (no backward ran)")
+    for p, g in zip(model._param_list, model._grad_views):
+        pg = p.grad
+        if pg is not None and pg is not g and pg.data_ptr() != g.data_ptr():
+            # _publish_grads adds into a p.grad that is not a view of the flat buffer; clipping the buffer would
+            # leave that gradient, which the torch optimizer reads, unclipped
+            raise RuntimeError("clip_grad_norm_flat_: a parameter's .grad lives outside the flat gradient buffer; "
+                               "set it to None (optimizer.zero_grad()) before backward")
+    begin, length = model._tensor_table()
+    if model._clip_partials is None:
+        model._clip_partials = ops.lamb_partials(model._flat_grad.numel(), begin.numel(), device=model._flat.device)
+    norm = ops.grad_clip_flat(model._flat_grad, begin, length, model._clip_partials, max_norm, grad_scale,
+                              tensor_norms_out=tensor_norms)
+    model._last_grad_norm = norm
+    return norm
 
 
 def _check_loss_choice():
@@ -910,12 +954,21 @@ def _check_optimizer_choice():
     return kind
 
 
+def _check_clip_choice():
+    """--clip_grad_norm (host only, before any device work): 0 is off, anything else a finite maximum norm."""
+    v = float(getattr(opt, "clip_grad_norm", 0.0) or 0.0)
+    if not (math.isfinite(v) and v >= 0.0):
+        raise ValueError("--clip_grad_norm must be 0 (off) or a finite maximum norm > 0 (got %r)" % (v,))
+    return v
+
+
 def create_model(n_classes, n_rels=0):
     """Reference: mlp/model.py:578-609 — same selection logic and return triple.  --loss bce / ce swap in the
     multi-label BCE or the softmax cross-entropy for the reference's max-margin losses; --optimizer lamb swaps in
-    FlatLamb for Adam."""
+    FlatLamb for Adam.  --clip_grad_norm is checked here; the training loop applies it."""
     loss_kind = _check_loss_choice()
     optimizer_kind = _check_optimizer_choice()
+    _check_clip_choice()
     if opt.device != "cuda":
         raise RuntimeError("lirec_b200 runs on a B200 only (opt.device='%s'); no CPU fallback" % opt.device)
     if opt.tr_maximize:

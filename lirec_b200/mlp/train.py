@@ -4,7 +4,8 @@ zero_grad, backward, Adam step, periodic evaluation and checkpoints in the refer
 Differences on purpose: batches are PackedBatches prefetched to the GPU asynchronously; the loss
 value is read back every 10 iterations instead of every step (mlp/train.py:59 syncs each step);
 with `opt.dp` the clips of every global batch are split over the ranks and the flat gradient buffer
-is all-reduced over NCCL before the optimizer step (lirec_b200/dp.py).  Batches of a single clip
+is all-reduced over NCCL before the optimizer step (lirec_b200/dp.py); with --clip_grad_norm the
+reduced gradient is clipped to that global L2 norm before the step.  Batches of a single clip
 are skipped like the reference does (:55-56)."""
 import copy
 import time
@@ -23,9 +24,12 @@ from lirec_b200.utils.model_saver import ModelSaver
 from lirec_b200.utils.util_functions import Averaging, dir_check
 
 
-def train_step(model, loss, optimizer, pb, world=1, fused=None):
+def train_step(model, loss, optimizer, pb, world=1, fused=None, max_norm=0.0):
     """One optimisation step on a device PackedBatch; returns the (device) loss tensor.  `fused`: the
     in-switch reduce+Adam of dp.SwitchReduceAdam.attach (None: NCCL all_reduce, then the optimizer).
+    max_norm > 0 (--clip_grad_norm): the reduced gradient is clipped to that global L2 norm before the
+    optimizer step (dp.reduce_and_step; needs fused=None); the pre-clip norm stays on the device as
+    model._last_grad_norm.
     With lirec_b200's own model and loss the forward, loss and backward run as three native calls
     without the autograd engine (`mlp.model.train_step`, `--native_step 1`, the default); any other
     combination takes the reference's four-call sequence (mlp/train.py:57-63)."""
@@ -37,7 +41,7 @@ def train_step(model, loss, optimizer, pb, world=1, fused=None):
         loss._dp_world = world
         dp_empty_shard_collectives(loss, model._flat.device)
         loss._dp_world = 1
-        dp.reduce_and_step(model, optimizer, fused, 0, pb.global_clips)
+        dp.reduce_and_step(model, optimizer, fused, 0, pb.global_clips, max_norm)
         return model._flat_grad.new_zeros(())
     loss._dp_world = world                       # multi-task losses normalise their relationship term globally
     if fused is not None:                        # bucket 0 of the exchange / Adam overlaps the rest of backward
@@ -55,7 +59,7 @@ def train_step(model, loss, optimizer, pb, world=1, fused=None):
         local = pb.B
         global_clips = getattr(pb.host, "global_clips", None) if getattr(pb, "host", None) is not None else None
     loss._dp_world = 1                           # evaluation (mlp/test.py) runs the losses without collectives
-    dp.reduce_and_step(model, optimizer, fused, local, global_clips)
+    dp.reduce_and_step(model, optimizer, fused, local, global_clips, max_norm)
     return loss_values
 
 
@@ -64,6 +68,9 @@ def training(train_dataset, **kwargs):
     print("set parameters and model, train start time: %s" % train_start_time)
     model, loss, optimizer = kwargs["model"], kwargs["loss"], kwargs["optimizer"]
     rank, world, fused = 0, 1, None
+    # --clip_grad_norm: the fused exchange + Adam and the overlapped gate + head Adam pass both update parameters
+    # before the global norm exists, so clipping takes NCCL all_reduce (with --dp) and the optimizer's own step
+    max_norm = float(getattr(opt, "clip_grad_norm", 0.0) or 0.0)
     if getattr(opt, "dp", 0):
         rank, world, _ = dp.init_from_env()
         model._sync_flat()
@@ -71,11 +78,12 @@ def training(train_dataset, **kwargs):
         model.set_rank(rank)                               # dropout / sampled-assignment streams differ per rank
         if hasattr(loss, "set_rank"):
             loss.set_rank(rank)
-        if int(getattr(opt, "dp_switch_reduce", 1)):
+        if int(getattr(opt, "dp_switch_reduce", 1)) and not max_norm:
             fused = dp.SwitchReduceAdam.attach(model, optimizer)     # None without NVSwitch multicast / FlatAdam
-    if fused is None and world == 1 and int(getattr(opt, "overlap_adam", 0)):
+    if fused is None and world == 1 and int(getattr(opt, "overlap_adam", 0)) and not max_norm:
         fused = dp.SwitchReduceAdam.attach(model, optimizer, single_gpu=True)    # None unless FlatAdam
     batch_time, data_time, losses = Averaging(), Averaging(), Averaging()
+    grad_norm = float("nan")
     print("epochs: %s", opt.epochs)
     model_saver_val = ModelSaver(path=opt.store_root)
     dev = torch.device("cuda", torch.cuda.current_device())
@@ -102,16 +110,22 @@ def training(train_dataset, **kwargs):
             data_time.update(time.time() - end)
             if getattr(pb.host, "global_clips", pb.B) == 1:
                 continue
-            loss_values = train_step(model, loss, optimizer, pb, world, fused)
+            loss_values = train_step(model, loss, optimizer, pb, world, fused, max_norm)
             counter += pb.B
             if i % 10 == 0 and pb.B:
-                losses.update(loss_values.item(), pb.B)      # device->host sync only here
+                if max_norm:                                 # the loss and the last pre-clip norm in one read-back
+                    lv, grad_norm = torch.stack([loss_values.detach().float().reshape(()),
+                                                 model._last_grad_norm]).tolist()
+                else:
+                    lv = loss_values.item()
+                losses.update(lv, pb.B)                      # device->host sync only here
             batch_time.update(time.time() - end)
             end = time.time()
             if i % 10 == 0 and i and rank == 0:
                 print("Epoch: [{0}][{1}/{2}]\tTime {bt.val:.3f} ({bt.avg:.3f})\tData {dt.val:.3f} ({dt.avg:.3f})\t"
                       "Loss {loss.val:.4f} ({loss.avg:.4f})\t".format(epoch, i, n_batches, bt=batch_time,
-                                                                       dt=data_time, loss=losses))
+                                                                       dt=data_time, loss=losses)
+                      + ("Grad norm {:.4f}\t".format(grad_norm) if max_norm else ""))
         print(counter)
         print("loss: %f" % losses.avg)
         losses.reset()

@@ -12,7 +12,7 @@ from ._ext import (ACT_NONE, ACT_RELU, ACT_TANH, OUT_F32, OUT_SPLIT, OUT_SPLIT_T
                    POST_NONE, POST_SIGN_MASK)
 
 __all__ = ["gemm_problem", "gemm_grouped", "seg_reduce", "seg_softmax_pool", "seg_softmax_pool_bwd", "SegSoftmaxPool", "rows_expand_fwd", "rows_expand_bwd", "split_f32",
-           "cast_bf16", "gather_rows", "roi_max_pool", "loss_track", "loss_rowmargin", "loss_ce", "loss_bce", "loss_bce_track", "predict_tracks", "adam_flat", "lamb_partials", "lamb_flat", "dp_exchange", "dp_reduce_adam_bcast", "dp_reduce_adam_bcast_peer", "dropout_desc"]
+           "cast_bf16", "gather_rows", "roi_max_pool", "loss_track", "loss_rowmargin", "loss_ce", "loss_bce", "loss_bce_track", "predict_tracks", "adam_flat", "lamb_partials", "lamb_flat", "grad_clip_flat", "dp_exchange", "dp_reduce_adam_bcast", "dp_reduce_adam_bcast_peer", "dropout_desc"]
 
 
 def dropout_desc(p=0.0, seed=0, stream_id=0, col_off=0):
@@ -321,6 +321,36 @@ def lamb_flat(param, grad, exp_avg, exp_avg_sq, param_bf16, tensor_begin, tensor
         _ext.ptr(tensor_begin), _ext.ptr(tensor_len), int(n_tensors), int(param.numel()), _ext.ptr(partials),
         int(partials.numel() // 2), float(lr), 1.0 - float(beta1), 1.0 - float(beta2), float(eps), float(weight_decay),
         int(step), float(grad_scale), _ext.ptr(trust_out), sp))
+
+
+def grad_clip_flat(grad, tensor_begin, tensor_len, partials, max_norm, grad_scale=1.0, norm_out=None,
+                   tensor_norms_out=None, stream=None):
+    """Global-norm clipping of the flat gradient buffer in place (lirec_grad_clip_flat): norm = ||grad_scale * grad||
+    over the tensor table, grad *= min(max_norm / (norm + 1e-6), 1).  tensor_begin / tensor_len: int64 device tensors
+    [n_tensors] in floats; partials: lamb_partials(grad.numel(), n_tensors); norm_out: optional float32 device tensor
+    of one element (allocated when None); tensor_norms_out: optional float32 device tensor [n_tensors].  Returns
+    norm_out, which the kernels fill on the stream without a host sync."""
+    n_tensors = tensor_begin.numel()
+    if grad.dtype != torch.float32 or not grad.is_contiguous():
+        raise ValueError("grad_clip_flat: grad must be a contiguous float32 tensor")
+    for t in (tensor_begin, tensor_len):
+        if t.dtype != torch.int64 or t.numel() != n_tensors or not t.is_contiguous():
+            raise ValueError("grad_clip_flat: tensor_begin / tensor_len must be contiguous int64 tensors of one length")
+    if partials.dtype != torch.float64 or not partials.is_contiguous():
+        raise ValueError("grad_clip_flat: partials must be a contiguous float64 tensor (ops.lamb_partials)")
+    if norm_out is None:
+        norm_out = torch.empty((), dtype=torch.float32, device=grad.device)
+    elif norm_out.dtype != torch.float32 or norm_out.numel() != 1:
+        raise ValueError("grad_clip_flat: norm_out must be a float32 tensor of one element")
+    if tensor_norms_out is not None and (tensor_norms_out.dtype != torch.float32 or
+                                         tensor_norms_out.numel() < n_tensors):
+        raise ValueError("grad_clip_flat: tensor_norms_out must be float32 with one entry per tensor")
+    sp = _ext.stream_ptr() if stream is None else C.c_void_p(stream.cuda_stream)
+    _ext.check(_ext.lib().lirec_grad_clip_flat(
+        _ext.ptr(grad), _ext.ptr(tensor_begin), _ext.ptr(tensor_len), int(n_tensors), int(grad.numel()),
+        _ext.ptr(partials), int(partials.numel() // 2), float(max_norm), float(grad_scale), _ext.ptr(norm_out),
+        _ext.ptr(tensor_norms_out), sp))
+    return norm_out
 
 
 def dp_reduce_adam_bcast(grad_mc, param, param_mc, bf16_mc, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, weight_decay,

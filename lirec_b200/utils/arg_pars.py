@@ -131,6 +131,11 @@ _FLAGS = [
                          help="adam: the reference's Adam (torch.optim.Adam, or the fused kernel with --fused_adam); "
                               "lamb: fused LAMB (layer-wise trust ratio, decoupled --weight_decay) for large global "
                               "batches, whatever --fused_adam says")),
+    ("--clip_grad_norm", dict(default=0.0, type=float,
+                              help="> 0: clip the gradient to this global L2 norm before every optimizer step, like "
+                                   "torch.nn.utils.clip_grad_norm_ (fused, no host sync; with --dp, the norm of the "
+                                   "averaged gradient); turns off the fused exchange + Adam and --overlap_adam. "
+                                   "0: off")),
     ("--world_movies", dict(default=6, type=int)),
     ("--world_scenes", dict(default=40, type=int)),
 ]
