@@ -520,6 +520,23 @@ int lirec_grad_clip_flat(float* grad, const int64_t* tensor_begin, const int64_t
                          int64_t n, double* partials, int64_t n_partials, float max_norm, float grad_scale,
                          float* norm_out, float* tensor_norms_out, void* stream);
 
+/* Exponential moving average of the flat weights, for evaluation and checkpoints (the update of
+ * torch.optim.swa_utils.AveragedModel with get_ema_multi_avg_fn(decay), i.e. torch._foreach_lerp_):
+ *   ema[i] = lerp(ema[i], param[i], a),  a = one_minus_decay = 1 - decay, elementwise in fp32, i in [0, n):
+ *     a < 0.5:  ema + a * (param - ema)          otherwise:  param - (param - ema) * (1 - a)
+ * each rounded as one FMA, as torch.lerp's kernel computes it.  NaN and Inf propagate like torch.lerp.  param is read
+ * and never written.  Pass the complement, formed in double: fp32 holds 1 - decay to full precision where
+ * 1 - fp32(0.9999) loses digits.  One launch, no host sync.  one_minus_decay must be finite and in (0, 1).  */
+int lirec_ema_update_flat(float* ema, const float* param, int64_t n, float one_minus_decay, void* stream);
+
+/* Exchange param[i] and ema[i] for i in [0, n) (evaluate the average, then swap back), and when param_bf16 is not
+ * NULL write param_bf16[i] = rn_bf16(new param[i]) with lirec_cast_bf16's rounding, so the shadow equals
+ * lirec_cast_bf16(param) bit for bit afterwards.  Two swaps restore all three buffers when the shadow was
+ * lirec_cast_bf16(param) to begin with.  One launch.                                                          */
+int lirec_ema_swap_flat(float* param, float* ema, void* param_bf16, int64_t n, void* stream);
+/* Both EMA entry points refuse a NULL param / ema, n < 0 and a buffer that is not 16-byte aligned; n == 0 enqueues
+ * nothing.                                                                                                     */
+
 /* ---- data parallel: in-switch gradient exchange, bucket by bucket --------
  * Replaces ncclAllReduce(flat gradient) of a data-parallel step (the reference is single-process, SURVEY.md
  * §2.3; the optimizer stays torch.optim.Adam's arithmetic, mlp/model.py:599-601, through lirec_adam_flat on the

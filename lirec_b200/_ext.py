@@ -159,6 +159,8 @@ def lib():
         C.c_int32, C.c_float, C.c_void_p, C.c_void_p]
     L.lirec_grad_clip_flat.argtypes = [C.c_void_p] * 3 + [C.c_int32, C.c_int64, C.c_void_p, C.c_int64, C.c_float,
                                                           C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.lirec_ema_update_flat.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_float, C.c_void_p]
+    L.lirec_ema_swap_flat.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
     L.lirec_profile_sample.argtypes = [C.c_int32]
     L.lirec_dp_flag_words.argtypes = [C.c_int32]
     L.lirec_dp_flag_words.restype = C.c_int
@@ -195,7 +197,7 @@ EXPORTED_SYMBOLS = [
     "lirec_gemm_grouped", "lirec_profile_begin", "lirec_profile_end", "lirec_seg_reduce_f32", "lirec_seg_softmax_pool_fwd", "lirec_seg_softmax_pool_bwd", "lirec_rows_expand_fwd", "lirec_rows_expand_bwd",
     "lirec_split_f32", "lirec_cast_bf16", "lirec_gather_rows", "lirec_roi_max_pool_f32", "lirec_loss_track_fwd_bwd", "lirec_loss_rowmargin_fwd_bwd", "lirec_loss_ce_fwd_bwd",
     "lirec_loss_bce_fwd_bwd", "lirec_loss_bce_track_fwd_bwd", "lirec_predict_tracks",
-    "lirec_model_workspace_bytes", "lirec_model_workspace_layout", "lirec_model_forward", "lirec_model_backward", "lirec_adam_flat", "lirec_lamb_flat", "lirec_grad_clip_flat", "lirec_profile_sample", "lirec_dp_flag_words", "lirec_dp_exchange", "lirec_dp_reduce_adam_bcast", "lirec_dp_reduce_adam_bcast_peer",
+    "lirec_model_workspace_bytes", "lirec_model_workspace_layout", "lirec_model_forward", "lirec_model_backward", "lirec_adam_flat", "lirec_lamb_flat", "lirec_grad_clip_flat", "lirec_ema_update_flat", "lirec_ema_swap_flat", "lirec_profile_sample", "lirec_dp_flag_words", "lirec_dp_exchange", "lirec_dp_reduce_adam_bcast", "lirec_dp_reduce_adam_bcast_peer",
     "lirec_collate_arena_bound", "lirec_collate_tables", "lirec_collate_gather",
 ]
 

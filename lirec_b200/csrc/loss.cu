@@ -878,6 +878,66 @@ clip_scale_kernel(float* __restrict__ g, const int64_t* __restrict__ begin, cons
   for (int i = 4 * n4 + threadIdx.x; i < n; i += CHUNK_THREADS) gc[i] = __fmul_rn(gc[i], c);
 }
 
+// ---- Exponential moving average of the flat weights (FlatEMA, --ema_decay)
+//   ema_update_kernel: e <- lerp(e, w, a), a = 1 - decay, with torch.lerp's arithmetic as nvcc builds ATen's lerp
+//                      (contracted to one FMA): a < 0.5: e + a*(w - e), else w - (w - e)*(1 - a)
+//   ema_swap_kernel  : p <-> e, and the bf16 shadow of the new p with cast_bf16_kernel's / adam_kernel's rounding
+// Both are grid-stride loops with 128-bit accesses over the bulk (the entry points require 16-byte aligned buffers)
+// and a scalar tail; the rounding is spelled out with _rn intrinsics so that FMA contraction cannot change it.
+__device__ __forceinline__ float ema_lerp(float e, float w, float a, float one_minus_a, bool small) {
+  const float d = __fsub_rn(w, e);
+  return small ? __fmaf_rn(a, d, e) : __fmaf_rn(-d, one_minus_a, w);
+}
+
+__global__ void __launch_bounds__(256)
+ema_update_kernel(float* __restrict__ e, const float* __restrict__ w, int64_t n, float a) {
+  pdl_wait();
+  pdl_trigger();
+  const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
+  const int64_t tid = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+  const bool small = a < 0.5f;
+  const float b = __fsub_rn(1.f, a);
+  const int64_t n4 = n / 4;
+  for (int64_t i = tid; i < n4; i += stride) {
+    float4 ev = reinterpret_cast<const float4*>(e)[i];
+    const float4 wv = reinterpret_cast<const float4*>(w)[i];
+    ev.x = ema_lerp(ev.x, wv.x, a, b, small);
+    ev.y = ema_lerp(ev.y, wv.y, a, b, small);
+    ev.z = ema_lerp(ev.z, wv.z, a, b, small);
+    ev.w = ema_lerp(ev.w, wv.w, a, b, small);
+    reinterpret_cast<float4*>(e)[i] = ev;
+  }
+  for (int64_t i = 4 * n4 + tid; i < n; i += stride) e[i] = ema_lerp(e[i], w[i], a, b, small);
+}
+
+__global__ void __launch_bounds__(256)
+ema_swap_kernel(float* __restrict__ p, float* __restrict__ e, __nv_bfloat16* __restrict__ pb, int64_t n) {
+  pdl_wait();
+  pdl_trigger();
+  const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
+  const int64_t tid = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+  const int64_t n4 = n / 4;
+  for (int64_t i = tid; i < n4; i += stride) {
+    const float4 pv = reinterpret_cast<const float4*>(p)[i];
+    const float4 ev = reinterpret_cast<const float4*>(e)[i];
+    reinterpret_cast<float4*>(p)[i] = ev;
+    reinterpret_cast<float4*>(e)[i] = pv;
+    if (pb) {
+      const __nv_bfloat162 lo = __floats2bfloat162_rn(ev.x, ev.y), hi = __floats2bfloat162_rn(ev.z, ev.w);
+      uint2 q;
+      q.x = *reinterpret_cast<const uint32_t*>(&lo);
+      q.y = *reinterpret_cast<const uint32_t*>(&hi);
+      reinterpret_cast<uint2*>(pb)[i] = q;
+    }
+  }
+  for (int64_t i = 4 * n4 + tid; i < n; i += stride) {
+    const float pv = p[i], ev = e[i];
+    p[i] = ev;
+    e[i] = pv;
+    if (pb) pb[i] = __float2bfloat16_rn(ev);
+  }
+}
+
 }  // namespace loss
 }  // namespace lirec
 
@@ -1073,5 +1133,39 @@ extern "C" int lirec_grad_clip_flat(float* grad, const int64_t* tensor_begin, co
   LIREC_CUDA_OK(launch_pdl(loss::clip_scale_kernel, grid, dim3(loss::CHUNK_THREADS), 0, s, grad, tensor_begin,
                            tensor_len, n_tensors, static_cast<const float*>(coef)));
   note_launch(3);
+  return LIREC_OK;
+}
+
+// Grid of the two EMA passes: like lirec_adam_flat's, one float4 per thread up to 16 CTAs per SM, then grid-stride.
+static int ema_grid(int64_t n) {
+  return static_cast<int>(std::min<int64_t>((n / 4 + 255) / 256 + 1, 148 * 16));
+}
+
+static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+extern "C" int lirec_ema_update_flat(float* ema, const float* param, int64_t n, float one_minus_decay, void* stream) {
+  LIREC_ENTER();
+  LIREC_REQUIRE(ema && param, "ema update: null pointer");
+  LIREC_REQUIRE(n >= 0, "ema update: n=%lld", static_cast<long long>(n));
+  LIREC_REQUIRE(aligned16(ema) && aligned16(param), "ema update: buffers must be 16-byte aligned");
+  LIREC_REQUIRE(std::isfinite(one_minus_decay) && one_minus_decay > 0.f && one_minus_decay < 1.f,
+                "ema update: one_minus_decay=%g (finite, in (0, 1))", one_minus_decay);
+  if (n == 0) return LIREC_OK;
+  LIREC_CUDA_OK(launch_pdl(loss::ema_update_kernel, dim3(ema_grid(n)), dim3(256), 0, static_cast<cudaStream_t>(stream),
+                           ema, param, n, one_minus_decay));
+  note_launch();
+  return LIREC_OK;
+}
+
+extern "C" int lirec_ema_swap_flat(float* param, float* ema, void* param_bf16, int64_t n, void* stream) {
+  LIREC_ENTER();
+  LIREC_REQUIRE(param && ema, "ema swap: null pointer");
+  LIREC_REQUIRE(n >= 0, "ema swap: n=%lld", static_cast<long long>(n));
+  LIREC_REQUIRE(aligned16(param) && aligned16(ema) && aligned16(param_bf16),
+                "ema swap: buffers must be 16-byte aligned");
+  if (n == 0) return LIREC_OK;
+  LIREC_CUDA_OK(launch_pdl(loss::ema_swap_kernel, dim3(ema_grid(n)), dim3(256), 0, static_cast<cudaStream_t>(stream),
+                           param, ema, reinterpret_cast<__nv_bfloat16*>(param_bf16), n));
+  note_launch();
   return LIREC_OK;
 }

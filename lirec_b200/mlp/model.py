@@ -9,6 +9,7 @@ C ABI of include/lirec_b200.h); the nn.Linear submodules below only OWN paramete
 storage is re-pointed into one flat fp32 buffer (plus a flat gradient buffer and a bf16 shadow)
 that the kernels read and write in place.  There is no PyTorch or CPU fallback.
 """
+import contextlib
 import ctypes as C
 import math
 
@@ -23,7 +24,7 @@ from lirec_b200.utils.arg_pars import opt
 __all__ = ["Modalities", "MidFusionMultiClip", "MidFusionMultiClipMaxTracks", "GatingUnit",
            "MultiTaskCrossEntropyLoss", "MultiTaskMaxMargin", "MaxMarginCrossEntropyLoss", "MarginLoss",
            "MarginTrackRelsLoss", "MultiLabelBCELoss", "TrackBCELoss", "create_model", "ModelOutput", "FlatAdam",
-           "FlatLamb", "clip_grad_norm_flat_"]
+           "FlatLamb", "clip_grad_norm_flat_", "FlatEMA"]
 
 _SLOTS = ("txt", "vis", "tracks1", "tracks2")
 _SECOND = ("txt2", "vis2", "tracks12", "tracks22")
@@ -931,6 +932,93 @@ def clip_grad_norm_flat_(model, max_norm, grad_scale=1.0, tensor_norms=None):
     return norm
 
 
+class FlatEMA:
+    """Exponential moving average of a lirec_b200 model's parameters in one flat fp32 buffer laid out like the
+    model's flat parameter buffer, for evaluation and checkpoints (--ema_decay).  The semantics are those of
+    torch.optim.swa_utils.AveragedModel(model, multi_avg_fn=get_ema_multi_avg_fn(decay)): the buffer starts as a copy
+    of the weights, the first update() copies them again, and every later update() is ema = lerp(ema, w, 1 - decay)
+    in fp32 (torch._foreach_lerp_) as one launch of lirec_ema_update_flat.  The update only reads the weights, so it
+    cannot change training.  swap() exchanges the weights and the average in one launch that also refreshes the bf16
+    shadow; applied() evaluates the average inside a with-block.  The model's flat buffers are looked up at every call
+    (data parallelism may swap them for symmetric memory); their size may not change."""
+
+    def __init__(self, model, decay):
+        decay = float(decay)
+        if not (math.isfinite(decay) and 0.0 < decay < 1.0):
+            raise ValueError("FlatEMA: decay must be finite and in (0, 1) (got %r)" % (decay,))
+        model._sync_flat()
+        self.model, self.decay, self.n_averaged = model, decay, 0
+        self._ema = model._flat.detach().clone()
+
+    def _flat(self):
+        flat = self.model._flat
+        if flat.numel() != self._ema.numel() or flat.device != self._ema.device:
+            raise RuntimeError("FlatEMA: the model's flat buffer changed size or device (%d floats on %s, the average "
+                               "holds %d on %s)" % (flat.numel(), flat.device, self._ema.numel(), self._ema.device))
+        return flat
+
+    @torch.no_grad()
+    def update(self):
+        """Fold the current weights into the average (after every optimizer step), on the current stream."""
+        flat = self._flat()
+        if self.n_averaged == 0:
+            self._ema.copy_(flat)
+        else:
+            ops.ema_update_flat(self._ema, flat, self.decay)
+        self.n_averaged += 1
+
+    @torch.no_grad()
+    def swap(self):
+        """Exchange the model's weights and the average; the bf16 shadow follows the new weights."""
+        m = self.model
+        m._sync_flat()
+        ops.ema_swap_flat(self._flat(), self._ema, m._flat_bf16)
+        m.mark_bf16_fresh()
+
+    @contextlib.contextmanager
+    def applied(self):
+        """with ema.applied(): the model holds the average inside the block and its own weights again after it,
+        also when the block raises."""
+        self.swap()
+        try:
+            yield self.model
+        finally:
+            self.swap()
+
+    def _param_slices(self):
+        m = self.model
+        m._sync_flat()
+        for (name, p), q, off in zip(m.named_parameters(), m._param_list, m._offsets):
+            assert p is q
+            yield name, self._ema[off:off + p.numel()].view(p.shape)
+
+    @torch.no_grad()
+    def state_dict(self):
+        """{"decay", "n_averaged", "state_dict"}: the inner state_dict has model.state_dict()'s keys and shapes, so a
+        plain model can load_state_dict() the average.  Parameters are copies of the average; any other entry is the
+        live model's."""
+        avg = dict(self._param_slices())
+        sd = {k: (avg[k] if k in avg else v).detach().clone() for k, v in self.model.state_dict().items()}
+        return {"decay": self.decay, "n_averaged": self.n_averaged, "state_dict": sd}
+
+    @torch.no_grad()
+    def load_state_dict(self, state):
+        """Restore the average and n_averaged of state_dict() bit for bit (the decay stays the one given to the
+        constructor)."""
+        sd = state["state_dict"]
+        slices = dict(self._param_slices())
+        missing = sorted(set(slices) - set(sd))
+        if missing:
+            raise KeyError("FlatEMA.load_state_dict: the average has no entry for %s" % ", ".join(missing))
+        for name, dst in slices.items():
+            src = sd[name]
+            if tuple(src.shape) != tuple(dst.shape):
+                raise ValueError("FlatEMA.load_state_dict: %s has shape %s, the model %s"
+                                 % (name, tuple(src.shape), tuple(dst.shape)))
+            dst.copy_(src)
+        self.n_averaged = int(state["n_averaged"])
+
+
 def _check_loss_choice():
     """--loss against the rest of the configuration (host only, before any device work)."""
     kind = getattr(opt, "loss", "margin")
@@ -962,13 +1050,22 @@ def _check_clip_choice():
     return v
 
 
+def _check_ema_choice():
+    """--ema_decay (host only, before any device work): 0 is off, anything else a finite decay in (0, 1)."""
+    v = float(getattr(opt, "ema_decay", 0.0) or 0.0)
+    if not (v == 0.0 or (math.isfinite(v) and 0.0 < v < 1.0)):
+        raise ValueError("--ema_decay must be 0 (off) or a finite decay in (0, 1) (got %r)" % (v,))
+    return v
+
+
 def create_model(n_classes, n_rels=0):
     """Reference: mlp/model.py:578-609 — same selection logic and return triple.  --loss bce / ce swap in the
     multi-label BCE or the softmax cross-entropy for the reference's max-margin losses; --optimizer lamb swaps in
-    FlatLamb for Adam.  --clip_grad_norm is checked here; the training loop applies it."""
+    FlatLamb for Adam.  --clip_grad_norm and --ema_decay are checked here; the training loop applies them."""
     loss_kind = _check_loss_choice()
     optimizer_kind = _check_optimizer_choice()
     _check_clip_choice()
+    _check_ema_choice()
     if opt.device != "cuda":
         raise RuntimeError("lirec_b200 runs on a B200 only (opt.device='%s'); no CPU fallback" % opt.device)
     if opt.tr_maximize:

@@ -12,7 +12,7 @@ from ._ext import (ACT_NONE, ACT_RELU, ACT_TANH, OUT_F32, OUT_SPLIT, OUT_SPLIT_T
                    POST_NONE, POST_SIGN_MASK)
 
 __all__ = ["gemm_problem", "gemm_grouped", "seg_reduce", "seg_softmax_pool", "seg_softmax_pool_bwd", "SegSoftmaxPool", "rows_expand_fwd", "rows_expand_bwd", "split_f32",
-           "cast_bf16", "gather_rows", "roi_max_pool", "loss_track", "loss_rowmargin", "loss_ce", "loss_bce", "loss_bce_track", "predict_tracks", "adam_flat", "lamb_partials", "lamb_flat", "grad_clip_flat", "dp_exchange", "dp_reduce_adam_bcast", "dp_reduce_adam_bcast_peer", "dropout_desc"]
+           "cast_bf16", "gather_rows", "roi_max_pool", "loss_track", "loss_rowmargin", "loss_ce", "loss_bce", "loss_bce_track", "predict_tracks", "adam_flat", "lamb_partials", "lamb_flat", "grad_clip_flat", "ema_update_flat", "ema_swap_flat", "dp_exchange", "dp_reduce_adam_bcast", "dp_reduce_adam_bcast_peer", "dropout_desc"]
 
 
 def dropout_desc(p=0.0, seed=0, stream_id=0, col_off=0):
@@ -351,6 +351,36 @@ def grad_clip_flat(grad, tensor_begin, tensor_len, partials, max_norm, grad_scal
         _ext.ptr(partials), int(partials.numel() // 2), float(max_norm), float(grad_scale), _ext.ptr(norm_out),
         _ext.ptr(tensor_norms_out), sp))
     return norm_out
+
+
+def _ema_pair(what, a, b):
+    for t in (a, b):
+        if t.dtype != torch.float32 or not t.is_contiguous():
+            raise ValueError("%s: param and ema must be contiguous float32 tensors" % what)
+    if a.numel() != b.numel() or a.device != b.device:
+        raise ValueError("%s: param and ema must have one size and one device (%d, %d)" % (what, a.numel(), b.numel()))
+
+
+def ema_update_flat(ema, param, decay, stream=None):
+    """ema <- lerp(ema, param, 1 - decay) in place (lirec_ema_update_flat): the update of torch.optim.swa_utils'
+    get_ema_multi_avg_fn(decay), torch.lerp's arithmetic in fp32.  1 - decay is formed here in double; the entry
+    point refuses it unless it is finite and in (0, 1)."""
+    _ema_pair("ema_update_flat", param, ema)
+    sp = _ext.stream_ptr() if stream is None else C.c_void_p(stream.cuda_stream)
+    _ext.check(_ext.lib().lirec_ema_update_flat(_ext.ptr(ema), _ext.ptr(param), int(param.numel()),
+                                                1.0 - float(decay), sp))
+
+
+def ema_swap_flat(param, ema, param_bf16=None, stream=None):
+    """Exchange param and ema in place, and refresh the bf16 shadow param_bf16 (optional) from the new param with
+    cast_bf16's rounding (lirec_ema_swap_flat)."""
+    _ema_pair("ema_swap_flat", param, ema)
+    if param_bf16 is not None and (param_bf16.dtype != torch.bfloat16 or not param_bf16.is_contiguous() or
+                                   param_bf16.numel() != param.numel() or param_bf16.device != param.device):
+        raise ValueError("ema_swap_flat: param_bf16 must be a contiguous bfloat16 tensor the size of param")
+    sp = _ext.stream_ptr() if stream is None else C.c_void_p(stream.cuda_stream)
+    _ext.check(_ext.lib().lirec_ema_swap_flat(_ext.ptr(param), _ext.ptr(ema), _ext.ptr(param_bf16),
+                                              int(param.numel()), sp))
 
 
 def dp_reduce_adam_bcast(grad_mc, param, param_mc, bf16_mc, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, weight_decay,

@@ -136,6 +136,13 @@ _FLAGS = [
                                    "torch.nn.utils.clip_grad_norm_ (fused, no host sync; with --dp, the norm of the "
                                    "averaged gradient); turns off the fused exchange + Adam and --overlap_adam. "
                                    "0: off")),
+    ("--ema_decay", dict(default=0.0, type=float,
+                         help="in (0, 1): keep an exponential moving average of the parameters, like "
+                              "torch.optim.swa_utils.AveragedModel with get_ema_multi_avg_fn(decay): the first "
+                              "optimizer step copies the weights, every later one does ema = lerp(ema, w, 1 - decay) "
+                              "in fp32 (fused, no host sync; training is unchanged). Evaluation and checkpoint "
+                              "ranking use the average, checkpoints add it as 'ema'; --resume evaluates it. "
+                              "0: off")),
     ("--world_movies", dict(default=6, type=int)),
     ("--world_scenes", dict(default=40, type=int)),
 ]

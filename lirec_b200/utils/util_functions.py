@@ -72,3 +72,8 @@ def load_model(name=""):
 
 def load_optimizer():
     return torch.load(opt.resume_str, map_location="cpu")["optimizer"]
+
+
+def load_ema():
+    """The checkpoint's weight average (mlp.model.FlatEMA.state_dict(), saved under --ema_decay), or None."""
+    return torch.load(opt.resume_str, map_location="cpu").get("ema")
