@@ -70,7 +70,10 @@ int lirec_dropout_keep_host(uint32_t seed, uint32_t stream_id, uint32_t row, uin
  * index M (or N), cols index K.  MN-major use (mn_major=1): rows index K, cols
  * index M (or N) — this is how dgrad reads W[out,in] and wgrad reads dY / X
  * without a transposed copy.  A pass is one K-segment; several passes
- * accumulate into the same tile (hi/lo split operands, concatenated inputs). */
+ * accumulate into the same tile (hi/lo split operands, concatenated inputs).
+ * Pass p contributes sum_{k < k_len} A[a_mn_off + m, a_k_off + k] * B[b_mn_off + n, b_k_off + k]
+ * (indices (row, col) of a K-major view; swapped for an MN-major one): exactly k_len elements of K,
+ * whatever the view holds past a_k_off + k_len / b_k_off + k_len.  Elements outside a view read as 0. */
 #define LIREC_GEMM_MAX_PASSES 4
 #define LIREC_GEMM_MAX_PROBLEMS 32
 #define LIREC_GEMM_MAX_MAPS 64
@@ -83,9 +86,10 @@ typedef struct lirec_operand {
 
 typedef struct lirec_gemm_pass {
   lirec_operand a, b;
-  int32_t a_mn_off, a_k_off;  /* element offsets inside the view             */
+  int32_t a_mn_off, a_k_off;  /* element offsets inside the view; the one along the view's cols
+                               * (k_off K-major, mn_off MN-major) is a multiple of 8 (16 bytes) */
   int32_t b_mn_off, b_k_off;
-  int32_t k_len;              /* reduction length of this pass (elements)    */
+  int32_t k_len;              /* reduction length of this pass (elements, any count >= 1) */
 } lirec_gemm_pass;
 
 enum lirec_act { LIREC_ACT_NONE = 0, LIREC_ACT_RELU = 1, LIREC_ACT_TANH = 2 };
@@ -121,7 +125,7 @@ typedef struct lirec_epilogue {
   int64_t out_ld_m, out_ld_n; /* F32: &out[m*ld_m + n*ld_n]; SPLIT / SPLIT_T: ld_m only (row pitch) */
   int32_t out_col_off;      /* SPLIT: hi at col_off+n, lo at col_off+lo_off+n */
   int32_t out_lo_off;
-  int32_t accumulate;       /* F32 only: out += v                            */
+  int32_t accumulate;       /* out += v; F32 outputs only (refused otherwise) */
 } lirec_epilogue;
 
 typedef struct lirec_gemm_problem {
@@ -130,10 +134,13 @@ typedef struct lirec_gemm_problem {
   int32_t num_passes;
   lirec_gemm_pass pass[LIREC_GEMM_MAX_PASSES];
   lirec_epilogue epi;
-  /* split-K: when split_k > 1 the reduction range of every pass is cut into split_k slices of whole
-   * 64-element k-blocks; slice s runs as its own tiles and writes its partial result to
-   * out + s * split_stride (elements).  The caller sums the slices (fixed order = deterministic).
-   * Needs an F32 output without activation, post op or accumulate; a bias is added in slice 0 only. */
+  /* split-K: when split_k > 1 the reduction range of every pass is cut into slices of whole 64-element
+   * k-blocks; slice s runs as its own tiles and writes its partial result to out + s * split_stride
+   * (elements).  With kb = the k-block count ceil(k_len / 64) of the longest pass, every slice takes
+   * c = ceil(kb / min(split_k, kb)) k-blocks and the problem writes S = ceil(kb / c) slices, which may be
+   * fewer than split_k (kb = 9, split_k = 4: c = 3, S = 3); slices S .. split_k-1 are not written.  The
+   * caller sums the S slices (fixed order = deterministic).  Needs an F32 output without activation, post
+   * op or accumulate; a bias is added in slice 0 only. */
   int32_t split_k;
   int64_t split_stride;
 } lirec_gemm_problem;

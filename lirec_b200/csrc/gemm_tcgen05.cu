@@ -338,7 +338,9 @@ __device__ __forceinline__ void split_bf16x2(float a, float b, uint32_t& hi2, ui
   lo2 = *reinterpret_cast<const uint32_t*>(&l);
 }
 
-__device__ __forceinline__ void load_bf16x32(const __nv_bfloat16* p, bool vec, float (&out)[32]) {
+// vec: 16-byte loads of a full chunk; otherwise element loads of the first nvalid columns (the rest read as 0 —
+// columns past N may lie past the end of the tensor)
+__device__ __forceinline__ void load_bf16x32(const __nv_bfloat16* p, bool vec, int nvalid, float (&out)[32]) {
   if (vec) {
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
@@ -352,7 +354,7 @@ __device__ __forceinline__ void load_bf16x32(const __nv_bfloat16* p, bool vec, f
     }
   } else {
 #pragma unroll
-    for (int j = 0; j < 32; ++j) out[j] = __bfloat162float(p[j]);
+    for (int j = 0; j < 32; ++j) out[j] = j < nvalid ? __bfloat162float(p[j]) : 0.f;
   }
 }
 
@@ -459,7 +461,7 @@ __device__ __forceinline__ void epilogue_chunk(const DevEpi& e, int M, int N, in
   } else if (e.post == LIREC_POST_DRELU) {
     float g[32];
     if (aux.ready) unpack_bf16x32(aux.hi, g);
-    else load_bf16x32(e.aux + static_cast<int64_t>(m) * e.aux_ld + e.aux_col_off + n0, full && e.aux_vec_ok, g);
+    else load_bf16x32(e.aux + static_cast<int64_t>(m) * e.aux_ld + e.aux_col_off + n0, full && e.aux_vec_ok, nvalid, g);
 #pragma unroll
     for (int j = 0; j < 32; ++j) v[j] = (g[j] > 0.f) ? v[j] * e.post_scale : 0.f;
   } else if (e.post == LIREC_POST_DTANH) {
@@ -469,8 +471,8 @@ __device__ __forceinline__ void epilogue_chunk(const DevEpi& e, int M, int N, in
       unpack_bf16x32(aux.hi, hi);
       unpack_bf16x32(aux.lo, lo);
     } else {
-      load_bf16x32(ap, full && e.aux_vec_ok, hi);
-      load_bf16x32(ap + e.aux_lo_off, full && e.aux_vec_ok, lo);
+      load_bf16x32(ap, full && e.aux_vec_ok, nvalid, hi);
+      load_bf16x32(ap + e.aux_lo_off, full && e.aux_vec_ok, nvalid, lo);
     }
     const float unscale = 1.0f - e.drop_p;   // undo the 1/(1-p) of the forward dropout
     uint32_t rkey = 0, thr = 0, pair0 = 0;
@@ -1215,8 +1217,15 @@ int run_grouped(const lirec_gemm_problem* probs, int nprobs, cudaStream_t stream
   static thread_local GemmParams P;  // 16 KB: keep it off the stack
   std::vector<MapKey> keys;
   keys.reserve(MAX_MAPS);
-  auto map_index = [&](const lirec_operand& op, bool mn_major, int tile_mn) -> int {
+  // A pass reads exactly [k_off, k_off + k_len) of its operands, but TMA fetches whole 64-element k-blocks: when
+  // k_len is not a multiple of 64 the pass's map ends its K extent (cols K-major, rows MN-major) at k_off + k_len,
+  // so the rest of the last k-block is zero fill instead of the operand's next columns / rows.
+  auto map_index = [&](const lirec_operand& op, bool mn_major, int tile_mn, int k_off, int k_len) -> int {
     MapKey k{op.ptr, op.rows, op.cols, op.ld, mn_major ? BK : tile_mn};
+    if (k_len % BK != 0) {
+      int64_t& k_extent = mn_major ? k.rows : k.cols;
+      k_extent = std::min<int64_t>(k_extent, static_cast<int64_t>(k_off) + k_len);
+    }
     for (size_t i = 0; i < keys.size(); ++i)
       if (keys[i] == k) return (int)i;
     if ((int)keys.size() >= MAX_MAPS) return -1;
@@ -1252,15 +1261,16 @@ int run_grouped(const lirec_gemm_problem* probs, int nprobs, cudaStream_t stream
     d.tiles_mn = tiles_m * d.tiles_n;
     int max_kb = 0;
     for (int ps = 0; ps < g.num_passes; ++ps) max_kb = std::max(max_kb, (g.pass[ps].k_len + BK - 1) / BK);
-    int split = std::max(1, std::min(g.split_k, max_kb));
+    const int split = split_k_slices(max_kb, g.split_k);
     LIREC_REQUIRE(split == 1 || g.epi.out_kind == LIREC_OUT_F32, "problem %d: split-K needs an fp32 output", idx);
     LIREC_REQUIRE(split == 1 || (g.epi.act == LIREC_ACT_NONE && g.epi.post == LIREC_POST_NONE && !g.epi.accumulate),
                   "problem %d: split-K partial sums cannot carry an activation, post op or accumulate", idx);
     LIREC_REQUIRE(g.epi.out_kind == LIREC_OUT_F32 || g.epi.out_kind == LIREC_OUT_SPLIT_BF16 ||
                       g.epi.out_kind == LIREC_OUT_SPLIT_BF16_T,
                   "problem %d: out_kind=%d", idx, g.epi.out_kind);
+    LIREC_REQUIRE(!g.epi.accumulate || g.epi.out_kind == LIREC_OUT_F32, "problem %d: accumulate needs an fp32 output",
+                  idx);
     d.split_chunk = (split > 1) ? (max_kb + split - 1) / split : 0x3fffffff;
-    if (split > 1) split = (max_kb + d.split_chunk - 1) / d.split_chunk;   // every slice non-empty
     d.split_stride = g.split_stride;
     d.a_mn_major = g.a_mn_major ? 1 : 0;
     d.b_mn_major = g.b_mn_major ? 1 : 0;
@@ -1275,8 +1285,12 @@ int run_grouped(const lirec_gemm_problem* probs, int nprobs, cudaStream_t stream
     for (int ps = 0; ps < g.num_passes; ++ps) {
       const lirec_gemm_pass& s = g.pass[ps];
       LIREC_REQUIRE(s.k_len > 0, "problem %d pass %d: k_len=%d", idx, ps, s.k_len);
-      const int ia = map_index(s.a, d.a_mn_major, BM);
-      const int ib = map_index(s.b, d.b_mn_major, b_box);
+      // a TMA box starts 16-byte aligned along the view's columns (k_off K-major, mn_off MN-major); an unaligned
+      // start never completes its load and the pipeline would wait forever
+      LIREC_REQUIRE((d.a_mn_major ? s.a_mn_off : s.a_k_off) % 8 == 0 && (d.b_mn_major ? s.b_mn_off : s.b_k_off) % 8 == 0,
+                    "problem %d pass %d: offsets along an operand's columns must be multiples of 8 elements", idx, ps);
+      const int ia = map_index(s.a, d.a_mn_major, BM, s.a_k_off, s.k_len);
+      const int ib = map_index(s.b, d.b_mn_major, b_box, s.b_k_off, s.k_len);
       if (ia < 0 || ib < 0) return fail(LIREC_ERR_LIMIT, "more than %d tensor maps in one launch", MAX_MAPS);
       const Spec sa{ia, s.a_mn_off, s.a_k_off}, sb{ib, s.b_mn_off, s.b_k_off};
       const int kb = (s.k_len + BK - 1) / BK;
@@ -1358,8 +1372,9 @@ int run_grouped(const lirec_gemm_problem* probs, int nprobs, cudaStream_t stream
         (g.N % 32 != 0 || e.aux_ld < g.N / 32 || (reinterpret_cast<uintptr_t>(e.aux) & 3) != 0))
       return fail(LIREC_ERR_ARG, "problem %d: sign mask needs N %% 32 == 0 and aux_ld >= N / 32 words", idx);
     const uintptr_t ob = reinterpret_cast<uintptr_t>(e.out);
-    if (e.out_kind == LIREC_OUT_F32)
-      de.vec_ok = (e.out_ld_n == 1 && (ob & 15) == 0 && (e.out_ld_m % 4) == 0) ? 1 : 0;
+    if (e.out_kind == LIREC_OUT_F32)   // every split-K slice starts 16-byte aligned too
+      de.vec_ok = (e.out_ld_n == 1 && (ob & 15) == 0 && (e.out_ld_m % 4) == 0 && (split == 1 || g.split_stride % 4 == 0))
+                      ? 1 : 0;
     else if (e.out_kind == LIREC_OUT_SPLIT_BF16_T)   // 16-byte pieces of eight consecutive m (staged store)
       de.vec_ok = ((ob & 15) == 0 && (e.out_ld_m % 8) == 0) ? 1 : 0;
     else

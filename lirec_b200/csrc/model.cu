@@ -567,10 +567,9 @@ int forward(const lirec_model_cfg& cfg, const lirec_model_params& P, const lirec
     ReduceJobs jobs;
     jobs.n = 0;
     if (S > 1 && (size_t)S * d.Ni * d.C <= w.pool_floats) {
-      const int kb = (width + 63) / 64, chunk = (kb + S - 1) / S;
       ReduceJob& j = jobs.job[jobs.n++];
       j.dst = out_ints; j.dst_ld = d.C; j.src = w.pool; j.M = d.Ni; j.N = d.C;
-      j.S = (kb + chunk - 1) / chunk;
+      j.S = gemm::split_k_slices((width + 63) / 64, S);
       g.split_k = S;
       g.split_stride = (int64_t)d.Ni * d.C;
       g.epi.out = w.pool;
@@ -661,8 +660,7 @@ static void push_reduction(std::vector<lirec_gemm_problem>& pr, lirec_gemm_probl
     j.dst_ld = transposed ? g.epi.out_ld_n : g.epi.out_ld_m;
     j.src = sc.pool + sc.used;
     j.M = out_f; j.N = in_f;
-    const int kb = (rows + 63) / 64, chunk = (kb + S - 1) / S;
-    j.S = (kb + chunk - 1) / chunk;                       // the slice count the GEMM will actually use
+    j.S = gemm::split_k_slices((rows + 63) / 64, S);     // the slice count the GEMM will actually use
     g.split_k = S;
     g.split_stride = (int64_t)out_f * in_f;
     g.epi.out = sc.pool + sc.used;
